@@ -3,6 +3,8 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c2w|c2d5|c5|c3]      our arm (CUDA, libpgp.so)
   python bench.py --impl reference [...]                                                 the reference's CPU code on the host cores
+  python bench.py [...] --dump-outputs DIR      also write what the last timed step computed (counts, scores, merged top-k) as
+                                                DIR/<name>.npy; the inputs are seeded, so two builds can be compared array by array
 
 Configs (BASELINE.json `configs`, SURVEY.md 8):
   c2    configs[1], the headline: 2k-pt model, 100k-pt scene, 100k hypotheses per GPU, delta = 1 cm, Verify (count)      weak scaling
@@ -32,8 +34,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: leave no __pycache__ behind
 
 TOPK = 64
+DUMP_MAX_HYP = 1 << 20                  # per-hypothesis arrays beyond this are dumped as a fixed, seeded sample (<= 20 MB)
 METRIC = "LCP hypotheses scored/sec at 1/2/4/8 B200 (2k-pt model, 100k-pt scene)"
 UNIT = "hyp/s"
 CONFIGS = {
@@ -238,7 +242,7 @@ def run_reference(args, rank):
         return
     cfg = CONFIGS[args.config]
     if args.config == "c3":
-        base, ms = cpu_pcs_run(cfg, max(1, min(args.steps, 5)))
+        base, ms = cpu_pcs_run(cfg, args.steps)
         sample_n = None
     else:
         prob, T, _ = make_inputs(dict(cfg, n_hyp=min(cfg["n_hyp"], 100_000)), 0, 1)
@@ -479,6 +483,13 @@ def run_scoring(args, D: Dist, local_rank: int):
     exchange_tail_ms = ev[-1][0].elapsed_time(ev[-1][1])
     wall_ms = D.reduce(wall_ms)
     value = n_step_total * args.steps / (total_ms * 1e-3)
+    outputs = {}
+    if args.dump_outputs:       # the last timed step's counts / scores (later passes reuse the buffers) and its merged top-k
+        sfx = f"_rank{rank}" if world > 1 else ""
+        per_hyp = hypothesis_arrays(counts_dev.cpu().numpy(), scores_dev.cpu().numpy(), index_base, world)
+        outputs = {k + sfx: v for k, v in per_hyp.items()}
+        if rank == 0:
+            outputs.update(topk_arrays(top))
 
     # ---- the same K steps back to back WITHOUT the L2 flush, one event pair around all of them incl. the last exchange: what a
     # pipelined caller sees (warm L2; reported next to the headline, not instead of it)
@@ -615,6 +626,8 @@ def run_scoring(args, D: Dist, local_rank: int):
             line["parity"] = {"checked": int(n_chk * world), "mismatches": int(mism_total), "against": kind, "what": f"{n_chk} hypotheses of every rank's shard"}
             line["sharding_invariance"] = invariance
         emit(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     eng.close()
 
 
@@ -626,7 +639,7 @@ def run_pcs(args, D: Dist, local_rank: int):
     import torch
 
     from physimglobalpose_b200 import synth
-    from physimglobalpose_b200.engine import PoseEngine
+    from physimglobalpose_b200.engine import HYP_DTYPE, PoseEngine
     from physimglobalpose_b200.sharding import comm_init_from_env, shard_range
 
     cfg = CONFIGS["c3"]
@@ -648,11 +661,14 @@ def run_pcs(args, D: Dist, local_rank: int):
     lo, hi = shard_range(B, rank, world)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
+    kept = {}                                       # object -> (global index of this rank's first hypothesis, hypotheses it kept)
+
     def request(o, seed):
         seg = objs[o]
         eng.set_scene(seg.scene_xyz, seg.scene_nrm, cfg["delta"])
-        eng.generate_pcs_range(o, lo, hi, seed=seed, max_hyp=cfg["n_hyp"], mode=1, n_bases=B)
+        n_gen = eng.generate_pcs_range(o, lo, hi, seed=seed, max_hyp=cfg["n_hyp"], mode=1, n_bases=B)
         base, total = eng.sync_generated(o, cfg["n_hyp"])
+        kept[o] = (base, max(0, min(n_gen, total - base)))     # the global cap is filled in rank order
         eng.score_generated(o, "weighted")
         return eng.topk_begin(o, TOPK, base), total
 
@@ -721,6 +737,20 @@ def run_pcs(args, D: Dist, local_rank: int):
                 "note": "top64_digest must be identical for every --gpus N (same seed -> same bases -> same hypotheses whichever GPU generates them)"}
         line["cpu_baseline"] = cpu
         emit(line)
+    if args.dump_outputs:       # the last timed step: per object, the merged top-64 and a sample of this rank's generated hypotheses
+        top = np.zeros((cfg["objects"], TOPK), HYP_DTYPE)
+        top["index"] = -1                           # a list shorter than TOPK is padded like the engine pads it
+        for o, t in enumerate(tops):
+            top[o, :len(t)] = t
+        sfx = f"_rank{rank}" if world > 1 else ""
+        outputs = dict(topk_arrays(top), hypotheses_generated=np.array([n], np.float64)) if rank == 0 else {}
+        for o in range(cfg["objects"]):
+            base, n_kept = kept[o]
+            T_gen, c_gen, s_gen = (a[:n_kept] for a in eng.get_generated(o))
+            per_hyp = hypothesis_arrays(c_gen, s_gen, base, world * cfg["objects"] * 2)      # / 2: T too, 68 bytes a hypothesis
+            per_hyp["generated_T"] = T_gen[(per_hyp["hypothesis_index"] - base).astype(np.int64)].astype(np.float32)
+            outputs.update({f"object{o}_{k}{sfx}": v for k, v in per_hyp.items()})
+        dump_outputs(args.dump_outputs, outputs)
     eng.close()
 
 
@@ -747,6 +777,27 @@ def _claim_stdout():
     os.dup2(2, 1)
 
 
+def topk_arrays(top: np.ndarray) -> dict:
+    """Merged top-k records (engine.HYP_DTYPE, any leading shape) as the arrays a caller reads from them."""
+    return {"topk_index": top["index"].astype(np.float64), "topk_count": top["count"].astype(np.float64),
+            "topk_score": top["score"].astype(np.float32), "topk_T": top["T"].reshape(*top.shape, 3, 4).astype(np.float32)}
+
+
+def hypothesis_arrays(counts: np.ndarray, scores: np.ndarray, index_base: int, world: int) -> dict:
+    """Per-hypothesis counts and scores of a rank's batch with their global hypothesis indices; a batch larger than this rank's
+    share of DUMP_MAX_HYP is reduced to a sample drawn with a fixed seed, so two runs dump the same hypotheses."""
+    n, cap = len(counts), DUMP_MAX_HYP // world
+    sel = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    return {"hypothesis_index": (sel + index_base).astype(np.float64), "counts": counts[sel].astype(np.float64),
+            "scores": scores[sel].astype(np.float32)}
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def emit(line: dict):
     data = (json.dumps(line) + "\n").encode()
     if _RESULT_FD is None:
@@ -763,9 +814,15 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"c5": 5, "c3": 3}.get(args.config, 20)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libs4ref.so")
 PORT_SO = os.path.join(ROOT, "oracle", "_build", "liblcp_oracle.so")
 
-pytestmark = pytest.mark.skipif(not (os.path.exists(REF_SO) or os.path.exists(PORT_SO)), reason="no CPU checker built (python -c 'import __graft_entry__ as g; g.build()')")
+needs_checker = pytest.mark.skipif(not (os.path.exists(REF_SO) or os.path.exists(PORT_SO)), reason="no CPU checker built (python -c 'import __graft_entry__ as g; g.build()')")
 
 KEYS = {"impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config",
         "cpu_baseline", "e2e"}
@@ -25,6 +25,7 @@ def _one_json_line(out: str) -> dict:
     return json.loads(lines[0])
 
 
+@needs_checker
 @pytest.mark.timeout(300)
 def test_reference_arm_prints_one_contract_line():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"], capture_output=True, text=True, cwd=ROOT)
@@ -39,6 +40,7 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+@needs_checker
 @pytest.mark.timeout(300)
 def test_reference_arm_under_a_two_rank_launch():
     """The driver launches the reference arm like the GPU arm (torchrun): rank 0 alone works and prints, rank 1 exits 0 silently."""
@@ -59,6 +61,34 @@ def test_hypothesis_ranges_tile_the_global_list():
     parts = [synth.make_hypotheses_range(prob, lo, hi, seed=9, block=1024) for lo, hi in ((0, 700), (700, 700), (700, 2049), (2049, 3000))]
     assert np.array_equal(np.concatenate(parts), whole)
     assert not np.array_equal(whole[:1024], whole[1024:2048])          # blocks are drawn with their own generators
+
+
+def test_dumped_outputs_are_float_seeded_and_bounded(tmp_path):
+    """--dump-outputs: every array is float32 / float64, a batch beyond DUMP_MAX_HYP is the same seeded sample on every call (split
+    over the ranks), indices are global, and the top-k keeps its records' shape."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from physimglobalpose_b200.engine import HYP_DTYPE
+    n = bench.DUMP_MAX_HYP + 4321
+    counts = (np.arange(n, dtype=np.int64) * 7919 % 2001).astype(np.int32)
+    scores = counts.astype(np.float32) / np.float32(2000)
+    a, b = (bench.hypothesis_arrays(counts, scores, 1000, 2) for _ in range(2))
+    assert len(a["counts"]) == bench.DUMP_MAX_HYP // 2 and all(np.array_equal(a[k], b[k]) for k in a)
+    idx = a["hypothesis_index"].astype(np.int64) - 1000
+    assert np.all(np.diff(idx) > 0) and np.array_equal(a["counts"], counts[idx]) and np.array_equal(a["scores"], scores[idx])
+    small = bench.hypothesis_arrays(counts[:500], scores[:500], 0, 1)
+    assert np.array_equal(small["hypothesis_index"], np.arange(500))
+    top = np.zeros((4, 64), HYP_DTYPE)
+    top["index"], top["T"] = np.arange(256).reshape(4, 64), 1.5
+    t = bench.topk_arrays(top)
+    assert t["topk_T"].shape == (4, 64, 3, 4) and np.array_equal(t["topk_index"], np.arange(256).reshape(4, 64))
+    bench.dump_outputs(str(tmp_path / "out"), dict(a, **t))
+    total = 0
+    for name in list(a) + list(t):
+        arr = np.load(tmp_path / "out" / f"{name}.npy")
+        assert arr.dtype in (np.float32, np.float64)
+        total += arr.nbytes
+    assert total <= 64 << 20
 
 
 def test_clock_sampler_parses_nvidia_smi_rows(tmp_path, monkeypatch):

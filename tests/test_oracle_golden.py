@@ -84,10 +84,23 @@ def test_lcp_invariants(port_lib):
         last = cur
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference tree (build container only)")
-def test_port_equals_reference_live(port_lib):
-    """Fresh seeded inputs, reference engine compiled in place (oracle/_ref) vs the C restatement."""
-    port_lib.build_ref()
+def test_port_equals_reference_live(port_lib, lcp):
+    """The C restatement, its multi-threaded CPU-baseline driver included, against the reference's own Verify / WeightedVerify /
+    running-best answers stored in lcp_small.npz and lcp_full_shapes.npz; where the reference engine is built (oracle/_ref), also
+    against the reference itself on fresh seeded inputs."""
+    o = _port(port_lib, lcp)
+    assert np.array_equal(o.verify(lcp["T"]), lcp["counts"])
+    ws, wn = o.weighted_verify(lcp["T"])
+    assert np.array_equal(ws, lcp["weighted_score"]) and np.array_equal(wn, lcp["weighted_nreg"])
+    frac, best = o.verify_running_best(lcp["T"])
+    assert best == int(lcp["running_best"]) and np.array_equal(frac, lcp["running_frac"])
+    assert np.array_equal(o.verify_mt(lcp["T"], 3)[0], lcp["counts"])
+    g = np.load(os.path.join(G, "lcp_full_shapes.npz"))
+    prob, T = _full_shape(g, "c2")
+    full = port_lib.PortOracle(prob.scene_xyz, prob.scene_nrm, prob.model_xyz, prob.model_nrm, prob.model_xyz, prob.model_nrm, prob.delta)
+    assert np.array_equal(full.verify_mt(T, 3)[0], g["c2_counts"])
+    if not port_lib.have_ref():
+        return
     prob = synth.make_problem(400, 9000, 0.01, seed=31)
     T = synth.make_hypotheses(prob, 200, seed=32)
     args = (prob.scene_xyz, prob.scene_nrm, prob.model_xyz, prob.model_nrm, prob.model_xyz, prob.model_nrm, prob.delta)
