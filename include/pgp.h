@@ -101,7 +101,9 @@ PGP_API int pgp_set_scene(pgp_ctx* ctx, const float* xyz_host, const float* nrm_
  * pin-hole projection of the un-centred point through K (row-major 3x3).  img: rows x cols uint16.
  * (The reference indexes the image unchecked; here row/col are clamped into the image.) */
 PGP_API int pgp_set_scene_prior_image(pgp_ctx* ctx, const uint16_t* img_host, int rows, int cols, const float* K9);
-/* Or hand the priors over directly (orig_probabilities_, one per scene point). */
+/* Or hand the priors over directly (orig_probabilities_, one per scene point).  Any finite value is accepted, negative ones too:
+ * a weighted score is then the exact ordered sum and may be negative, and selection orders it as an fp32 value (a score <= 0
+ * never enters the improving chain).  A NaN or infinite prior is refused with PGP_E_INVALID and the previous priors stay. */
 PGP_API int pgp_set_scene_priors(pgp_ctx* ctx, const float* prior_host);
 PGP_API int pgp_get_scene_priors(pgp_ctx* ctx, float* prior_host);
 
@@ -187,14 +189,16 @@ PGP_API int pgp_topk_end(pgp_ctx* ctx, int ticket, pgp_hyp* out_host);
  * the exchange with events on its own stream; not needed for correctness). */
 PGP_API int pgp_topk_stream_wait(pgp_ctx* ctx, int ticket);
 /* Same, asynchronous, with the k records written straight into caller-owned DEVICE memory (the
- * send buffer of the multi-GPU all-gather); slots beyond the batch size get index = -1. */
+ * send buffer of the multi-GPU all-gather); slots beyond the batch size get index = -1.  Always local:
+ * PGP_INDEX_AUTO means base 0. */
 PGP_API int pgp_topk_dev(pgp_ctx* ctx, int obj, int k, int64_t index_base, pgp_hyp* out_dev);
 /* Deterministic merge of per-rank top-k lists (n_lists x k_each records, e.g. the output of an
  * all-gather): same order as pgp_topk on the union.  Host-side, no context needed. */
 PGP_API int pgp_topk_merge(const pgp_hyp* lists, int n_lists, int k_each, int k, pgp_hyp* out);
 /* The strictly-improving chain in generation order that Perform_N_steps returns as
  * hypothesisSet (match4pcsBase.cc:1888-1914); its last element is bestHypothesis.
- * Returns the chain length (<= cap) or PGP_E_CAPACITY.  Collective on a communicator context, like pgp_topk: the chain over the
+ * Returns the chain length (<= cap) or PGP_E_CAPACITY: for a chain of at most 4096 elements out_host then holds its last cap
+ * elements; a longer chain leaves out_host unusable.  Collective on a communicator context, like pgp_topk: the chain over the
  * ranks' batches in rank order (each rank may contribute at most PGP_CHAIN_EXCHANGE_CAP elements). */
 PGP_API int pgp_improving_chain(pgp_ctx* ctx, int obj, int64_t index_base, pgp_hyp* out_host, int cap);
 

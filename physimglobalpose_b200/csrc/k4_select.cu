@@ -4,12 +4,13 @@
 // and the result shaping of :1903-1914 / ComputeTransformation :1787-1796.
 //
 // Order: (score desc, generation index asc).  The pair is packed into ONE unique 64-bit key
-//   key = score_bits << ibits | (n - 1 - i)
-// so "top-k" = the k largest keys; an MSB-first radix select (11-bit digits) finds the k-th key
-// exactly, a compaction gathers the k survivors, one CTA sorts them.  Everything runs in ONE
-// cooperative launch (one CTA per SM, software grid barrier between the passes), because at the
-// benchmark size the whole selection is a few hundred KB of L2 reads and would otherwise be
-// launch-latency bound.
+//   key = key32(score) << ibits | (n - 1 - i)
+// where key32 is the count itself (COUNT mode) or the fp32 score mapped to an unsigned integer of the same order
+// (WEIGHTED mode, float_key below: negative scores rank below +0, -0 ties with +0), so "top-k" = the k largest
+// keys; an MSB-first radix select (11-bit digits) finds the k-th key exactly, a compaction gathers the k
+// survivors, one CTA sorts them.  Everything runs in ONE cooperative launch (one CTA per SM, software grid
+// barrier between the passes), because at the benchmark size the whole selection is a few hundred KB of L2
+// reads and would otherwise be launch-latency bound.
 #include <algorithm>
 #include <math.h>
 
@@ -21,10 +22,11 @@ constexpr int ST = 1024;          // threads per CTA
 constexpr int DIGIT = 11;
 constexpr int BINS = 1 << DIGIT;
 constexpr int MAX_PASSES = 6;
-constexpr int KMAX = 4096;
+constexpr int KMAX = K4_MAX_K;
 
 struct SelParams {
-  const uint32_t* key32;     // counts, or float score bits (scores are >= 0, so the bits are monotone)
+  const uint32_t* key32;     // counts, or the bits of the fp32 scores (float_keys: mapped by float_key before any comparison)
+  bool float_keys;
   const float* scores;       // may be null
   const uint32_t* counts;    // may be null
   const float* T;
@@ -60,8 +62,22 @@ __device__ __forceinline__ void grid_barrier(unsigned* bar, unsigned& epoch) {
   __syncthreads();
 }
 
+// fp32 bits -> unsigned key with the order of the float values.  Priors may be negative (pgp_set_scene_priors), so a weighted score
+// may be too: -0 is folded into +0 (they compare equal, the index decides), negative values are bit-inverted (below 0x80000000, the
+// more negative the smaller), non-negative ones get the top bit set.
+__device__ __forceinline__ uint32_t float_key(uint32_t bits) {
+  const uint32_t u = bits == 0x80000000u ? 0u : bits;
+  return (u >> 31) ? ~u : (u | 0x80000000u);
+}
+constexpr uint32_t FLOAT_KEY_ZERO = 0x80000000u;   // float_key(+0.f)
+
+__device__ __forceinline__ uint32_t key32_at(const SelParams& p, long long i) {
+  const uint32_t v = p.key32[i];
+  return p.float_keys ? float_key(v) : v;
+}
+
 __device__ __forceinline__ unsigned long long make_key(const SelParams& p, long long i) {
-  return ((unsigned long long)p.key32[i] << p.ibits) | (unsigned long long)(p.n - 1 - i);
+  return ((unsigned long long)key32_at(p, i) << p.ibits) | (unsigned long long)(p.n - 1 - i);
 }
 
 __device__ void write_record(const SelParams& p, int slot, unsigned long long key) {
@@ -175,13 +191,14 @@ __global__ void __launch_bounds__(ST, 1) k4_select_kernel(const SelParams p) {
       }
     }
   } else {
-    // improving chain: i is kept iff key32[i] > max(key32[0..i)) and key32[i] > 0 (best_LCP_ starts at 0,
-    // strict '>' at match4pcsBase.cc:1891).  Contiguous segment per CTA.
+    // improving chain: i is kept iff key32[i] > max(key32[0..i)) and score i > 0 (best_LCP_ starts at 0, strict '>' at
+    // match4pcsBase.cc:1891: a score <= 0 never enters, a later positive one still does).  Contiguous segment per CTA.
+    const uint32_t floor = p.float_keys ? FLOAT_KEY_ZERO : 0u;
     const long long seg = (p.n + gridDim.x - 1) / gridDim.x;
     const long long s0 = min(p.n, seg * blockIdx.x), s1 = min(p.n, s0 + seg);
     uint32_t* s_max = s_hist;     // reuse
     uint32_t mx = 0;
-    for (long long i = s0 + threadIdx.x; i < s1; i += ST) mx = max(mx, p.key32[i]);
+    for (long long i = s0 + threadIdx.x; i < s1; i += ST) mx = max(mx, key32_at(p, i));
     mx = __reduce_max_sync(0xffffffffu, mx);
     if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = mx;
     __syncthreads();
@@ -196,7 +213,7 @@ __global__ void __launch_bounds__(ST, 1) k4_select_kernel(const SelParams p) {
     // inside the segment: chunks of ST elements, block-wide exclusive max-scan per chunk
     for (long long c0 = s0; c0 < s1; c0 += ST) {
       long long i = c0 + threadIdx.x;
-      uint32_t v = i < s1 ? p.key32[i] : 0u;
+      uint32_t v = i < s1 ? key32_at(p, i) : 0u;
       uint32_t incl = v;
 #pragma unroll
       for (int o = 1; o < 32; o <<= 1) { uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((threadIdx.x & 31) >= o) incl = max(incl, t); }
@@ -207,7 +224,7 @@ __global__ void __launch_bounds__(ST, 1) k4_select_kernel(const SelParams p) {
       __syncthreads();
       uint32_t before = run, chunk = 0;
       for (int w = 0; w < ST / 32; ++w) { uint32_t t = s_max[w]; if (w < (int)(threadIdx.x >> 5)) before = max(before, t); chunk = max(chunk, t); }
-      before = max(before, excl);
+      before = max(max(before, excl), floor);
       if (i < s1 && v > before) {
         unsigned pos = atomicAdd(p.n_cand, 1u);
         if (pos < KMAX) p.cand[pos] = make_key(p, i);
@@ -249,7 +266,7 @@ int run_select(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, pgp_
   if (b.mode == PGP_LCP_COUNT) { p.key32 = b.counts; p.kbits = bits_for((unsigned long long)m.nv); }
   else {
     if (!b.scores) return pgp_fail(ctx, PGP_E_NO_SCORES, "weighted selection needs the score array");
-    p.key32 = reinterpret_cast<const uint32_t*>(b.scores); p.kbits = 32;
+    p.key32 = reinterpret_cast<const uint32_t*>(b.scores); p.kbits = 32; p.float_keys = true;
   }
   (void)binary_weight;
   if (p.ibits + p.kbits > 63) return pgp_fail(ctx, PGP_E_INVALID, "batch too large for a 64-bit selection key");

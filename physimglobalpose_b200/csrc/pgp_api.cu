@@ -193,6 +193,10 @@ int pgp_set_scene_priors(pgp_ctx* ctx, const float* prior) {
   Scene& s = ctx->scene;
   if (!s.ready) return pgp_fail(ctx, PGP_E_NO_SCENE, "pgp_set_scene first");
   if (!prior) return pgp_fail(ctx, PGP_E_INVALID, "null priors");
+  // Any finite value is a valid prior, negative ones included (the reference does not restrict orig_probabilities_, and the ordered
+  // weighted sum handles them exactly).  A NaN or an infinity would make scores that have no order, so it is refused here.
+  for (int i = 0; i < s.n; ++i)
+    if (!std::isfinite(prior[i])) return pgp_fail(ctx, PGP_E_INVALID, "prior %d is not finite (%g)", i, (double)prior[i]);
   PGP_CUDA(ctx, cudaMemcpyAsync(s.prior.p, prior, (size_t)s.n * 4, cudaMemcpyHostToDevice, ctx->stream));
   return k1_refresh_sorted_priors(ctx);
 }
@@ -602,6 +606,7 @@ int pgp_topk_dev(pgp_ctx* ctx, int obj, int k, int64_t index_base, pgp_hyp* out_
   CHECK_CTX(ctx);
   if (ctx->last.obj != obj || ctx->last.n <= 0) return pgp_fail(ctx, PGP_E_NO_SCORES, "no scored batch for object %d", obj);
   if (k <= 0 || !out_dev) return pgp_fail(ctx, PGP_E_INVALID, "bad k / output");
+  if (index_base == PGP_INDEX_AUTO) index_base = 0;     // a local selection, like pgp_topk without a communicator
   return k4_topk_dev(ctx, ctx->last, k, index_base, out_dev);
 }
 
@@ -614,7 +619,13 @@ int pgp_improving_chain(pgp_ctx* ctx, int obj, int64_t index_base, pgp_hyp* out,
   int n_out = 0;
   int rc = k4_chain(ctx, ctx->last, index_base, out, cap, &n_out);
   if (rc) return rc;
-  if (n_out > cap) return pgp_fail(ctx, PGP_E_CAPACITY, "improving chain has %d elements, capacity %d (the last %d were written)", n_out, cap, cap);
+  if (n_out > cap) {
+    // up to 4096 candidates the kernel sorts the whole chain and writes its last cap elements; beyond that the compaction kept an
+    // arbitrary subset (in atomic order), so nothing written can be used
+    if (n_out > K4_MAX_K)
+      return pgp_fail(ctx, PGP_E_CAPACITY, "improving chain has %d elements, more than %d: the output is unusable", n_out, K4_MAX_K);
+    return pgp_fail(ctx, PGP_E_CAPACITY, "improving chain has %d elements, capacity %d (the last %d were written)", n_out, cap, cap);
+  }
   return n_out;
 }
 

@@ -176,7 +176,7 @@ int find_free_slot(Comm* c) {
 }
 
 int check_batch(pgp_ctx* ctx, Comm* c, int obj, int k) {
-  if (k <= 0 || k > 4096) return pgp_fail(ctx, PGP_E_INVALID, "k = %d outside 1..4096", k);
+  if (k <= 0 || k > K4_MAX_K) return pgp_fail(ctx, PGP_E_INVALID, "k = %d outside 1..%d", k, K4_MAX_K);
   if (obj < 0 || obj >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "object slot %d out of range", obj);
   if (c->world == 1 && (ctx->last.obj != obj || ctx->last.n <= 0)) return pgp_fail(ctx, PGP_E_NO_SCORES, "no scored batch for object %d", obj);
   return PGP_OK;

@@ -124,7 +124,7 @@ struct Model {
   // generated hypotheses (K2)
   DevBuf gen_T, gen_counts, gen_scores;
   int64_t n_gen = 0;
-  int64_t gen_index_base = 0;   // global index of the first generated hypothesis (bases sharded over ranks: pgp_comm_sync_generated); -1 = not known yet
+  int64_t gen_index_base = -1;  // global index of the first generated hypothesis (bases sharded over ranks: pgp_comm_sync_generated); -1 = not known yet
   int n_gen_bases = 0;
   bool gen_scored = false;
   // PPF map of the SEARCH cloud (operMode 1 / StoCS): sorted packed keys -> pair lists, + presence bitset
@@ -215,6 +215,7 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
 bool k3_streams_upload(pgp_ctx* ctx, int mode);
 int k3_nearest(pgp_ctx* ctx, const Model& m, const float* T_dev, int32_t* idx_dev, int gate);
 // k4_select.cu
+constexpr int K4_MAX_K = 4096;   // largest k of a selection, and the most chain candidates one launch can sort
 int k4_topk(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, pgp_hyp* out_host, int* n_out);
 int k4_topk_dev(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, pgp_hyp* out_dev);
 int k4_chain(pgp_ctx* ctx, const LastBatch& b, int64_t index_base, pgp_hyp* out_host, int cap, int* n_out);

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 from physimglobalpose_b200 import _lib, sharding, synth
-from physimglobalpose_b200.engine import HYP_DTYPE, PoseEngine, topk_merge
+from physimglobalpose_b200.engine import HYP_DTYPE, PoseEngine, exchange_merge, topk_merge, wire_block
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -69,24 +69,70 @@ def _records(rng, n, base):
     return r
 
 
+def _signed_records(rng, n, base):
+    """Scores with negative values, -0.0 and +0.0 (priors may be negative): many ties, zeros of both signs tie."""
+    r = _records(rng, n, base)
+    r["score"] = rng.choice(np.array([-1.5, -0.25, -1e-30, -0.0, 0.0, 1e-30, 0.25, 1.5], np.float32), size=n)
+    return r
+
+
+def _fp32_order(rec):
+    """(score desc, index asc) with scores compared as fp32 values: -0 == +0, the index decides."""
+    s = rec["score"].astype(np.float64)
+    s[s == 0] = 0.0
+    return np.lexsort((rec["index"], -s))
+
+
 def test_topk_merge_is_independent_of_the_sharding(lib):
-    rng = np.random.default_rng(0)
-    allrec = _records(rng, 4000, 0)
-    order = np.lexsort((allrec["index"], -allrec["score"]))
-    want = allrec[order][:64]
-    for world in (1, 2, 4, 8):
-        lists = []
-        for r in range(world):
-            lo, hi = sharding.shard_range(len(allrec), r, world)
-            part = allrec[lo:hi]
-            o = np.lexsort((part["index"], -part["score"]))
-            lists.append(part[o][:64])
-        got = topk_merge(lists, 64)
-        assert np.array_equal(got["index"], want["index"]) and np.array_equal(got["score"], want["score"])
-        assert np.array_equal(got["T"], want["T"])
+    for make in (_records, _signed_records):
+        rng = np.random.default_rng(0)
+        allrec = make(rng, 4000, 0)
+        want = allrec[_fp32_order(allrec)][:64]
+        for world in (1, 2, 4, 8):
+            lists = []
+            for r in range(world):
+                lo, hi = sharding.shard_range(len(allrec), r, world)
+                part = allrec[lo:hi]
+                lists.append(part[_fp32_order(part)][:64])
+            got = topk_merge(lists, 64)
+            assert got.tobytes() == want.tobytes(), make.__name__
     # short lists are padded with index = -1 and skipped
     got = topk_merge([allrec[:3], allrec[3:5]], 64)
     assert len(got) == 5
+
+
+def test_exchange_merge_orders_signed_scores_like_the_serial_scan(lib):
+    """WEIGHTED records with negative, -0.0 and +0.0 scores: the merged top-k is the fp32 order over the union, and the merged
+    chain is the serial scan over the concatenation (best starts at 0, strict '>': a score <= 0 never enters)."""
+    rng = np.random.default_rng(4)
+    allrec = _signed_records(rng, 3000, 0)
+    allrec["index"] = np.arange(len(allrec))                              # generation order: the chain scans it
+    allrec["score"][:40] = -np.arange(1, 41, dtype=np.float32)          # a negative prefix: a positive score later still enters
+    rise = np.sort(rng.choice(np.arange(40, 3000), 30, replace=False))
+    allrec["score"][rise] = np.arange(2, 32, dtype=np.float32)
+    want = allrec[_fp32_order(allrec)][:64]
+    best, keep = np.float32(0), []
+    for i, s in enumerate(allrec["score"]):
+        if s > best:
+            keep.append(i)
+            best = s
+    want_chain = allrec[keep]
+    assert len(want_chain) >= 30 and np.all(want_chain["score"] > 0)
+    for world in (1, 2, 3, 8):
+        blocks, chains = [], []
+        for r in range(world):
+            lo, hi = sharding.shard_range(len(allrec), r, world)
+            part = allrec[lo:hi].copy()
+            part["index"] -= lo                                              # shard-local indices: auto_base numbers them
+            blocks.append(wire_block(part[_fp32_order(part)][:64], hi - lo, 64))
+            b, ch = np.float32(0), []
+            for i, s in enumerate(part["score"]):
+                if s > b:
+                    ch.append(i)
+                    b = s
+            chains.append(wire_block(part[ch], hi - lo, 255))
+        assert exchange_merge(np.concatenate(blocks), world, 64, auto_base=True).tobytes() == want.tobytes()
+        assert exchange_merge(np.concatenate(chains), world, 255, kind=1, mode="weighted", auto_base=True).tobytes() == want_chain.tobytes()
 
 
 def test_synth_pose_round_trip():
