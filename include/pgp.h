@@ -345,8 +345,17 @@ PGP_API int pgp_host_max_eigvec4(const double* N16_rowmajor, double* q4);
  * UCTState.cpp:121-204) / utilities::performTrICP (PPE/src/misc/utilities.cpp:651-680) ->
  * pcl::recognition::TrimmedICP::align.  poses: k x 16 doubles, row-major camera-frame
  * model->scene poses, refined in place.  seg_xyz: ns x 3 camera frame.  trim: kept fraction
- * (0.5 at the MCTS call site), ratio: new-to-old energy ratio (0.99), max_iter: safety cap.
- * iters_out / energy_out (k each) may be NULL. */
+ * (0.5 at the MCTS call site), ratio: new-to-old energy ratio (0.99), max_iter: safety cap
+ * (values below 1 act as 1).  iters_out / energy_out (k each) may be NULL.
+ * PGP_E_INVALID, before anything runs and with the poses untouched: trim or ratio not > 0 (NaN
+ * included), a NaN or infinite segment coordinate or pose entry.  k = 0 is a no-op.
+ * n_keep = min(ns, (int)|trim * ns|) in fp32; n_keep < 3 leaves every pose as given with
+ * iters_out = 0, energy_out = 0.  Ties at the trim threshold are kept in the Morton order of the
+ * segment over its bounding cube.  A finite pose whose squared distances overflow fp32 (e.g. a
+ * translation of 1e20): every such query takes model point 0 at FLT_MAX; if the trimmed energy is
+ * then not finite the pose stops after that iteration, is returned exactly as given, and reports
+ * energy_out = +Inf (iters_out = 1 when it overflows from the start).  Other poses of the batch are
+ * unaffected: each pose's result does not depend on the rest of the batch. */
 PGP_API int pgp_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, double* poses16_host, int k,
                       float trim, float ratio, int max_iter, int* iters_out, float* energy_out);
 
@@ -359,7 +368,9 @@ PGP_API int pgp_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, 
 PGP_API int pgp_remove_explained(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, const double* placed_poses16, int n_placed,
                                  float threshold, uint8_t* explained);
 /* One MCTS expansion's refinement (UCTState::performTrICP, :121-204) for k candidate poses of object `obj` at once:
- * explained-point removal, then pgp_tricp on the unexplained segment.  n_unexplained may be NULL. */
+ * explained-point removal, then pgp_tricp on the unexplained segment.  n_unexplained may be NULL.
+ * The input checks of pgp_tricp apply (k = 0 is refused here); when fewer than 3 points remain the poses stay as given
+ * with iters_out = 0, energy_out = 0. */
 PGP_API int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, const double* placed_poses16, int n_placed,
                            float threshold, double* poses16_host, int k, float trim, float ratio, int max_iter, int* iters_out,
                            float* energy_out, int* n_unexplained);

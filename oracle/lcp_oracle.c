@@ -624,8 +624,14 @@ int lo_tricp(const float* src, int ns, const float* tgt, int nt, float* T, float
       for (int r = 0; r < 3; ++r) q[r] = T[4 * r] * p[0] + T[4 * r + 1] * p[1] + T[4 * r + 2] * p[2] + T[4 * r + 3];
       /* exact unbounded 1-NN: restricted query with an infinite radius */
       int32_t id = lo_tree_closest_within(&tree, q, FLT_MAX);
-      float dx = q[0] - tgt[3 * id], dy = q[1] - tgt[3 * id + 1], dz = q[2] - tgt[3 * id + 2];
-      corr[i].d2 = dx * dx + dy * dy + dz * dz;
+      if (id >= 0) {
+        float dx = q[0] - tgt[3 * id], dy = q[1] - tgt[3 * id + 1], dz = q[2] - tgt[3 * id + 2];
+        corr[i].d2 = dx * dx + dy * dy + dz * dz;
+      } else {
+        /* no squared distance below FLT_MAX (NaN or overflowing query): target 0 at FLT_MAX, as K5 */
+        id = 0;
+        corr[i].d2 = FLT_MAX;
+      }
       corr[i].src = i; corr[i].tgt = id;
     }
     qsort(corr, (size_t)ns, sizeof(lo_corr), lo_corr_cmp);
@@ -636,6 +642,7 @@ int lo_tricp(const float* src, int ns, const float* tgt, int nt, float* T, float
       for (int a = 0; a < 3; ++a) { cs[a] += src[3 * corr[k].src + a]; cg[a] += tgt[3 * corr[k].tgt + a]; }
     }
     energy = (float)e;
+    if (!(energy <= FLT_MAX)) { ++it; break; }     /* a kept squared distance overflowed: T stays, as K5 */
     for (int a = 0; a < 3; ++a) { cs[a] /= n_keep; cg[a] /= n_keep; }
     double H[3][3] = {{0}};
     for (int k = 0; k < n_keep; ++k)

@@ -61,6 +61,11 @@ __global__ void k5_tgrid_scatter(const float4* __restrict__ pts, int n, const ui
 // search stops once best <= (r g)^2 -- or, with a finite cap2, once (r g)^2 >= cap2: then every unvisited point is farther than
 // sqrt(cap2) and the caller only needs to know THAT (the trimmed set keeps the n_keep smallest distances; a point beyond the
 // current trim radius is dropped whatever its exact distance).  A result <= cap2 is always the exact nearest neighbour.
+// In fp32 the cell coordinate fl(fl(x - lo) * inv_g) of a point or query is off by up to 3 * 2^-24 * u cells (u <= rmax inside the
+// grid; a clamped query is farther out than its cell says), so a point just across a face can sit (r - 1 - 6 * 2^-24 * rmax) g
+// from the query: the bound subtracts that (as 4 FLT_EPSILON * rmax cells), and the 1e-6 factor covers the rounding of d2.
+// The returned id is always in [0, nt): a query whose squared distances are all NaN or overflow (none below FLT_MAX) gets id 0
+// with d2 = FLT_MAX, as the capped branch reports a point beyond the cap.
 __device__ __forceinline__ void nn_search(const TricpParams& p, float qx, float qy, float qz, float cap2, float& best, int& best_id) {
   const TGrid& tg = p.tg;
   const int cx = min(max((int)floorf((qx - tg.lo[0]) * tg.inv_g), 0), tg.dim[0] - 1);
@@ -68,9 +73,10 @@ __device__ __forceinline__ void nn_search(const TricpParams& p, float qx, float 
   const int cz = min(max((int)floorf((qz - tg.lo[2]) * tg.inv_g), 0), tg.dim[2] - 1);
   best = FLT_MAX; best_id = -1;
   const int rmax = max(tg.dim[0], max(tg.dim[1], tg.dim[2]));
+  const float slack = 4.0f * FLT_EPSILON * (float)rmax * tg.g;
   for (int r = 0; r <= rmax; ++r) {
     if (r > 0) {
-      const float bound = (float)(r - 1) * tg.g;     // ring r-1 is complete: unvisited points are >= (r-1) g away
+      const float bound = fmaxf((float)(r - 1) * tg.g - slack, 0.f);   // ring r-1 is complete: unvisited points are >= (r-1) g away
       const float b2 = bound * bound * 0.999999f;
       if (best_id >= 0 && best <= b2) break;
       if (b2 >= cap2) { if (!(best <= cap2)) { best = FLT_MAX; best_id = 0; } break; }
@@ -108,6 +114,7 @@ __device__ __forceinline__ void nn_search(const TricpParams& p, float qx, float 
         }
       }
   }
+  if (best_id < 0) best_id = 0;
 }
 
 __device__ void jacobi4(double A[4][4], double V[4][4]) {
@@ -350,9 +357,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
       for (int k = 0; k < 16; ++k) S[k] = cr ? r_part[k] + s_part[k] : s_part[k] + r_part[k];      // CTA 0's half + CTA 1's half, in both
       old_energy = energy;
       energy = (float)S[0];
-      float Tn[12];
-      rigid_fit((double)p.n_keep, S + 1, Tn);
-      for (int k = 0; k < 12; ++k) sT[k] = Tn[k];
+      if (energy <= FLT_MAX) {                     // a kept squared distance overflowed: no fit, and the ratio test below stops
+        float Tn[12];
+        rigid_fit((double)p.n_keep, S + 1, Tn);
+        for (int k = 0; k < 12; ++k) sT[k] = Tn[k];
+      }
       ++it;
       s_cont = ((energy / old_energy) < p.ratio && it < p.max_iter) ? 1 : 0;
     }
@@ -438,7 +447,8 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   TScratch& ts = tscratch_of(ctx);
   int rc = build_target_grid(ctx, m);
   if (rc) return rc;
-  const int n_keep = std::min(ns, (int)fabsf(trim * (float)ns));      // abs(numPoints) on a float, UCTState.cpp:181,194
+  const float keep_f = fabsf(trim * (float)ns);                          // abs(numPoints) on a float, UCTState.cpp:181,194
+  const int n_keep = keep_f < 2147483648.f ? std::min(ns, (int)keep_f) : ns;
   if (n_keep < 3) {
     for (int i = 0; i < k; ++i) { if (iters_out) iters_out[i] = 0; if (energy_out) energy_out[i] = 0.f; }
     return PGP_OK;
@@ -497,11 +507,13 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   PGP_CUDA(ctx, cudaMemcpyAsync(en.data(), ts.energy.p, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream));
   PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   for (int i = 0; i < k; ++i) {
-    double M[16] = {0}, inv[16];
-    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) M[4 * r + c] = (double)T[12 * (size_t)i + 4 * r + c];
-    M[15] = 1;
-    invert_pose(M, inv);                                                 // pose = inverse(tform), UCTState.cpp:195-203
-    memcpy(poses16_host + 16 * i, inv, sizeof(inv));
+    if (en[i] <= FLT_MAX) {                                              // (non-finite energy: the pose stays as it was given)
+      double M[16] = {0}, inv[16];
+      for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) M[4 * r + c] = (double)T[12 * (size_t)i + 4 * r + c];
+      M[15] = 1;
+      invert_pose(M, inv);                                               // pose = inverse(tform), UCTState.cpp:195-203
+      memcpy(poses16_host + 16 * i, inv, sizeof(inv));
+    }
     if (iters_out) iters_out[i] = it[i];
     if (energy_out) energy_out[i] = en[i];
   }

@@ -785,11 +785,20 @@ int pgp_get_bases(pgp_ctx* ctx, int obj, int32_t* ids, float* inv, uint8_t* ok, 
   return rc ? rc : n;
 }
 
+// trimmed ICP inputs: every segment coordinate and every pose entry finite
+static bool tricp_inputs_finite(const float* seg, int ns, const double* poses, int k) {
+  for (size_t i = 0; i < (size_t)ns * 3; ++i) if (!std::isfinite(seg[i])) return false;
+  for (size_t i = 0; i < (size_t)k * 16; ++i) if (!std::isfinite(poses[i])) return false;
+  return true;
+}
+
 int pgp_tricp(pgp_ctx* ctx, int obj, const float* seg, int ns, double* poses, int k, float trim, float ratio, int max_iter, int* iters, float* energy) {
   CHECK_CTX(ctx);
   Model* m = get_model(ctx, obj);
   if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "no model in slot %d", obj);
   if (!seg || ns <= 0 || !poses || k < 0) return pgp_fail(ctx, PGP_E_INVALID, "bad argument");
+  if (!(trim > 0.f) || !(ratio > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp: trim and ratio must be > 0");
+  if (!tricp_inputs_finite(seg, ns, poses, k)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp: non-finite segment point or pose");
   if (k == 0) return PGP_OK;
   return k5_tricp(ctx, *m, seg, ns, poses, k, trim, ratio, max_iter, iters, energy);
 }
@@ -814,6 +823,7 @@ int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg, int ns, const double
   if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "no model in slot %d", obj);
   if (!seg || ns <= 0 || !poses || k <= 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_mcts_tricp: empty input");
   if (!(trim > 0.f) || !(ratio > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_mcts_tricp: trim and ratio must be > 0");
+  if (!tricp_inputs_finite(seg, ns, poses, k)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_mcts_tricp: non-finite segment point or pose");
   std::vector<uint8_t> flag((size_t)ns, 0);
   int kept = ns;
   if (n_placed > 0) {
