@@ -393,6 +393,58 @@ PGP_API int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const u
                                 const float* K9, float leaf, float normal_radius, float outlier_radius, int min_neighbors,
                                 float* xyz_out, float* nrm_out, int cap, int* n_valid_pixels);
 
+/* ---------------------------------------------------------------- K8: rendered-depth cost --- */
+
+/* The render + compare step of an MCTS node evaluation (UCTState::render followed by UCTState::computeCost,
+ * PPE/src/hypothesis_verification/mcts/UCTState.cpp:93-116; renderer depth_sim/src/renderScene.cpp:36-84).  RESTATED, PARITY
+ * UNPINNED: the reference renders with OpenGL (a pcl::simulation fork) and the body of computeCost is not available, so K8 has
+ * its own exact contract and returns exact per-object pixel counts from which a per-pixel depth-agreement cost is composed on
+ * the host.  The contract, in order (oracle/render_port.py restates it line by line):
+ *  1. pose -> fp32 3x4 (as K6); camera-frame vertex (X, Y, Z) per row ((m0 x + m1 y) + m2 z) + m3, unfused fp32.
+ *  2. sx = ((fx X) / Z) + cx, sy = ((fy Y) / Z) + cy, fp32, each operation rounded.  Pixel (row r, col c) samples the point
+ *     (c, r), the convention of K7's back-projection.
+ *  3. vertices snap to 1/256 px: rint(s * 256) to int64, ties to even.  A triangle is dropped whole (no clipping) when a vertex has
+ *     a non-finite X, Y or Z, Z <= 0.1f (fp32 compare), or |sx| or |sy| > 2^20 px (or NaN), or when its snapped area is 0.  No
+ *     back-face culling.
+ *  4. edge function E(a, b, p) = (b.x - a.x)(p.y - a.y) - (b.y - a.y)(p.x - a.x) in int64 on snapped coordinates (exact).  The
+ *     triangle (v0, v1, v2) is reoriented (v1 <-> v2) so that its area A = E(v0, v1, v2) > 0; E_0 = E(v1, v2, p),
+ *     E_1 = E(v2, v0, p), E_2 = E(v0, v1, p).  p is covered when every E_i > 0, or == 0 on an edge a -> b that owns it:
+ *     dy < 0, or dy == 0 && dx > 0 (top-left rule; a shared edge or vertex covers each sample exactly once).
+ *  5. depth = (float)((double)A / (((double)E_0 iz_0 + (double)E_1 iz_1) + (double)E_2 iz_2)), iz_i = 1.0 / (double)Z_i, double,
+ *     unfused, A = E_0 + E_1 + E_2 exact in int64.
+ *  6. per pixel the minimum of the 64-bit key (float_bits(depth) << 32) | slot wins (slot = position in the state; equal depths go
+ *     to the smaller slot).  Independent of triangle order.
+ *  7. per front pixel of a slot: rendered += 1.  Observed o = K7's decode; if (double)o > 0.1 && (double)o < 2.0 exactly one of
+ *     agree (fabsf(r - o) <= tau), in_front (o - r > tau: the object would hide a surface the camera sees), behind (r - o > tau:
+ *     the object is occluded) += 1.  on_segment += 1 where class_mask == the mesh's class_id.  Pixels without a valid observation:
+ *     rendered - agree - in_front - behind.
+ * Image sides are limited to 1 .. 16384 px, meshes to 2^24 vertices and 2^24 triangles. */
+
+/* Triangle mesh of object slot `obj` (model frame: the frame pgp_tricp's poses map from).  vert_xyz: nv x 3, tri3: nt x 3 vertex
+ * indices, class_id: the object's label in the class mask (-1: none).  Independent of pgp_set_model.  Replaces a previous mesh.
+ * PGP_E_INVALID: nv < 3, nt < 1, a non-finite vertex, an index outside [0, nv). */
+PGP_API int pgp_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, const int32_t* tri3, int nt, int class_id);
+
+/* Observed frame: depth_raw as stored in frame-*.depth.png (decoded exactly as pgp_prepare_segment does), class_mask (NULL: none;
+ * on_segment then stays 0), K9 row-major intrinsics (fx = K[0], fy = K[4], cx = K[2], cy = K[5], as K7).  class_pixels_out
+ * (256 entries, NULL allowed): pixels of each label with valid depth (all 0 without a mask).  PGP_E_INVALID: rows or cols
+ * outside 1 .. 16384, a non-finite K9 entry, fx <= 0 or fy <= 0. */
+PGP_API int pgp_set_depth_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols,
+                                      const float* K9, int64_t* class_pixels_out);
+
+/* One state rendered in full: depth_out rows x cols fp32 metres (0 = nothing), slot_out rows x cols (-1 = nothing; NULL allowed). */
+PGP_API int pgp_render_depth(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n, float* depth_out, int32_t* slot_out);
+
+typedef struct pgp_depth_counts { int32_t rendered, agree, in_front, behind, on_segment; } pgp_depth_counts;
+/* n_states states in CSR form: state s places obj_ids[state_offsets[s] .. state_offsets[s+1]) at the matching poses16 (row-major 4x4
+ * model->camera doubles).  out: one record per placed object (state_offsets[n_states] records), counted over the pixels where that
+ * object is the front surface.  Each state's records equal that state evaluated alone.
+ * PGP_E_INVALID before anything runs, outputs untouched: no observation set, state_offsets not non-decreasing from 0, more than
+ * PGP_MAX_OBJECTS objects in a state, an object id outside [0, PGP_MAX_OBJECTS), a non-finite pose entry, tau < 0 or not finite.
+ * PGP_E_NO_MODEL: an object without a mesh.  n_states = 0 and empty states are valid. */
+PGP_API int pgp_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16,
+                           float tau, pgp_depth_counts* out);
+
 #define PGP_MAX_OBJECTS 64
 #define PGP_MAX_CELLS (1ll << 29)
 

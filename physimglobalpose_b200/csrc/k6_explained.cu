@@ -66,8 +66,7 @@ int k6_remove_explained(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int n
   cudaStream_t st = ctx->stream;
   std::vector<float> seg4((size_t)ns * 4, 0.f), T((size_t)n_placed * 12);
   for (int i = 0; i < ns; ++i) for (int c = 0; c < 3; ++c) seg4[4 * (size_t)i + c] = seg_xyz_host[3 * i + c];
-  for (int k = 0; k < n_placed; ++k)                       // utilities::convertToMatrix: Isometry3d -> Matrix4f
-    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) T[12 * (size_t)k + 4 * r + c] = (float)placed16_host[16 * k + 4 * r + c];
+  for (int k = 0; k < n_placed; ++k) pose16_to_f32x12(placed16_host + 16 * (size_t)k, &T[12 * (size_t)k]);
   const int ne = m.nv * n_placed;
   PGP_CUDA(ctx, sc.seg.reserve((size_t)ns * 16));
   PGP_CUDA(ctx, sc.expl.reserve((size_t)ne * 16));

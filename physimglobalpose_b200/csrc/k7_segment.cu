@@ -22,17 +22,12 @@ namespace {
 
 constexpr int T = 256;
 
-__device__ __forceinline__ float decode_depth(uint16_t raw) {
-  const uint16_t d = (uint16_t)((raw << 13) | (raw >> 3));
-  return __fdiv_rn((float)d, 10000.0f);
-}
-
 // pass 1: validity flag per pixel; pass 2 (after the scan): emit points in row-major pixel order
 __global__ void k7_flags(const uint16_t* __restrict__ depth, const uint8_t* __restrict__ mask, int n, int cls, uint32_t* __restrict__ flag) {
   const int i = blockIdx.x * T + threadIdx.x;
   if (i >= n) return;
   const float d = mask[i] == cls ? decode_depth(depth[i]) : 0.f;
-  flag[i] = ((double)d > 0.1 && (double)d < 2.0) ? 1u : 0u;          // depth > 0.1 && depth < 2.0 compares a float with double literals
+  flag[i] = depth_valid(d) ? 1u : 0u;
 }
 __global__ void k7_emit(const uint16_t* __restrict__ depth, const uint8_t* __restrict__ mask, int n, int cols, int cls, float fx, float fy, float cx,
                         float cy, const uint32_t* __restrict__ off, float4* __restrict__ pts, int* __restrict__ ijk_min, float leaf) {

@@ -125,6 +125,7 @@ void pgp_destroy(pgp_ctx* ctx) {
   k5_release(ctx);
   k6_release(ctx);
   k7_release(ctx);
+  k8_release(ctx);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   cudaStreamDestroy(ctx->own_stream);
   cudaStreamDestroy(ctx->copy_stream);
@@ -853,4 +854,71 @@ int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* 
   int rc = k7_prepare_segment(ctx, depth_raw, class_mask, rows, cols, class_id, K9, leaf, normal_radius, outlier_radius, min_neighbors, xyz_out, nrm_out,
                               cap, &n, n_valid_pixels);
   return rc ? rc : n;
+}
+
+// ---------------------------------------------------------------- K8: rendered-depth cost
+#define K8_MAX_SIDE 16384          // image side: keeps every edge function below 2^59 and a pixel box in int16
+#define K8_MAX_MESH (1 << 24)      // vertices / triangles of one mesh
+
+int pgp_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, const int32_t* tri3, int nt, int class_id) {
+  CHECK_CTX(ctx);
+  if (obj < 0 || obj >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_mesh: object slot %d out of range", obj);
+  if (!vert_xyz || !tri3 || nv < 3 || nt < 1 || nv > K8_MAX_MESH || nt > K8_MAX_MESH)
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_mesh: need 3 .. 2^24 vertices and 1 .. 2^24 triangles (nv %d, nt %d)", nv, nt);
+  for (size_t i = 0; i < (size_t)nv * 3; ++i)
+    if (!std::isfinite(vert_xyz[i])) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_mesh: vertex %zu is not finite", i / 3);
+  for (size_t i = 0; i < (size_t)nt * 3; ++i)
+    if (tri3[i] < 0 || tri3[i] >= nv) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_mesh: triangle %zu indexes vertex %d of %d", i / 3, tri3[i], nv);
+  return k8_set_mesh(ctx, obj, vert_xyz, nv, tri3, nt, class_id);
+}
+
+int pgp_set_depth_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, const float* K9,
+                              int64_t* class_pixels_out) {
+  CHECK_CTX(ctx);
+  if (!depth_raw || !K9 || rows < 1 || cols < 1 || rows > K8_MAX_SIDE || cols > K8_MAX_SIDE)
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: need a depth frame of 1 .. %d px per side and K9", K8_MAX_SIDE);
+  for (int i = 0; i < 9; ++i)
+    if (!std::isfinite(K9[i])) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: K[%d] is not finite", i);
+  if (!(K9[0] > 0.f) || !(K9[4] > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: fx and fy must be > 0");
+  return k8_set_observation(ctx, depth_raw, class_mask, rows, cols, K9, class_pixels_out);
+}
+
+// the checks shared by the two depth calls: objects with meshes, finite poses
+static int check_placed(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int64_t n) {
+  for (int64_t i = 0; i < n; ++i)
+    if (obj_ids[i] < 0 || obj_ids[i] >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "object id %d out of range", obj_ids[i]);
+  for (int64_t i = 0; i < n * 16; ++i)
+    if (!std::isfinite(poses16[i])) return pgp_fail(ctx, PGP_E_INVALID, "pose %lld is not finite", (long long)(i / 16));
+  for (int64_t i = 0; i < n; ++i)
+    if (!k8_has_mesh(ctx, obj_ids[i])) return pgp_fail(ctx, PGP_E_NO_MODEL, "no mesh in slot %d (pgp_set_mesh)", obj_ids[i]);
+  return PGP_OK;
+}
+
+int pgp_render_depth(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n, float* depth_out, int32_t* slot_out) {
+  CHECK_CTX(ctx);
+  if (!k8_has_observation(ctx)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_render_depth: pgp_set_depth_observation first");
+  if (n < 0 || n > PGP_MAX_OBJECTS || !depth_out || (n > 0 && (!obj_ids || !poses16)))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_render_depth: bad argument (n = %d, at most %d objects)", n, PGP_MAX_OBJECTS);
+  int rc = check_placed(ctx, obj_ids, poses16, n);
+  return rc ? rc : k8_render(ctx, obj_ids, poses16, n, depth_out, slot_out);
+}
+
+int pgp_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16, float tau,
+                   pgp_depth_counts* out) {
+  CHECK_CTX(ctx);
+  if (!k8_has_observation(ctx)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: pgp_set_depth_observation first");
+  if (n_states < 0 || (n_states > 0 && !state_offsets)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: bad state list");
+  if (!std::isfinite(tau) || !(tau >= 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: tau must be finite and >= 0");
+  if (n_states == 0) return PGP_OK;
+  if (state_offsets[0] != 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state_offsets[0] must be 0");
+  for (int s = 0; s < n_states; ++s) {
+    const int64_t k = state_offsets[s + 1] - state_offsets[s];
+    if (k < 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state_offsets decrease at state %d", s);
+    if (k > PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state %d places %lld objects (at most %d)", s, (long long)k, PGP_MAX_OBJECTS);
+  }
+  const int64_t n = state_offsets[n_states];
+  if (n > INT32_MAX) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: more than 2^31 - 1 placed objects");
+  if (n > 0 && (!obj_ids || !poses16 || !out)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: null argument");
+  int rc = check_placed(ctx, obj_ids, poses16, n);
+  return rc ? rc : k8_depth_cost(ctx, state_offsets, n_states, obj_ids, poses16, tau, out);
 }

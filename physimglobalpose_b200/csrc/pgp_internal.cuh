@@ -182,6 +182,7 @@ struct pgp_ctx {
   void* k5_scratch = nullptr;              // k5_tricp.cu (k5_release)
   void* k6_scratch = nullptr;              // k6_explained.cu (k6_release)
   void* k7_scratch = nullptr;              // k7_segment.cu (k7_release)
+  void* k8_scratch = nullptr;              // k8_render.cu: meshes, observation, rasterizer scratch (k8_release)
   int k7_mls = 1;                          // segment preparation: 1 = MLS polynomial projection + normals (what the reference runs), 0 = PCA normals on the centroids
   int stream_upload = 1;  // pgp_score_lcp: overlap the batch upload with the scoring launch (0: upload first; use under profilers)
   int tail_split = 4;     // K3 fine kernel: model chunks per hypothesis in the last wave (1 = off)
@@ -263,9 +264,29 @@ __device__ __forceinline__ float dot3_tree(float a0, float a1, float a2, float b
 // cell coordinate of a centred coordinate; the SAME function bins scene points and queries, and
 // it is monotone, which is what the 27-cell completeness argument needs.
 __device__ __forceinline__ float cell_coord(float x, float lo, float inv_h) { return __fmul_rn(__fsub_rn(x, lo), inv_h); }
+// utilities::convertToMatrix (Isometry3d -> Matrix4f): the top 3x4 of a row-major 4x4 double pose, each entry rounded to fp32
+// (K6 placed poses, K8 rendered poses)
+inline void pose16_to_f32x12(const double* pose16, float* T12) {
+  for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) T12[4 * r + c] = (float)pose16[4 * r + c];
+}
+// utilities::readDepthImage (PPE/src/misc/utilities.cpp:47-61): ((d << 13) | (d >> 3)) as u16, / 10000 (K7 segments, K8 observations)
+__device__ __forceinline__ float decode_depth(uint16_t raw) {
+  const uint16_t d = (uint16_t)((raw << 13) | (raw >> 3));
+  return __fdiv_rn((float)d, 10000.0f);
+}
+// utilities::convert3dUnOrganizedRGB's depth > 0.1 && depth < 2.0: a float compared with double literals
+__device__ __forceinline__ bool depth_valid(float d) { return (double)d > 0.1 && (double)d < 2.0; }
 // k6_explained.cu
 int k6_remove_explained(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, const double* placed16_host, int n_placed, float threshold,
                         uint8_t* flags_host, int* n_unexplained);
 // k7_segment.cu
 int k7_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_host, const uint8_t* mask_host, int rows, int cols, int cls, const float* K9, float leaf,
                        float normal_r, float outlier_r, int min_nb, float* xyz_host, float* nrm_host, int cap, int* n_out, int* n_raw_out);
+// k8_render.cu (arguments checked by the C ABI in pgp_api.cu)
+int k8_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, const int32_t* tri3, int nt, int class_id);
+bool k8_has_mesh(pgp_ctx* ctx, int obj);
+bool k8_has_observation(pgp_ctx* ctx);
+int k8_set_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, const float* K9, int64_t* class_pixels_out);
+int k8_render(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n, float* depth_out, int32_t* slot_out);
+int k8_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16, float tau, pgp_depth_counts* out);
+void k8_release(pgp_ctx* ctx);

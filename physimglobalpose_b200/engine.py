@@ -425,6 +425,48 @@ class PoseEngine:
                                                       C.byref(nraw)))
         return xyz[:n].copy(), nrm[:n].copy(), nraw.value
 
+    # ------------------------------------------------------------------ K8
+    def set_mesh(self, obj: int, vert_xyz, tri3, class_id: int = -1):
+        """Triangle mesh of object slot `obj` in its model frame; class_id = its label in the class mask (-1: none)."""
+        v = _f32(vert_xyz, 3)
+        t = np.ascontiguousarray(tri3, np.int32).reshape(-1, 3)
+        self._check(self._lib.pgp_set_mesh(self._ctx, int(obj), _ptr(v), len(v), _ptr(t), len(t), int(class_id)))
+
+    def set_depth_observation(self, depth_raw_u16, class_mask_u8, K) -> np.ndarray:
+        """Observed frame (raw depth as stored, class mask or None, 3x3 intrinsics).  Returns the pixels of each label with valid depth."""
+        d = np.ascontiguousarray(depth_raw_u16, np.uint16)
+        assert d.ndim == 2
+        m = None if class_mask_u8 is None else np.ascontiguousarray(class_mask_u8, np.uint8)
+        assert m is None or m.shape == d.shape
+        K = _f32(K).reshape(9)
+        hist = np.zeros(256, np.int64)
+        self._check(self._lib.pgp_set_depth_observation(self._ctx, _ptr(d), _ptr(m), d.shape[0], d.shape[1], _ptr(K), _ptr(hist)))
+        self._frame = d.shape
+        return hist
+
+    def render_depth(self, obj_ids, poses44):
+        """One state rendered in full: (depth rows x cols fp32 metres, 0 = nothing; slot rows x cols int32, -1 = nothing)."""
+        ids = np.ascontiguousarray(obj_ids, np.int32).reshape(-1)
+        P = np.ascontiguousarray(poses44, np.float64).reshape(-1, 16)
+        rows, cols = getattr(self, "_frame", (1, 1))
+        depth = np.zeros((rows, cols), np.float32)
+        slot = np.zeros((rows, cols), np.int32)
+        self._check(self._lib.pgp_render_depth(self._ctx, _ptr(ids), _ptr(P), len(ids), _ptr(depth), _ptr(slot)))
+        return depth, slot
+
+    def depth_cost(self, states, tau: float) -> np.ndarray:
+        """states: [(obj_ids, poses44), ...].  Returns (n_slots, 5) int32 {rendered, agree, in_front, behind, on_segment}, one row per
+        placed object in state order."""
+        ids = [np.asarray(o, np.int32).reshape(-1) for o, _ in states]
+        poses = [np.asarray(p, np.float64).reshape(-1, 16) for _, p in states]
+        offs = np.zeros(len(states) + 1, np.int64)
+        offs[1:] = np.cumsum([len(i) for i in ids])
+        flat_ids = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32), np.int32)
+        flat_P = np.ascontiguousarray(np.concatenate(poses) if poses else np.zeros((0, 16)), np.float64)
+        out = np.zeros((int(offs[-1]), 5), np.int32)
+        self._check(self._lib.pgp_depth_cost(self._ctx, _ptr(offs), len(states), _ptr(flat_ids), _ptr(flat_P), float(tau), _ptr(out)))
+        return out
+
 
 class PoseGroup:
     """One process, n GPUs (pgp_group_*): replicated scene / models, bases or hypotheses sharded over the devices, NCCL

@@ -47,6 +47,46 @@ def sample_box(rng: np.random.Generator, n: int, dims) -> tuple[np.ndarray, np.n
     return pts, nrm
 
 
+def box_mesh(dims, n: int = 1) -> tuple[np.ndarray, np.ndarray]:
+    """Box centred at 0, every face an n x n grid of quads split into two triangles: 12 n^2 triangles, fp32 vertices, int32
+    indices.  Neighbouring faces do not share vertices (a render of the box is closed all the same: the seams coincide)."""
+    half = np.asarray(dims, np.float64) / 2
+    g = np.linspace(-1.0, 1.0, n + 1)
+    verts, tris = [], []
+    for ax in range(3):
+        o1, o2 = [a for a in range(3) if a != ax]
+        for sgn in (1.0, -1.0):
+            u, v = np.meshgrid(g, g, indexing="ij")
+            p = np.zeros((n + 1, n + 1, 3))
+            p[..., ax] = sgn * half[ax]
+            p[..., o1] = u * half[o1]
+            p[..., o2] = v * half[o2]
+            base = sum(len(x) for x in verts)
+            i = np.arange(n)[:, None] * (n + 1) + np.arange(n)[None, :]
+            q = np.stack([i, i + n + 1, i + n + 2, i + 1], -1).reshape(-1, 4) + base
+            tris.append(np.concatenate([q[:, [0, 1, 2]], q[:, [0, 2, 3]]]))
+            verts.append(p.reshape(-1, 3))
+    return np.concatenate(verts).astype(np.float32), np.concatenate(tris).astype(np.int32)
+
+
+def ellipsoid_mesh(radii, n_lat: int, n_lon: int) -> tuple[np.ndarray, np.ndarray]:
+    """UV-sphere scaled to `radii`: 2 n_lon (n_lat - 1) triangles, shared vertices, poles included."""
+    th = np.linspace(0, np.pi, n_lat + 1)[1:-1]
+    ph = np.linspace(0, 2 * np.pi, n_lon, endpoint=False)
+    T, P = np.meshgrid(th, ph, indexing="ij")
+    ring = np.stack([np.sin(T) * np.cos(P), np.sin(T) * np.sin(P), np.cos(T)], -1).reshape(-1, 3)
+    verts = np.concatenate([[[0, 0, 1]], ring, [[0, 0, -1]]]) * np.asarray(radii, np.float64)
+    j = np.arange(n_lon)
+    jn = (j + 1) % n_lon
+    tris = [np.stack([np.zeros(n_lon, int), 1 + j, 1 + jn], -1)]
+    for r in range(n_lat - 2):
+        a, b = 1 + r * n_lon, 1 + (r + 1) * n_lon
+        tris += [np.stack([a + j, b + j, b + jn], -1), np.stack([a + j, b + jn, a + jn], -1)]
+    last, pole = 1 + (n_lat - 2) * n_lon, len(verts) - 1
+    tris.append(np.stack([last + j, np.full(n_lon, pole), last + jn], -1))
+    return verts.astype(np.float32), np.concatenate(tris).astype(np.int32)
+
+
 def seq_centroid_f32(xyz: np.ndarray) -> np.ndarray:
     """Sequential fp32 sum / n, the way Match4PCSBase::init accumulates centroids
     (/root/reference/src/3rdparty/super4pcs/src/super4pcs/algorithms/match4pcsBase.cc:242-250)."""
