@@ -319,8 +319,7 @@ __global__ void __launch_bounds__(128) k2_join_query(JoinParams p, const uint32_
                                                      const uint32_t* __restrict__ key_of, uint32_t* __restrict__ cnt, int4* __restrict__ out, long long cap,
                                                      const unsigned char* __restrict__ in_order, const uint32_t* __restrict__ list = nullptr,
                                                      const uint32_t* __restrict__ n_list = nullptr, uint32_t* __restrict__ list_out = nullptr,
-                                                     uint32_t* __restrict__ n_list_out = nullptr, uint32_t* __restrict__ cone_cache = nullptr,
-                                                     uint32_t* __restrict__ unordered_hit = nullptr) {
+                                                     uint32_t* __restrict__ n_list_out = nullptr, uint32_t* __restrict__ cone_cache = nullptr) {
   const long long t_id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (list ? t_id >= (long long)*n_list : t_id >= p.n2) return;
   const long long i = list ? (long long)list[t_id] : t_id;
@@ -392,7 +391,6 @@ __global__ void __launch_bounds__(128) k2_join_query(JoinParams p, const uint32_
         for (int t = 0; t < 11; ++t) cone_cache[(size_t)slot * 12 + t] = col_keep[t];
       }
     }
-    if (unordered_hit && n > 1 && !ordered) atomicOr(unordered_hit, 1u);      // an over-long bucket: this query's quads need a sort
   }
 }
 
@@ -521,16 +519,14 @@ __global__ void __launch_bounds__(128) k2_join_select(JoinParams p, const uint32
   }
 }
 
-// per-base output sizes min(staged, max_quads) -> exclusive scan (one CTA, like k2b_base_out); flags a staging overflow
-__global__ void __launch_bounds__(1024) k2c_stage_out(const uint32_t* __restrict__ stage_n, int nb, int max_quads, int stage_cap, uint32_t* __restrict__ outoff,
-                                                      uint32_t* __restrict__ overflow) {
+// One CTA of 1024 threads: outoff[b] = exclusive scan of count(b) (a base's output size, capped by the caller) over the nb bases
+// of a chunk, outoff[nb] = the total.  Thread t owns the contiguous bases [t per, (t + 1) per).
+template <class Count>
+__device__ __forceinline__ void capped_base_scan(int nb, Count count, uint32_t* __restrict__ outoff) {
   __shared__ uint32_t s_warp[32];
   const int per = (nb + 1023) / 1024, b0 = threadIdx.x * per, b1 = min(nb, b0 + per);
   uint32_t mine = 0;
-  for (int b = b0; b < b1; ++b) {
-    if (stage_n[b] > (uint32_t)stage_cap) atomicOr(overflow, 1u);
-    mine += min(stage_n[b], (uint32_t)max_quads);
-  }
+  for (int b = b0; b < b1; ++b) mine += count(b);
   uint32_t incl = mine;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)(threadIdx.x & 31) >= o) incl += t; }
@@ -538,8 +534,16 @@ __global__ void __launch_bounds__(1024) k2c_stage_out(const uint32_t* __restrict
   __syncthreads();
   uint32_t run = incl - mine;
   for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) run += s_warp[w];
-  for (int b = b0; b < b1; ++b) { outoff[b] = run; run += min(stage_n[b], (uint32_t)max_quads); }
+  for (int b = b0; b < b1; ++b) { outoff[b] = run; run += count(b); }
   if (threadIdx.x == 1023) outoff[nb] = run;
+}
+
+// per-base output sizes min(staged, max_quads) -> exclusive scan; flags a staging overflow
+__global__ void __launch_bounds__(1024) k2c_stage_out(const uint32_t* __restrict__ stage_n, int nb, int max_quads, int stage_cap, uint32_t* __restrict__ outoff,
+                                                      uint32_t* __restrict__ overflow) {
+  for (int b = threadIdx.x; b < nb; b += 1024)
+    if (stage_n[b] > (uint32_t)stage_cap) atomicOr(overflow, 1u);
+  capped_base_scan(nb, [&](int b) { return min(stage_n[b], (uint32_t)max_quads); }, outoff);
 }
 
 // one warp per base: rank of every staged entry by its order key (unique within a base), the first max_quads go out in that order
@@ -1011,33 +1015,56 @@ __device__ int block_discrete_draw(float* w, double* wd, int n, MinStd& gen, boo
   return pick;
 }
 
+// The draw of k2s_select_bases<SHARED> from the weights w[0..n), normalised first when `normalise` is set; every thread returns
+// the index.  SHARED: w and its double copy wd in shared memory, the block-cooperative block_discrete_draw.  Otherwise w is in
+// global memory and thread 0 does it all in the reference's order (sequential float sum, division, discrete_draw), broadcast
+// through s_i[0].
+template <bool SHARED>
+__device__ __forceinline__ int stocs_draw(float* w, double* wd, int n, MinStd& gen, bool normalise, int tid, float* s_f, double* s_dd, int* s_i) {
+  if (SHARED) return block_discrete_draw(w, wd, n, gen, normalise, tid, s_f, s_dd, s_i);
+  if (tid == 0) {
+    if (normalise) {
+      float sum = 0.f;
+      for (int i = 0; i < n; ++i) sum = __fadd_rn(sum, w[i]);
+      for (int i = 0; i < n; ++i) w[i] = __fdiv_rn(w[i], sum);
+    }
+    s_i[0] = discrete_draw(w, n, gen);
+  }
+  __syncthreads();
+  return s_i[0];
+}
+
 // One CTA per base: Match4PCSBase::SelectQuadrilateralStoCS (match4pcsBase.cc:600-792).  Each of the four points is drawn from
 // prior x "the PPF of the edge to the previous point exists in the model's map" (x the coplanarity / spread filters for the
-// 4th / 3rd point); the weights live in shared memory and are evaluated by all threads; the float normalisation and the draw
-// reproduce the reference's sequential arithmetic bit for bit (block_discrete_draw), so that a given engine seed reproduces the
-// reference's draw.  Dynamic shared memory: n floats + n doubles.
-__global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, BaseOut* __restrict__ out) {
+// 4th / 3rd point); the weights are evaluated by all threads, and the float normalisation and the draw reproduce the reference's
+// sequential arithmetic bit for bit (stocs_draw), so that a given engine seed reproduces the reference's draw.
+//   SHARED = true:  the weights (n floats + n doubles) in dynamic shared memory, K2S_T threads, block-cooperative draw;
+//   SHARED = false: for scenes whose weights do not fit shared memory, one slice of sp.curr per base, 256 threads, the draw on
+//                   thread 0.
+template <bool SHARED>
+__global__ void __launch_bounds__(SHARED ? K2S_T : 256, SHARED ? 8 : 0) k2s_select_bases(StocsParams sp, BaseOut* __restrict__ out) {
+  constexpr int NT = SHARED ? K2S_T : 256;
   extern __shared__ __align__(16) unsigned char k2s_smem[];
   __shared__ int s_any;
-  __shared__ int s_i[32];
-  __shared__ float s_f[12];
-  __shared__ double s_dd[12];
+  __shared__ int s_i[SHARED ? 32 : 2];
+  __shared__ float s_f[SHARED ? 12 : 1];
+  __shared__ double s_dd[SHARED ? 12 : 1];
   const int base = blockIdx.x, tid = threadIdx.x, n = sp.n;
   double* wd = reinterpret_cast<double*>(k2s_smem);
-  float* curr = reinterpret_cast<float*>(wd + n);
+  float* curr = SHARED ? reinterpret_cast<float*>(wd + n) : sp.curr + (size_t)base * n;
   const float4* P = sp.P;
   BaseOut o{};
   for (int attempt = 0; attempt < 16; ++attempt) {      // Perform_N_steps re-draws until a base is accepted (:1831-1852)
     MinStd gen(stocs_base_seed(sp.seed, sp.base0 + base, attempt));
     // ---- point 1 ~ priors
-    for (int i = tid; i < n; i += K2S_T) curr[i] = sp.aux[i].w;
+    for (int i = tid; i < n; i += NT) curr[i] = sp.aux[i].w;
     __syncthreads();
-    const int b1 = block_discrete_draw(curr, wd, n, gen, false, tid, s_f, s_dd, s_i);
+    const int b1 = stocs_draw<SHARED>(curr, wd, n, gen, false, tid, s_f, s_dd, s_i);
     const float4 p1 = P[b1], a1 = sp.aux[b1];
     // ---- point 2: prior_i * prior_b1 * edge(b1, i)
     if (tid == 0) s_any = 0;
     __syncthreads();
-    for (int i = tid; i < n; i += K2S_T) {
+    for (int i = tid; i < n; i += NT) {
       float w = 0.f;
       const float c = curr[i];
       if (i != b1 && c != 0.f) {
@@ -1050,13 +1077,13 @@ __global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, Bas
     }
     __syncthreads();
     if (!s_any) { __syncthreads(); continue; }
-    const int b2 = block_discrete_draw(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
+    const int b2 = stocs_draw<SHARED>(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
     const float4 p2 = P[b2], a2 = sp.aux[b2];
     // ---- point 3: curr_i * prior_b2 * edge(b2, i), minus the points whose (un-normalised!) angle test fails (:670-676)
     if (tid == 0) s_any = 0;
     __syncthreads();
     const float v1x = __fsub_rn(p2.x, p1.x), v1y = __fsub_rn(p2.y, p1.y), v1z = __fsub_rn(p2.z, p1.z);
-    for (int i = tid; i < n; i += K2S_T) {
+    for (int i = tid; i < n; i += NT) {
       float w = 0.f;
       const float c = curr[i];
       const float4 pi = P[i];
@@ -1080,7 +1107,7 @@ __global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, Bas
     }
     __syncthreads();
     if (!s_any) { __syncthreads(); continue; }
-    const int b3 = block_discrete_draw(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
+    const int b3 = stocs_draw<SHARED>(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
     const float4 p3 = P[b3], a3 = sp.aux[b3];
     // ---- point 4: near the plane of the three (<= 1 cm), >= 1 cm away from each of them, edge(b3, i)  (:717-763)
     if (tid == 0) s_any = 0;
@@ -1093,7 +1120,7 @@ __global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, Bas
       B = (float)((x2 * z1 - x3 * z1 - x1 * z2 + x3 * z2 + x1 * z3 - x2 * z3) / (double)denom);
       C = (float)((-x2 * y1 + x3 * y1 + x1 * y2 - x3 * y2 - x1 * y3 + x2 * y3) / (double)denom);
     }
-    for (int i = tid; i < n; i += K2S_T) {
+    for (int i = tid; i < n; i += NT) {
       float w = 0.f;
       const float c = curr[i];
       if (i != b1 && i != b2 && i != b3 && c != 0.f) {
@@ -1120,7 +1147,7 @@ __global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, Bas
     }
     __syncthreads();
     if (!s_any) { __syncthreads(); continue; }
-    const int b4 = block_discrete_draw(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
+    const int b4 = stocs_draw<SHARED>(curr, wd, n, gen, true, tid, s_f, s_dd, s_i);
     if (tid == 0) {
       const int ids[4] = {b1, b2, b3, b4};
       try_quadrilateral(P, ids, o);
@@ -1130,144 +1157,6 @@ __global__ void __launch_bounds__(K2S_T, 8) k2s_select_bases(StocsParams sp, Bas
     const int okk = s_i[1];
     __syncthreads();
     if (okk) break;
-  }
-  if (tid == 0) out[base] = o;
-}
-
-// Fallback of k2s_select_bases for scenes whose weight vectors do not fit shared memory (more than ~16 000 points): the same
-// procedure with the weights in global memory and every order-sensitive step on one thread.
-// One CTA per base: Match4PCSBase::SelectQuadrilateralStoCS (match4pcsBase.cc:600-792).  Each of the four points is drawn from
-// prior x "the PPF of the edge to the previous point exists in the model's map" (x the coplanarity / spread filters for the
-// 4th / 3rd point); the weights are evaluated by all threads, the float normalisation and the draw by thread 0, sequentially
-// and in the reference's order, so that a given engine seed reproduces the reference's draw.
-__global__ void __launch_bounds__(256) k2s_select_bases_global(StocsParams sp, BaseOut* __restrict__ out) {
-  __shared__ int s_pick;
-  __shared__ int s_any;
-  const int base = blockIdx.x, tid = threadIdx.x, n = sp.n;
-  float* curr = sp.curr + (size_t)base * n;
-  const float4* P = sp.P;
-  BaseOut o{};
-  for (int attempt = 0; attempt < 16; ++attempt) {      // Perform_N_steps re-draws until a base is accepted (:1831-1852)
-    MinStd gen(stocs_base_seed(sp.seed, sp.base0 + base, attempt));
-    // ---- point 1 ~ priors
-    for (int i = tid; i < n; i += 256) curr[i] = sp.aux[i].w;
-    __syncthreads();
-    if (tid == 0) s_pick = discrete_draw(curr, n, gen);
-    __syncthreads();
-    const int b1 = s_pick;
-    const float4 p1 = P[b1], a1 = sp.aux[b1];
-    // ---- point 2: prior_i * prior_b1 * edge(b1, i)
-    if (tid == 0) s_any = 0;
-    __syncthreads();
-    for (int i = tid; i < n; i += 256) {
-      float w = 0.f;
-      const float c = curr[i];
-      if (i != b1 && c != 0.f) {
-        const float4 ai = sp.aux[i];
-        const float e = ppf_present(sp.bits, ppf_key(p1, a1, P[i], ai)) ? 1.f : 0.f;
-        w = __fmul_rn(__fmul_rn(ai.w, a1.w), e);
-      }
-      curr[i] = w;
-      if (w != 0.f) s_any = 1;
-    }
-    __syncthreads();
-    if (!s_any) { __syncthreads(); continue; }
-    if (tid == 0) {
-      float sum = 0.f;
-      for (int i = 0; i < n; ++i) sum = __fadd_rn(sum, curr[i]);
-      for (int i = 0; i < n; ++i) curr[i] = __fdiv_rn(curr[i], sum);
-      s_pick = discrete_draw(curr, n, gen);
-    }
-    __syncthreads();
-    const int b2 = s_pick;
-    const float4 p2 = P[b2], a2 = sp.aux[b2];
-    // ---- point 3: curr_i * prior_b2 * edge(b2, i), minus the points whose (un-normalised!) angle test fails (:670-676)
-    if (tid == 0) s_any = 0;
-    __syncthreads();
-    const float v1x = __fsub_rn(p2.x, p1.x), v1y = __fsub_rn(p2.y, p1.y), v1z = __fsub_rn(p2.z, p1.z);
-    for (int i = tid; i < n; i += 256) {
-      float w = 0.f;
-      const float c = curr[i];
-      const float4 pi = P[i];
-      const float d = dot3_tree(v1x, v1y, v1z, __fsub_rn(pi.x, p1.x), __fsub_rn(pi.y, p1.y), __fsub_rn(pi.z, p1.z));
-      // |d| < 0.8: acos(d) lies in (36.8, 143.2) degrees, min(a, 180 - a) > 30 whatever the rounding -- the case for metre-scale
-      // vectors, whose un-normalised dot product is tiny; anything else takes the reference's arithmetic
-      bool far30 = fabsf(d) < 0.8f;
-      if (!far30) {
-        float ang = (float)((double)__fmul_rn((float)acos((double)d), 180.0f) / 3.14159265358979323846);
-        const float other = __fsub_rn(180.0f, ang);
-        ang = other < ang ? other : ang;               // std::min(a, b) = (b < a) ? b : a   (NaN stays NaN -> not rejected)
-        far30 = !(ang < 30.0f);
-      }
-      if (i != b1 && i != b2 && c != 0.f && far30) {
-        const float4 ai = sp.aux[i];
-        const float e = ppf_present(sp.bits, ppf_key(p2, a2, pi, ai)) ? 1.f : 0.f;
-        w = __fmul_rn(__fmul_rn(c, a2.w), e);
-      }
-      curr[i] = w;
-      if (w != 0.f) s_any = 1;
-    }
-    __syncthreads();
-    if (!s_any) { __syncthreads(); continue; }
-    if (tid == 0) {
-      float sum = 0.f;
-      for (int i = 0; i < n; ++i) sum = __fadd_rn(sum, curr[i]);
-      for (int i = 0; i < n; ++i) curr[i] = __fdiv_rn(curr[i], sum);
-      s_pick = discrete_draw(curr, n, gen);
-    }
-    __syncthreads();
-    const int b3 = s_pick;
-    const float4 p3 = P[b3], a3 = sp.aux[b3];
-    // ---- point 4: near the plane of the three (<= 1 cm), >= 1 cm away from each of them, edge(b3, i)  (:717-763)
-    if (tid == 0) s_any = 0;
-    __syncthreads();
-    const double x1 = p1.x, y1 = p1.y, z1 = p1.z, x2 = p2.x, y2 = p2.y, z2 = p2.z, x3 = p3.x, y3 = p3.y, z3 = p3.z;
-    const float denom = (float)(-x3 * y2 * z1 + x2 * y3 * z1 + x3 * y1 * z2 - x1 * y3 * z2 - x2 * y1 * z3 + x1 * y2 * z3);
-    float A = 0.f, B = 0.f, C = 0.f;
-    if (denom != 0.f) {
-      A = (float)((-y2 * z1 + y3 * z1 + y1 * z2 - y3 * z2 - y1 * z3 + y2 * z3) / (double)denom);
-      B = (float)((x2 * z1 - x3 * z1 - x1 * z2 + x3 * z2 + x1 * z3 - x2 * z3) / (double)denom);
-      C = (float)((-x2 * y1 + x3 * y1 + x1 * y2 - x3 * y2 - x1 * y3 + x2 * y3) / (double)denom);
-    }
-    for (int i = tid; i < n; i += 256) {
-      float w = 0.f;
-      const float c = curr[i];
-      if (i != b1 && i != b2 && i != b3 && c != 0.f) {
-        const float4 pi = P[i];
-        bool keep = true;
-        if (denom != 0.f) {
-          const float lin = __fadd_rn(__fadd_rn(__fmul_rn(A, pi.x), __fmul_rn(B, pi.y)), __fmul_rn(C, pi.z));
-          const float pd = fabsf(__fsub_rn(lin, 1.0f));        // (float) fabs((double) lin - 1.0): the double difference is exact, its rounding is this
-          auto nrm = [&](const float4 q) {
-            const float dx = __fsub_rn(pi.x, q.x), dy = __fsub_rn(pi.y, q.y), dz = __fsub_rn(pi.z, q.z);
-            return __fsqrt_rn(dot3_tree(dx, dy, dz, dx, dy, dz));
-          };
-          // float against the double 0.01 (fl32(0.01) = 0.0099999998 < 0.01): x > 0.01 <=> x > 0.01f,  x < 0.01 <=> x <= 0.01f
-          if (pd > 0.01f || nrm(p1) <= 0.01f || nrm(p2) <= 0.01f || nrm(p3) <= 0.01f) keep = false;
-        }
-        if (keep) {
-          const float4 ai = sp.aux[i];
-          const float e = ppf_present(sp.bits, ppf_key(p3, a3, pi, ai)) ? 1.f : 0.f;
-          w = __fmul_rn(__fmul_rn(c, a3.w), e);
-        }
-      }
-      curr[i] = w;
-      if (w != 0.f) s_any = 1;
-    }
-    __syncthreads();
-    if (!s_any) { __syncthreads(); continue; }
-    if (tid == 0) {
-      float sum = 0.f;
-      for (int i = 0; i < n; ++i) sum = __fadd_rn(sum, curr[i]);
-      for (int i = 0; i < n; ++i) curr[i] = __fdiv_rn(curr[i], sum);
-      const int b4 = discrete_draw(curr, n, gen);
-      const int ids[4] = {b1, b2, b3, b4};
-      try_quadrilateral(P, ids, o);
-      s_pick = o.ok;
-    }
-    __syncthreads();
-    if (s_pick) break;
-    __syncthreads();
   }
   if (tid == 0) out[base] = o;
 }
@@ -1702,31 +1591,12 @@ __global__ void k2v_quad_offsets(const uint32_t* __restrict__ scan, int nq, int 
   if (b <= nb) qoff[b] = scan[(size_t)b * nq];
 }
 
-// one thread: per-base kept counts (capped) -> output offsets
+// per-base kept counts (capped when max_quads > 0) -> exclusive scan
 __global__ void __launch_bounds__(1024) k2b_base_out(const uint32_t* __restrict__ fscan, const uint32_t* __restrict__ qoff, int nb, int max_quads, uint32_t* __restrict__ outoff) {
-  // one CTA: thread t owns the contiguous bases [t per, (t + 1) per); exclusive scan of the per-base output sizes
-  __shared__ uint32_t s_warp[32];
-  const int per = (nb + 1023) / 1024, b0 = threadIdx.x * per, b1 = min(nb, b0 + per);
-  uint32_t mine = 0;
-  for (int b = b0; b < b1; ++b) {
-    uint32_t k = fscan[qoff[b + 1]] - fscan[qoff[b]];
-    if (max_quads > 0 && k > (uint32_t)max_quads) k = (uint32_t)max_quads;
-    mine += k;
-  }
-  uint32_t incl = mine;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)(threadIdx.x & 31) >= o) incl += t; }
-  if ((threadIdx.x & 31) == 31) s_warp[threadIdx.x >> 5] = incl;
-  __syncthreads();
-  uint32_t run = incl - mine;
-  for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) run += s_warp[w];
-  for (int b = b0; b < b1; ++b) {
-    outoff[b] = run;
-    uint32_t k = fscan[qoff[b + 1]] - fscan[qoff[b]];
-    if (max_quads > 0 && k > (uint32_t)max_quads) k = (uint32_t)max_quads;
-    run += k;
-  }
-  if (threadIdx.x == 1023) outoff[nb] = run;
+  capped_base_scan(nb, [&](int b) {
+    const uint32_t k = fscan[qoff[b + 1]] - fscan[qoff[b]];
+    return max_quads > 0 && k > (uint32_t)max_quads ? (uint32_t)max_quads : k;
+  }, outoff);
 }
 
 __global__ void k2b_append(const float* __restrict__ T, const uint32_t* __restrict__ fscan, const uint32_t* __restrict__ qoff, int nb, int max_quads,
@@ -1777,65 +1647,32 @@ int v4pcs_chunk(pgp_ctx* ctx, const Model& m, const BaseOut* d_bases, int nb, fl
   return PGP_OK;
 }
 
-// pgp_generate_pcs in operMode 2: tetrahedron bases -> V4PCS quads -> rigid transforms -> per-base subset -> append
-int generate_v4pcs(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, int base_lo, int base_hi, int64_t max_hyp, float max_diam, int64_t* n_hyp) {
+// Unfused tail of a chunk of nb bases: the rigid transform of each of the nquads quads in sc.quads (base b's at
+// [qoff[b], qoff[b+1])), the per-base subset, and the kept transforms appended at dst, at most `room` of them.  *added = how many.
+int append_unfused(pgp_ctx* ctx, const Model& m, const pgp_pcs_opts* o, uint64_t seed, const BaseOut* d_bases, int base_global0, int nb,
+                   const uint32_t* qoff, uint64_t nquads, uint32_t* outoff, float* dst, int64_t room, int64_t* added) {
   Scratch& sc = scratch_of(ctx);
-  const Scene& s = ctx->scene;
   cudaStream_t st = ctx->stream;
-  const int nb_total = base_hi - base_lo, nq = m.nq, W = (nq + 31) / 32;
-  sc.bases_owner = &m;
-  const float eps = s.delta;
-  PGP_CUDA(ctx, sc.base.reserve((size_t)nb_total * sizeof(BaseOut) + 64));
-  PGP_CUDA(ctx, m.gen_T.reserve((size_t)std::max<int64_t>(max_hyp, 1) * 48));
-  BaseOut* d_bases_all = reinterpret_cast<BaseOut*>(sc.base.as<char>() + 64);
-  k2v_select_bases<<<nb_total, 256, 0, st>>>(s.unsorted.as<float4>(), s.n, max_diam, std::max(1, o->base_trials), seed, base_lo, d_bases_all);
+  PGP_CUDA(ctx, sc.T.reserve((size_t)nquads * 48));
+  PGP_CUDA(ctx, sc.flag.reserve((size_t)(nquads + 1) * 4));
+  uint32_t* flag = sc.flag.as<uint32_t>();
+  PGP_CUDA(ctx, cudaMemsetAsync(flag + nquads, 0, 4, st));
+  const unsigned gr = (unsigned)((nquads + 127) / 128);
+  k2b_rigid<<<gr, 128, 0, st>>>(ctx->scene.unsorted.as<float4>(), m.search.as<float4>(), d_bases, base_global0, qoff, nb, sc.quads.as<int4>(),
+                                (long long)nquads, o->max_quads_per_base, seed, sc.T.as<float>(), flag);
   ctx->launches++;
   PGP_CUDA(ctx, cudaGetLastError());
-  // bases per chunk: six nq x nq bit matrices each, about 1 GB in all
-  int chunk = (int)std::max<double>(1.0, std::min<double>(64.0, 1.0e9 / (24.0 * (double)nq * (double)W)));
-  int64_t cur = 0;
-  int nb = 0;
-  for (int base0 = 0; base0 < nb_total && cur < max_hyp; base0 += nb) {
-    nb = std::min(chunk, nb_total - base0);
-    const BaseOut* d_bases = d_bases_all + base0;
-    PGP_CUDA(ctx, sc.off.reserve((size_t)(4 * nb + 16) * 4 + 64));
-    uint32_t* qoff = sc.off.as<uint32_t>();            // nb + 1
-    uint32_t* outoff = qoff + nb + 2;                  // nb + 1
-    uint64_t nquads = 0;
-    int rc = v4pcs_chunk(ctx, m, d_bases, nb, eps, qoff, &nquads);
-    if (rc) return rc;
-    if (nquads == 0) continue;
-    if (nquads >= (1ull << 31)) {
-      if (nb > 1) { chunk = std::max(1, nb / 2); nb = 0; continue; }
-      return pgp_fail(ctx, PGP_E_TOO_LARGE, "congruent quads of one base exceed 2^31");
-    }
-    PGP_CUDA(ctx, sc.T.reserve((size_t)nquads * 48));
-    PGP_CUDA(ctx, sc.flag.reserve((size_t)(nquads + 1) * 4));
-    uint32_t* flag = sc.flag.as<uint32_t>();
-    PGP_CUDA(ctx, cudaMemsetAsync(flag + nquads, 0, 4, st));
-    const unsigned gr = (unsigned)((nquads + 127) / 128);
-    k2b_rigid<<<gr, 128, 0, st>>>(s.unsorted.as<float4>(), m.search.as<float4>(), d_bases, base_lo + base0, qoff, nb, sc.quads.as<int4>(), (long long)nquads,
-                                  o->max_quads_per_base, seed, sc.T.as<float>(), flag);
-    ctx->launches++;
-    PGP_CUDA(ctx, cudaGetLastError());
-    PGP_CUDA(ctx, ctx->scene.scratch.reserve((size_t)((nquads + 1) / 2048 + 4096) * 4));
-    rc = pgp_scan_exclusive_u32(ctx, flag, (int64_t)nquads + 1, ctx->scene.scratch.as<uint32_t>());
-    if (rc) return rc;
-    k2b_base_out<<<1, 1024, 0, st>>>(flag, qoff, nb, o->max_quads_per_base, outoff);
-    const int64_t room = max_hyp - cur;
-    k2b_append<<<gr, 128, 0, st>>>(sc.T.as<float>(), flag, qoff, nb, o->max_quads_per_base, outoff, (long long)nquads, m.gen_T.as<float>() + 12 * cur, room);
-    ctx->launches += 2;
-    PGP_CUDA(ctx, cudaGetLastError());
-    uint32_t added = 0;
-    PGP_CUDA(ctx, cudaMemcpyAsync(&added, outoff + nb, 4, cudaMemcpyDeviceToHost, st));
-    PGP_CUDA(ctx, cudaStreamSynchronize(st));
-    cur += std::min<int64_t>(room, (int64_t)added);
-  }
-  PGP_CUDA(ctx, cudaStreamSynchronize(st));
+  PGP_CUDA(ctx, ctx->scene.scratch.reserve((size_t)((nquads + 1) / 2048 + 4096) * 4));
+  int rc = pgp_scan_exclusive_u32(ctx, flag, (int64_t)nquads + 1, ctx->scene.scratch.as<uint32_t>());
+  if (rc) return rc;
+  k2b_base_out<<<1, 1024, 0, st>>>(flag, qoff, nb, o->max_quads_per_base, outoff);
+  k2b_append<<<gr, 128, 0, st>>>(sc.T.as<float>(), flag, qoff, nb, o->max_quads_per_base, outoff, (long long)nquads, dst, room);
+  ctx->launches += 2;
   PGP_CUDA(ctx, cudaGetLastError());
-  m.n_gen = std::min<int64_t>(cur, max_hyp);
-  m.n_gen_bases = nb_total;
-  *n_hyp = m.n_gen;
+  uint32_t n = 0;
+  PGP_CUDA(ctx, cudaMemcpyAsync(&n, outoff + nb, 4, cudaMemcpyDeviceToHost, st));
+  PGP_CUDA(ctx, cudaStreamSynchronize(st));
+  *added = std::min<int64_t>(room, (int64_t)n);
   return PGP_OK;
 }
 
@@ -1883,20 +1720,26 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
   const int nq = m.nq;
   float max_diam = o->max_base_diameter;
   if (!(max_diam > 0.f)) max_diam = m.search_diameter;   // P_diameter_ estimate of init() (:274-283)
-  if (o->mode == 2) return generate_v4pcs(ctx, m, o, seed, base_lo, base_hi, max_hyp, max_diam, n_hyp);
   const float eps = s.delta;          // distance_factor * options_.delta, distance_factor = 1 (match4pcsBase.h:99)
-  // join grid (IndexedNormalSet, normalset.h:117-123); buckets per base capped at 2^15 (collisions are filtered by the key)
-  const float eps_n = eps / m.unit_ratio;
-  int depth = (int)(-std::log2(eps_n));
-  if (depth < 0) depth = 0;
-  if (depth > 7) return pgp_fail(ctx, PGP_E_TOO_LARGE, "quad join: model diameter / delta too large (grid depth %d > 7)", depth);
-  const uint32_t nbk = 1u << std::min(3 * depth, 15);
-  // bases per chunk.  Every chunk costs ~25 launches and three host-read totals whatever its size, so chunks are made as large as
-  // the join's buffers allow (32 bytes per pair + 8 bytes per hash bucket; budget ~2 GB each of the B200's 180 GB): operMode 0 has
-  // ~10 % of nq^2 ordered pairs per (base, edge), operMode 1 the PPF map's mean row length.  A chunk that turns out too large is
-  // halved below (`shrink`); the hypotheses do not depend on the chunking.
-  const double pairs_per_base = o->mode == 1 ? 3.0 * (double)m.n_ppf_pairs / (double)std::max(1, m.n_ppf_keys) : 0.2 * (double)nq * (double)nq;
-  int chunk = (int)std::max(1.0, std::min({o->mode == 1 ? 4096.0 : 256.0, 6.0e7 / std::max(1.0, pairs_per_base), 2.5e8 / (double)nbk}));
+  int depth = 0, chunk;
+  uint32_t nbk = 0;
+  if (o->mode == 2) {
+    // bases per chunk: six nq x nq bit matrices each, about 1 GB in all
+    chunk = (int)std::max<double>(1.0, std::min<double>(64.0, 1.0e9 / (24.0 * (double)nq * (double)((nq + 31) / 32))));
+  } else {
+    // join grid (IndexedNormalSet, normalset.h:117-123); buckets per base capped at 2^15 (collisions are filtered by the key)
+    const float eps_n = eps / m.unit_ratio;
+    depth = (int)(-std::log2(eps_n));
+    if (depth < 0) depth = 0;
+    if (depth > 7) return pgp_fail(ctx, PGP_E_TOO_LARGE, "quad join: model diameter / delta too large (grid depth %d > 7)", depth);
+    nbk = 1u << std::min(3 * depth, 15);
+    // bases per chunk.  Every chunk costs ~25 launches and three host-read totals whatever its size, so chunks are made as large as
+    // the join's buffers allow (32 bytes per pair + 8 bytes per hash bucket; budget ~2 GB each of the B200's 180 GB): operMode 0 has
+    // ~10 % of nq^2 ordered pairs per (base, edge), operMode 1 the PPF map's mean row length.  A chunk that turns out too large is
+    // halved below (`shrink`); the hypotheses do not depend on the chunking.
+    const double pairs_per_base = o->mode == 1 ? 3.0 * (double)m.n_ppf_pairs / (double)std::max(1, m.n_ppf_keys) : 0.2 * (double)nq * (double)nq;
+    chunk = (int)std::max(1.0, std::min({o->mode == 1 ? 4096.0 : 256.0, 6.0e7 / std::max(1.0, pairs_per_base), 2.5e8 / (double)nbk}));
+  }
   PGP_CUDA(ctx, sc.base.reserve((size_t)nb_total * sizeof(BaseOut) + 64));
   PGP_CUDA(ctx, m.gen_T.reserve((size_t)std::max<int64_t>(max_hyp, 1) * 48));
   BaseOut* d_bases_all = reinterpret_cast<BaseOut*>(sc.base.as<char>() + 64);
@@ -1911,9 +1754,9 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
     sp.seed = seed;
     const size_t smem_sel = (size_t)s.n * 12 + 16;                    // the weights of one base: n floats + n doubles in shared memory
     if (smem_sel <= 200 * 1024) {
-      PGP_CUDA(ctx, cudaFuncSetAttribute(k2s_select_bases, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sel));
+      PGP_CUDA(ctx, cudaFuncSetAttribute(k2s_select_bases<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_sel));
       sp.curr = nullptr; sp.base0 = base_lo;
-      k2s_select_bases<<<nb_total, K2S_T, smem_sel, st>>>(sp, d_bases_all);
+      k2s_select_bases<true><<<nb_total, K2S_T, smem_sel, st>>>(sp, d_bases_all);
     } else {
       // larger scenes: one weight vector of |P| floats per base in global memory, the bases selected in batches of at most ~1 GB of them
       const int bsel = (int)std::max<int64_t>(1, std::min<int64_t>(nb_total, ((int64_t)1 << 28) / std::max(1, s.n)));
@@ -1921,10 +1764,12 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
       sp.curr = sc.curr.as<float>();
       for (int b0 = 0; b0 < nb_total; b0 += bsel) {
         sp.base0 = base_lo + b0;
-        k2s_select_bases_global<<<std::min(bsel, nb_total - b0), 256, 0, st>>>(sp, d_bases_all + b0);
+        k2s_select_bases<false><<<std::min(bsel, nb_total - b0), 256, 0, st>>>(sp, d_bases_all + b0);
         if (b0) ctx->launches++;
       }
     }
+  } else if (o->mode == 2) {
+    k2v_select_bases<<<nb_total, 256, 0, st>>>(s.unsorted.as<float4>(), s.n, max_diam, std::max(1, o->base_trials), seed, base_lo, d_bases_all);
   } else {
     k2_select_bases<<<nb_total, 256, 0, st>>>(s.unsorted.as<float4>(), s.n, max_diam, std::max(1, o->base_trials), seed, base_lo, d_bases_all);
   }
@@ -1941,15 +1786,32 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
     const int ncombo = 2 * nb;
     auto shrink = [&]() { if (nb <= 1) return false; chunk = std::max(1, nb / 2); nb = 0; return true; };   // nb = 0: the loop repeats base0
     const BaseOut* d_bases = d_bases_all + base0;
-    // ---- pairs of all 2 nb (base, edge) combos
-    const size_t ncnt = (size_t)ncombo * nq;
-    PGP_CUDA(ctx, sc.cnt.reserve((ncnt + 1) * 4));
     PGP_CUDA(ctx, sc.off.reserve((size_t)(4 * nb + 16) * 4 + 64));
-    uint32_t* cnt = sc.cnt.as<uint32_t>();
     uint32_t* coff = sc.off.as<uint32_t>();            // ncombo + 1
     uint32_t* qoff = coff + ncombo + 2;                // nb + 1
     uint32_t* outoff = qoff + nb + 2;                  // nb + 1
+    const int64_t room = max_hyp - cur;
+    int64_t added = 0;
     int rc;
+    if (o->mode == 2) {
+      // ---- V4PCS quads of the chunk, then the unfused tail
+      uint64_t nquads = 0;
+      rc = v4pcs_chunk(ctx, m, d_bases, nb, eps, qoff, &nquads);
+      if (rc) return rc;
+      if (nquads == 0) continue;
+      if (nquads >= (1ull << 31)) {
+        if (shrink()) continue;
+        return pgp_fail(ctx, PGP_E_TOO_LARGE, "congruent quads of one base exceed 2^31");
+      }
+      rc = append_unfused(ctx, m, o, seed, d_bases, base_lo + base0, nb, qoff, nquads, outoff, m.gen_T.as<float>() + 12 * cur, room, &added);
+      if (rc) return rc;
+      cur += added;
+      continue;
+    }
+    // ---- pairs of all 2 nb (base, edge) combos
+    const size_t ncnt = (size_t)ncombo * nq;
+    PGP_CUDA(ctx, sc.cnt.reserve((ncnt + 1) * 4));
+    uint32_t* cnt = sc.cnt.as<uint32_t>();
     int64_t ntot = 0;
     if (stocs) {
       // pair lists come out of the PPF map: count per combo, scan, copy
@@ -2035,19 +1897,16 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
     // that found quads -> fill pass on those
     PGP_CUDA(ctx, sc.list1.reserve((size_t)ntot * 4 + 16));
     PGP_CUDA(ctx, sc.list2.reserve((size_t)ntot * 4 + 16));
-    uint32_t* n_lists = reinterpret_cast<uint32_t*>(ctx->work.as<char>() + 384);      // [0] = |list1|, [1] = |list2|, [2] = a query hit an over-long bucket, [3] = staging overflow
-    PGP_CUDA(ctx, cudaMemsetAsync(n_lists, 0, 16, st));
+    uint32_t* n_lists = reinterpret_cast<uint32_t*>(ctx->work.as<char>() + 384);      // [0] = |list1|, [1] = |list2|, [2] = staging overflow
+    PGP_CUDA(ctx, cudaMemsetAsync(n_lists, 0, 12, st));
     k2_join_probe<<<gk, 256, 0, st>>>(p, bs, sc.sorted.as<uint32_t>(), sc.key_of.as<uint32_t>(), sc.list1.as<uint32_t>(), n_lists);
     const unsigned gq = (unsigned)((ntot + 127) / 128);
-    const bool want_fused = fused;
-    if (want_fused) PGP_CUDA(ctx, sc.cone.reserve((size_t)ntot * 48 + 64));
+    if (fused) PGP_CUDA(ctx, sc.cone.reserve((size_t)ntot * 48 + 64));
     k2_join_query<false><<<gq, 128, 0, st>>>(p, bs, sc.sorted.as<uint32_t>(), sc.key_of.as<uint32_t>(), cnt2, nullptr, 0, sc.in_order.as<unsigned char>(), sc.list1.as<uint32_t>(), n_lists,
-                                             sc.list2.as<uint32_t>(), n_lists + 1, want_fused ? sc.cone.as<uint32_t>() : nullptr, n_lists + 2);
+                                             sc.list2.as<uint32_t>(), n_lists + 1, fused ? sc.cone.as<uint32_t>() : nullptr);
     ctx->launches += 2;
     PGP_CUDA(ctx, cudaGetLastError());
     uint64_t nquads = 0;
-    uint32_t unordered = 0;
-    PGP_CUDA(ctx, cudaMemcpyAsync(&unordered, n_lists + 2, 4, cudaMemcpyDeviceToHost, st));
     rc = scan_u32(ctx, cnt2, ntot, &nquads);                                // sync 2
     if (rc) return rc;
     if (nquads == 0) continue;
@@ -2057,9 +1916,7 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
     }
     k2b_quad_offsets<<<(nb + 256) / 256, 256, 0, st>>>(cnt2, coff, nb, qoff);
     ctx->launches++;
-    const int64_t room = max_hyp - cur;
-    (void)unordered;
-    if (want_fused) {
+    if (fused) {
       // ---- fused: select (the reference's random subset of max_sampled_csets quads per base) BEFORE transforming; see k2_join_select
       const int stage_cap = o->max_quads_per_base * 5 / 2 + 64;            // mean 1.25 max_quads selected per base, sigma ~ sqrt of that
       PGP_CUDA(ctx, sc.stage_n.reserve((size_t)nb * 4 + 16));
@@ -2069,13 +1926,13 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
       k2_join_select<<<gq, 128, 0, st>>>(p, bs, sc.sorted.as<uint32_t>(), sc.key_of.as<uint32_t>(), cnt2, sc.list2.as<uint32_t>(), n_lists + 1, sc.cone.as<uint32_t>(),
                                          s.unsorted.as<float4>(), qoff, base_lo + base0, o->max_quads_per_base, seed, stage_cap, sc.stage_n.as<uint32_t>(),
                                          sc.stage_r.as<uint32_t>(), sc.stage_T.as<float>());
-      k2c_stage_out<<<1, 1024, 0, st>>>(sc.stage_n.as<uint32_t>(), nb, o->max_quads_per_base, stage_cap, outoff, n_lists + 3);
+      k2c_stage_out<<<1, 1024, 0, st>>>(sc.stage_n.as<uint32_t>(), nb, o->max_quads_per_base, stage_cap, outoff, n_lists + 2);
       k2c_stage_append<<<(unsigned)((nb * 32 + 255) / 256), 256, 0, st>>>(sc.stage_n.as<uint32_t>(), sc.stage_r.as<uint32_t>(), sc.stage_T.as<float>(), nb,
                                                                           o->max_quads_per_base, stage_cap, outoff, m.gen_T.as<float>() + 12 * cur, room);
       ctx->launches += 3;
       PGP_CUDA(ctx, cudaGetLastError());
       uint32_t overflow = 0;
-      PGP_CUDA(ctx, cudaMemcpyAsync(&overflow, n_lists + 3, 4, cudaMemcpyDeviceToHost, st));
+      PGP_CUDA(ctx, cudaMemcpyAsync(&overflow, n_lists + 2, 4, cudaMemcpyDeviceToHost, st));
       uint32_t added_f = 0;
       PGP_CUDA(ctx, cudaMemcpyAsync(&added_f, outoff + nb, 4, cudaMemcpyDeviceToHost, st));
       PGP_CUDA(ctx, cudaStreamSynchronize(st));                             // sync 3
@@ -2089,29 +1946,13 @@ int k2_generate(pgp_ctx* ctx, Model& m, const pgp_pcs_opts* o, uint64_t seed, in
       return pgp_fail(ctx, PGP_E_TOO_LARGE, "congruent quads of one base exceed the device memory");
     }
     PGP_CUDA(ctx, sc.quads.reserve((size_t)nquads * 16));
-    PGP_CUDA(ctx, sc.T.reserve((size_t)nquads * 48));
-    PGP_CUDA(ctx, sc.flag.reserve((size_t)(nquads + 1) * 4));
     k2_join_query<true><<<gq, 128, 0, st>>>(p, bs, sc.sorted.as<uint32_t>(), sc.key_of.as<uint32_t>(), cnt2, sc.quads.as<int4>(), (long long)nquads,
                                             sc.in_order.as<unsigned char>(), sc.list2.as<uint32_t>(), n_lists + 1);
-    // ---- transforms, subset, compaction behind the hypotheses already generated
-    uint32_t* flag = sc.flag.as<uint32_t>();
-    PGP_CUDA(ctx, cudaMemsetAsync(flag + nquads, 0, 4, st));
-    const unsigned gr = (unsigned)((nquads + 127) / 128);
-    k2b_rigid<<<gr, 128, 0, st>>>(s.unsorted.as<float4>(), m.search.as<float4>(), d_bases, base_lo + base0, qoff, nb, sc.quads.as<int4>(), (long long)nquads,
-                                  o->max_quads_per_base, seed, sc.T.as<float>(), flag);
-    ctx->launches += 2;
-    PGP_CUDA(ctx, cudaGetLastError());
-    PGP_CUDA(ctx, ctx->scene.scratch.reserve((size_t)((nquads + 1) / 2048 + 4096) * 4));
-    rc = pgp_scan_exclusive_u32(ctx, flag, (int64_t)nquads + 1, ctx->scene.scratch.as<uint32_t>());
+    ctx->launches++;
+    // ---- transforms, subset, compaction behind the hypotheses already generated (sync 3)
+    rc = append_unfused(ctx, m, o, seed, d_bases, base_lo + base0, nb, qoff, nquads, outoff, m.gen_T.as<float>() + 12 * cur, room, &added);
     if (rc) return rc;
-    k2b_base_out<<<1, 1024, 0, st>>>(flag, qoff, nb, o->max_quads_per_base, outoff);
-    k2b_append<<<gr, 128, 0, st>>>(sc.T.as<float>(), flag, qoff, nb, o->max_quads_per_base, outoff, (long long)nquads, m.gen_T.as<float>() + 12 * cur, room);
-    ctx->launches += 2;
-    PGP_CUDA(ctx, cudaGetLastError());
-    uint32_t added = 0;
-    PGP_CUDA(ctx, cudaMemcpyAsync(&added, outoff + nb, 4, cudaMemcpyDeviceToHost, st));
-    PGP_CUDA(ctx, cudaStreamSynchronize(st));                               // sync 3
-    cur += std::min<int64_t>(room, (int64_t)added);
+    cur += added;
   }
   PGP_CUDA(ctx, cudaStreamSynchronize(st));
   PGP_CUDA(ctx, cudaGetLastError());
