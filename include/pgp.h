@@ -337,6 +337,9 @@ PGP_API int pgp_bench_sector_gather(pgp_ctx* ctx, int64_t footprint_bytes, int l
  * then diagonalises with Jacobi. */
 PGP_API float pgp_host_chain_sum_equal(float c, long long m);
 PGP_API int pgp_host_max_eigvec4(const double* N16_rowmajor, double* q4);
+/* pgp_host_solve_plane6: x6 = H^+ g6, the truncated, scaled pseudo-inverse solve of pgp_tricp_plane's fit (H36 row-major,
+ * symmetric positive semi-definite); returns the number of eigenvalues kept. */
+PGP_API int pgp_host_solve_plane6(const double* H36_rowmajor, const double* g6, double* x6);
 
 /* ---------------------------------------------------------------- K5: trimmed ICP ---------- */
 
@@ -358,6 +361,24 @@ PGP_API int pgp_host_max_eigvec4(const double* N16_rowmajor, double* q4);
  * unaffected: each pose's result does not depend on the rest of the batch. */
 PGP_API int pgp_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, double* poses16_host, int k,
                       float trim, float ratio, int max_iter, int* iters_out, float* energy_out);
+
+/* Trimmed point-to-plane ICP: utilities::pointToPlaneICP (PPE/src/misc/utilities.cpp:709-739) -> PCL's
+ * TransformationEstimationPointToPlaneLLS, restated (PCL is not vendored: parity unpinned).  Arguments, refusals and result
+ * conventions are those of pgp_tricp, and so are the start transform, the queries, the nearest neighbours, the trim (the
+ * n_keep smallest POINT-TO-POINT squared distances, ties in Morton order), the stop rule and the final inversion.  Per kept pair,
+ * in double: q = the validation point as given, n = its unit validation normal (zero where pgp_set_model zeroed it), p' = the
+ * fp32 query, r = ((dx nx + dy ny) + dz nz) with d = p' - q, a = [p' x n, n].  Sums over the kept set: E = sum r^2,
+ * H = sum a a^T, g = -sum a r; energy_out = (float)E, the point-to-plane trimmed energy.  When it is finite:
+ * x = H^+ g with Jacobi scaling s_j = 1/sqrt(H_jj) (0 where H_jj <= 0), M = S H S = V L V^T by cyclic Jacobi in double (stop
+ * when the off-diagonal norm is <= 1e-15 |M|_F, or after 30 sweeps), eigenvalues <= 1e-9 lambda_max dropped (all when
+ * lambda_max <= 0), x = S V L^+ V^T S g; x = (alpha, beta, gamma, tx, ty, tz), dR = Rz(gamma) Ry(beta) Rx(alpha), and the
+ * transform becomes fp32(dR R, dR t + (tx, ty, tz)), computed in double from the fp32 transform.  A kept set that constrains
+ * only some directions (one plane: rank 3) moves the pose in those alone, with the minimum-norm update; normals that are all
+ * zero leave it in place, and the loop stops at the second ratio test.  A non-finite energy (overflow or NaN) returns the pose
+ * as given with energy_out = +Inf.
+ * PGP_E_INVALID in addition: the model slot was set with val_nrm == NULL. */
+PGP_API int pgp_tricp_plane(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int ns, double* poses16_host, int k,
+                            float trim, float ratio, int max_iter, int* iters_out, float* energy_out);
 
 /* ---------------------------------------------------------------- K6: MCTS node helpers ---- */
 

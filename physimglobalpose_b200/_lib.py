@@ -81,6 +81,7 @@ _SIGNATURES = {
     "pgp_mcts_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _vp, _i, _f, _f, _i, _vp, _vp, _vp]),
     "pgp_prepare_segment": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _f, _f, _f, _i, _vp, _vp, _i, _vp]),
     "pgp_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),
+    "pgp_tricp_plane": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),
     "pgp_set_mesh": (_i, [_vp, _i, _vp, _i, _vp, _i, _i]),
     "pgp_set_depth_observation": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp]),
     "pgp_render_depth": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
@@ -118,6 +119,7 @@ _SIGNATURES = {
     "pgp_generated_cap_split": (_i, [_vp, _i, _i64, _i, _vp, _vp, _vp]),
     "pgp_host_chain_sum_equal": (C.c_float, [C.c_float, C.c_longlong]),
     "pgp_host_max_eigvec4": (_i, [_vp, _vp]),
+    "pgp_host_solve_plane6": (_i, [_vp, _vp, _vp]),
 }
 
 _lib = None

@@ -12,6 +12,8 @@
 // (ring search with a proven stop bound), radix-select of the n_keep-th smallest squared distance,
 // 16 double sums (energy, two centroids, 3x3 cross products) block-reduced, Horn's closed-form
 // rotation from the 4x4 symmetric eigenproblem (Jacobi) -- the same fit as SVD/Umeyama without scale.
+// pgp_tricp_plane (utilities::pointToPlaneICP, utilities.cpp:709-739) runs the same kernel with the point-to-plane fit instead:
+// 28 double sums in two passes, a 6x6 truncated pseudo-inverse solve, and PCL's Rz Ry Rx update (restated, parity unpinned).
 #include <cooperative_groups.h>
 #include <float.h>
 #include <math.h>
@@ -35,6 +37,7 @@ struct TricpParams {
   float* T;                      // k x 12, in/out (source -> target)
   int n_keep; float ratio; int max_iter;
   int* iters; float* energy;
+  const float4* nrm_orig;        // unit normals of tgt_orig, same order (point-to-plane fit)
 };
 
 __global__ void k5_tgrid_count(const float4* __restrict__ pts, int n, TGrid tg, uint32_t* __restrict__ cell_of, uint32_t* __restrict__ counts) {
@@ -214,20 +217,181 @@ __device__ void rigid_fit(double n, const double* S, float* T) {
   }
 }
 
+// x = H^+ g for the 6x6 normal equations of the point-to-plane fit (symmetric positive semi-definite H, row-major): Jacobi scaling
+// s_j = 1 / sqrt(H_jj) (0 where H_jj <= 0), M = S H S = V diag(lambda) V^T by cyclic Jacobi in double (rows p < q in order; stop
+// when the off-diagonal norm is <= 1e-15 |M|_F, or after 30 sweeps), every lambda <= 1e-9 lambda_max dropped (all of them when
+// lambda_max <= 0), x = S V diag(lambda^+) V^T S g.  The truncation gives the minimum-norm update when the kept points leave
+// directions free (one face of a box: rank 3).  Returns the number of eigenvalues kept.
+#ifdef __CUDA_ARCH__
+#define K5_ROLLED _Pragma("unroll 1")      // one thread runs this: keep M and V in local memory rather than spill an unrolled copy
+#else
+#define K5_ROLLED
+#endif
+__host__ __device__ int solve_plane6(const double H[36], const double g[6], double x[6]) {
+  double s[6], M[6][6], V[6][6];
+  for (int j = 0; j < 6; ++j) s[j] = H[7 * j] > 0.0 ? 1.0 / sqrt(H[7 * j]) : 0.0;
+  double f2 = 0.0;
+  for (int i = 0; i < 6; ++i)
+    for (int j = 0; j < 6; ++j) { M[i][j] = (s[i] * H[6 * i + j]) * s[j]; V[i][j] = (i == j); f2 += M[i][j] * M[i][j]; }
+  K5_ROLLED
+  for (int sweep = 0; sweep < 30; ++sweep) {
+    double off = 0.0;
+    for (int i = 0; i < 6; ++i) for (int j = 0; j < 6; ++j) if (i != j) off += M[i][j] * M[i][j];
+    if (!(off > 1e-30 * f2)) break;
+    K5_ROLLED
+    for (int p = 0; p < 6; ++p)
+      K5_ROLLED
+      for (int q = p + 1; q < 6; ++q) {
+        if (M[p][q] == 0.0) continue;
+        const double theta = (M[q][q] - M[p][p]) / (2.0 * M[p][q]);
+        const double t = (theta >= 0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+        const double cs = 1.0 / sqrt(t * t + 1.0), sn = t * cs;
+        for (int k = 0; k < 6; ++k) { const double mkp = M[k][p], mkq = M[k][q]; M[k][p] = cs * mkp - sn * mkq; M[k][q] = sn * mkp + cs * mkq; }
+        for (int k = 0; k < 6; ++k) { const double mpk = M[p][k], mqk = M[q][k]; M[p][k] = cs * mpk - sn * mqk; M[q][k] = sn * mpk + cs * mqk; }
+        for (int k = 0; k < 6; ++k) { const double vkp = V[k][p], vkq = V[k][q]; V[k][p] = cs * vkp - sn * vkq; V[k][q] = sn * vkp + cs * vkq; }
+      }
+  }
+  double lmax = M[0][0];
+  for (int k = 1; k < 6; ++k) lmax = fmax(lmax, M[k][k]);
+  double w[6];
+  int rank = 0;
+  for (int k = 0; k < 6; ++k) {
+    double u = 0.0;
+    for (int i = 0; i < 6; ++i) u += V[i][k] * (s[i] * g[i]);
+    const bool keep = lmax > 0.0 && M[k][k] > 1e-9 * lmax;
+    w[k] = keep ? u / M[k][k] : 0.0;
+    rank += keep;
+  }
+  for (int i = 0; i < 6; ++i) {
+    double v = 0.0;
+    for (int k = 0; k < 6; ++k) v += V[i][k] * w[k];
+    x[i] = s[i] * v;
+  }
+  return rank;
+}
+
+// dR = Rz(gamma) Ry(beta) Rx(alpha) from x = (alpha, beta, gamma, ...): the construction of PCL's
+// TransformationEstimationPointToPlaneLLS as recalled (not vendored: restated, parity unpinned), in this association.
+__host__ __device__ void euler_zyx(const double x[3], double R[3][3]) {
+  const double ca = cos(x[0]), sa = sin(x[0]), cb = cos(x[1]), sb = sin(x[1]), cg = cos(x[2]), sg = sin(x[2]);
+  R[0][0] = cg * cb; R[0][1] = -sg * ca + (cg * sb) * sa; R[0][2] = sg * sa + (cg * sb) * ca;
+  R[1][0] = sg * cb; R[1][1] = cg * ca + (sg * sb) * sa;  R[1][2] = -cg * sa + (sg * sb) * ca;
+  R[2][0] = -sb;     R[2][1] = cb * sa;                   R[2][2] = cb * ca;
+}
+
+// One Gauss-Newton step of the point-to-plane fit from the 28 sums S = {E, sum a r (6), H upper triangle row by row (21)}:
+// x = H^+ g with g = -sum a r, T <- fp32(dR R_T, ((dR_0 t_T + dR_1 t_T) + dR_2 t_T) + dt) in double from the fp32 T.
+__device__ __noinline__ void plane_fit(const double* S, float* T) {
+  double H[36], g[6], x[6], R[3][3];
+  for (int i = 0, k = 7; i < 6; ++i)
+    for (int j = i; j < 6; ++j, ++k) H[6 * i + j] = H[6 * j + i] = S[k];
+  for (int j = 0; j < 6; ++j) g[j] = -S[1 + j];
+  solve_plane6(H, g, x);
+  euler_zyx(x, R);
+  float Tn[12];
+  for (int i = 0; i < 3; ++i)
+    for (int c = 0; c < 4; ++c) {
+      const double v = (R[i][0] * (double)T[c] + R[i][1] * (double)T[4 + c]) + R[i][2] * (double)T[8 + c];
+      Tn[4 * i + c] = (float)(c == 3 ? v + x[3 + i] : v);
+    }
+  for (int k = 0; k < 12; ++k) T[k] = Tn[k];
+}
+
+// Sums over the kept correspondences of this CTA's half into acc[16]: d2 below tau, and the values equal to tau admitted in source
+// order (CTA 0 holds the lower indices) until `rank` of them are in.  term(i, acc) adds point i's contributions.
+template <class Term>
+__device__ __forceinline__ void kept_sums(const float* d2, int i_lo, int i_hi, uint32_t tau, uint32_t rank, uint32_t eq_seen, bool all_eq,
+                                          uint32_t* s_warp, int tid, int lane, int warp, double acc[16], Term term) {
+#pragma unroll
+  for (int k = 0; k < 16; ++k) acc[k] = 0.0;
+  for (int i0 = i_lo; i0 < i_hi; i0 += TT) {
+    const int i = i0 + tid;
+    const uint32_t b = i < i_hi ? __float_as_uint(d2[i]) : 0xffffffffu;
+    const bool eq = i < i_hi && b == tau;
+    uint32_t before = 0, total = 0;
+    if (!all_eq) {                                 // (uniform over the cluster)
+      const unsigned bal = __ballot_sync(0xffffffffu, eq);
+      if (lane == 0) s_warp[warp] = __popc(bal);
+      __syncthreads();
+      before = eq_seen;
+      for (int w = 0; w < TT / 32; ++w) { const uint32_t c = s_warp[w]; if (w < warp) before += c; total += c; }
+      before += __popc(bal & ((1u << lane) - 1u));
+    }
+    const bool keep = i < i_hi && (b < tau || (eq && (all_eq || before < rank)));
+    if (keep) term(i, acc);
+    eq_seen += total;
+    if (!all_eq) __syncthreads();
+  }
+}
+
+// Block sum of acc[16] into out[16] (thread 0..15 write), in a fixed order: lanes by the butterfly below, warps in order.
+__device__ __forceinline__ void block_sum16(double acc[16], double (*s_red)[16], double* out, int tid, int lane, int warp) {
+  // 16 sums over the warp with 16 shuffles instead of 80: at every butterfly step a lane hands HALF of its partial sums to its
+  // partner and keeps the other half, so the values per lane halve while the lanes per value double; lane l ends with the
+  // complete sum number (bits 4..1 of l)
+#pragma unroll
+  for (int half = 8, off = 16; half >= 1; half >>= 1, off >>= 1) {
+    const bool upper = (lane & off) != 0;
+#pragma unroll
+    for (int j = 0; j < half; ++j) {
+      const double send = upper ? acc[j] : acc[j + half];
+      const double keep = upper ? acc[j + half] : acc[j];
+      acc[j] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+    }
+  }
+  acc[0] += __shfl_xor_sync(0xffffffffu, acc[0], 1);
+  if (!(lane & 1)) s_red[warp][((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1)] = acc[0];
+  __syncthreads();
+  if (tid < 16) { double v = 0; for (int w = 0; w < TT / 32; ++w) v += s_red[w][tid]; out[tid] = v; }
+}
+
+// Point-to-plane sums of kept point i, pass PASS of two: entries [16 PASS, 16 PASS + 16) of
+// {r^2, a r (6), a_j a_k for j <= k row by row (21), 0 (4)} with a = [p' x n, n], r = n . (p' - q), all in double.
+template <int PASS>
+__device__ __forceinline__ void plane_terms(const TricpParams& p, const float* sT, const int* nn, int i, double acc[16]) {
+  const float4 s = p.src[i];
+  const float qx = sT[0] * s.x + sT[1] * s.y + sT[2] * s.z + sT[3];
+  const float qy = sT[4] * s.x + sT[5] * s.y + sT[6] * s.z + sT[7];
+  const float qz = sT[8] * s.x + sT[9] * s.y + sT[10] * s.z + sT[11];
+  const float4 n = p.nrm_orig[nn[i]];
+  const double px = qx, py = qy, pz = qz, nx = n.x, ny = n.y, nz = n.z;
+  const double a[6] = {py * nz - pz * ny, pz * nx - px * nz, px * ny - py * nx, nx, ny, nz};
+  double v[32];
+  if (PASS == 0) {
+    const float4 g = p.tgt_orig[nn[i]];
+    const double r = ((px - (double)g.x) * nx + (py - (double)g.y) * ny) + (pz - (double)g.z) * nz;
+    v[0] = r * r;
+#pragma unroll
+    for (int j = 0; j < 6; ++j) v[1 + j] = a[j] * r;
+  }
+#pragma unroll
+  for (int j = 0, k = 7; j < 6; ++j)
+#pragma unroll
+    for (int l = j; l < 6; ++l, ++k) v[k] = a[j] * a[l];
+#pragma unroll
+  for (int k = 0; k < 16; ++k)
+    if (16 * PASS + k < 28) acc[k] += v[16 * PASS + k];
+}
+
 // Two CTAs (one thread-block cluster) per pose: CTA r owns the source points [r * ceil(ns / 2), ...) -- their correspondences, their
-// share of the radix-select histograms and of the 16 sums.  The halves meet through distributed shared memory: after a cluster
+// share of the radix-select histograms and of the sums.  The halves meet through distributed shared memory: after a cluster
 // barrier each CTA adds the partner's histogram (or partial sums) to its own IN THE SAME ORDER, so both take identical decisions
 // and carry identical transforms -- nothing is broadcast, and the serial fit runs redundantly on both.  64 poses then fill 128 of
 // the 148 SMs and the per-iteration critical path (the slowest pose decides the kernel's time) halves.
+// PLANE = false: the point-to-point fit (16 sums, Horn).  PLANE = true: the point-to-plane fit; its 28 sums do not fit the
+// 64-register budget of a 1024-thread CTA next to the search, so they take two passes of 16 over the kept set (the second one
+// 12 sums and 4 zeros), each through the same butterfly into its own half of s_part.
+template <bool PLANE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kernel(const TricpParams p) {
   namespace cg = cooperative_groups;
   cg::cluster_group cl = cg::this_cluster();
+  constexpr int NS = PLANE ? 32 : 16;    // sums exchanged between the CTAs
   __shared__ float sT[12];
   __shared__ uint32_t s_hist[2][256];    // double-buffered by pass parity: the partner may still read pass p while pass p+1 fills
   __shared__ uint32_t s_sel[4];          // prefix, remaining rank, CTA 0's count of values equal to tau
   __shared__ uint32_t s_warp[TT / 32];
   __shared__ double s_red[TT / 32][16];
-  __shared__ double s_part[16];
+  __shared__ double s_part[NS];
   __shared__ int s_cont;
   const unsigned cr = cl.block_rank();
   const uint32_t* r_hist = cl.map_shared_rank(&s_hist[0][0], cr ^ 1u);
@@ -303,25 +467,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
     cap2 = fmaxf(4.0f * __uint_as_float(tau), 1e-12f);
     // 3. sums over the kept correspondences (equal-to-tau ones admitted in index order: CTA 0 holds the lower indices)
     double acc[16];
-#pragma unroll
-    for (int k = 0; k < 16; ++k) acc[k] = 0.0;
-    uint32_t eq_seen = cr ? s_sel[2] : 0u;
+    const uint32_t eq_seen = cr ? s_sel[2] : 0u;
     const bool all_eq = s_sel[3] == rank;          // every value equal to tau is kept (the usual case: tau is unique): no ordering needed
-    for (int i0 = i_lo; i0 < i_hi; i0 += TT) {
-      const int i = i0 + tid;
-      const uint32_t b = i < i_hi ? __float_as_uint(d2[i]) : 0xffffffffu;
-      const bool eq = i < i_hi && b == tau;
-      uint32_t before = 0, total = 0;
-      if (!all_eq) {                                 // (uniform over the cluster)
-        const unsigned bal = __ballot_sync(0xffffffffu, eq);
-        if (lane == 0) s_warp[warp] = __popc(bal);
-        __syncthreads();
-        before = eq_seen;
-        for (int w = 0; w < TT / 32; ++w) { const uint32_t c = s_warp[w]; if (w < warp) before += c; total += c; }
-        before += __popc(bal & ((1u << lane) - 1u));
-      }
-      const bool keep = i < i_hi && (b < tau || (eq && (all_eq || before < rank)));
-      if (keep) {
+    if constexpr (PLANE) {
+      kept_sums(d2, i_lo, i_hi, tau, rank, eq_seen, all_eq, s_warp, tid, lane, warp, acc,
+                [&](int i, double* a) { plane_terms<0>(p, sT, nn, i, a); });
+      block_sum16(acc, s_red, s_part, tid, lane, warp);
+      __syncthreads();                             // s_red is refilled by the second pass
+      kept_sums(d2, i_lo, i_hi, tau, rank, eq_seen, all_eq, s_warp, tid, lane, warp, acc,
+                [&](int i, double* a) { plane_terms<1>(p, sT, nn, i, a); });
+      block_sum16(acc, s_red, s_part + 16, tid, lane, warp);
+    } else {
+      kept_sums(d2, i_lo, i_hi, tau, rank, eq_seen, all_eq, s_warp, tid, lane, warp, acc, [&](int i, double* acc) {
         const float4 s = p.src[i];
         const float4 g = p.tgt_orig[nn[i]];
         acc[0] += (double)d2[i];
@@ -330,37 +487,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
         acc[7] += (double)s.x * g.x; acc[8] += (double)s.x * g.y; acc[9] += (double)s.x * g.z;
         acc[10] += (double)s.y * g.x; acc[11] += (double)s.y * g.y; acc[12] += (double)s.y * g.z;
         acc[13] += (double)s.z * g.x; acc[14] += (double)s.z * g.y; acc[15] += (double)s.z * g.z;
-      }
-      eq_seen += total;
-      if (!all_eq) __syncthreads();
+      });
+      block_sum16(acc, s_red, s_part, tid, lane, warp);
     }
-    // 16 sums over the warp with 16 shuffles instead of 80: at every butterfly step a lane hands HALF of its partial sums to its
-    // partner and keeps the other half, so the values per lane halve while the lanes per value double; lane l ends with the
-    // complete sum number (bits 4..1 of l)
-#pragma unroll
-    for (int half = 8, off = 16; half >= 1; half >>= 1, off >>= 1) {
-      const bool upper = (lane & off) != 0;
-#pragma unroll
-      for (int j = 0; j < half; ++j) {
-        const double send = upper ? acc[j] : acc[j + half];
-        const double keep = upper ? acc[j + half] : acc[j];
-        acc[j] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-      }
-    }
-    acc[0] += __shfl_xor_sync(0xffffffffu, acc[0], 1);
-    if (!(lane & 1)) s_red[warp][((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1)] = acc[0];
-    __syncthreads();
-    if (tid < 16) { double v = 0; for (int w = 0; w < TT / 32; ++w) v += s_red[w][tid]; s_part[tid] = v; }
     cl.sync();
     if (tid == 0) {
-      double S[16];
-      for (int k = 0; k < 16; ++k) S[k] = cr ? r_part[k] + s_part[k] : s_part[k] + r_part[k];      // CTA 0's half + CTA 1's half, in both
+      double S[NS];
+      for (int k = 0; k < NS; ++k) S[k] = cr ? r_part[k] + s_part[k] : s_part[k] + r_part[k];      // CTA 0's half + CTA 1's half, in both
       old_energy = energy;
       energy = (float)S[0];
+      if (PLANE && !(energy <= FLT_MAX)) energy = INFINITY;      // (a NaN residual reports +Inf, as an overflowing one does)
       if (energy <= FLT_MAX) {                     // a kept squared distance overflowed: no fit, and the ratio test below stops
-        float Tn[12];
-        rigid_fit((double)p.n_keep, S + 1, Tn);
-        for (int k = 0; k < 12; ++k) sT[k] = Tn[k];
+        if constexpr (PLANE) {
+          plane_fit(S, sT);
+        } else {
+          float Tn[12];
+          rigid_fit((double)p.n_keep, S + 1, Tn);
+          for (int k = 0; k < 12; ++k) sT[k] = Tn[k];
+        }
       }
       ++it;
       s_cont = ((energy / old_energy) < p.ratio && it < p.max_iter) ? 1 : 0;
@@ -441,9 +585,15 @@ extern "C" PGP_API int pgp_host_max_eigvec4(const double* N16, double* q4) {
   return max_eigvec4(N, q4) ? 1 : 0;
 }
 
+// host-callable copy of solve_plane6 (the 6x6 solve of the point-to-plane fit) for the CPU test-suite: H36 row-major symmetric,
+// x6 = H^+ g6 as the kernel computes it; returns the number of eigenvalues kept
+extern "C" PGP_API int pgp_host_solve_plane6(const double* H36, const double* g6, double* x6) {
+  return solve_plane6(H36, g6, x6);
+}
+
 
 int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* poses16_host, int k, float trim, float ratio, int max_iter,
-             int* iters_out, float* energy_out) {
+             int* iters_out, float* energy_out, bool plane) {
   TScratch& ts = tscratch_of(ctx);
   int rc = build_target_grid(ctx, m);
   if (rc) return rc;
@@ -493,11 +643,13 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   TricpParams p{};
   p.src = ts.seg.as<float4>(); p.ns = ns;
   p.tgt = m.tgrid_pts.as<float4>(); p.tstart = m.tgrid_start.as<uint32_t>(); p.nt = m.nv; p.tgt_orig = m.val_raw.as<float4>();
+  p.nrm_orig = m.val_nrm_orig.as<float4>();
   memcpy(p.tg.lo, m.tg_lo, 12); p.tg.g = m.tg_g; p.tg.inv_g = 1.0f / m.tg_g; memcpy(p.tg.dim, m.tg_dim, 12);
   p.d2 = ts.d2.as<float>(); p.nn = ts.nn.as<int>(); p.T = ts.T.as<float>();
   p.n_keep = n_keep; p.ratio = ratio; p.max_iter = std::max(1, max_iter);
   p.iters = ts.iters.as<int>(); p.energy = ts.energy.as<float>();
-  k5_tricp_kernel<<<2 * k, TT, 0, ctx->stream>>>(p);      // one cluster of two CTAs per pose
+  if (plane) k5_tricp_kernel<true><<<2 * k, TT, 0, ctx->stream>>>(p);     // one cluster of two CTAs per pose
+  else k5_tricp_kernel<false><<<2 * k, TT, 0, ctx->stream>>>(p);
   ctx->launches++;
   PGP_CUDA(ctx, cudaGetLastError());
   PGP_CUDA(ctx, cudaMemcpyAsync(T.data(), ts.T.p, (size_t)k * 48, cudaMemcpyDeviceToHost, ctx->stream));

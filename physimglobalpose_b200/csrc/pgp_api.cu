@@ -227,7 +227,7 @@ int pgp_set_model(pgp_ctx* ctx, int obj, const float* sx, const float* sn, int n
   if (!sx || nq <= 0 || !vx || nv <= 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_model: empty cloud");
   Model& m = ctx->models[obj];
   m.ready = false;
-  m.nq = nq; m.nv = nv; m.n_gen = 0; m.tgrid_ready = false; m.val_rinf = 0.f;
+  m.nq = nq; m.nv = nv; m.n_gen = 0; m.tgrid_ready = false; m.val_rinf = 0.f; m.val_has_nrm = vn != nullptr;
   seq_centroid(sx, nq, m.cQ);   // centroid of the SEARCH cloud centres both clouds (:248-261)
   std::vector<float> s4((size_t)nq * 4), sn4((size_t)nq * 4), v4((size_t)nv * 4), vn4((size_t)nv * 4);
   for (int i = 0; i < nq; ++i) {
@@ -801,7 +801,20 @@ int pgp_tricp(pgp_ctx* ctx, int obj, const float* seg, int ns, double* poses, in
   if (!(trim > 0.f) || !(ratio > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp: trim and ratio must be > 0");
   if (!tricp_inputs_finite(seg, ns, poses, k)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp: non-finite segment point or pose");
   if (k == 0) return PGP_OK;
-  return k5_tricp(ctx, *m, seg, ns, poses, k, trim, ratio, max_iter, iters, energy);
+  return k5_tricp(ctx, *m, seg, ns, poses, k, trim, ratio, max_iter, iters, energy, false);
+}
+
+int pgp_tricp_plane(pgp_ctx* ctx, int obj, const float* seg, int ns, double* poses, int k, float trim, float ratio, int max_iter, int* iters,
+                    float* energy) {
+  CHECK_CTX(ctx);
+  Model* m = get_model(ctx, obj);
+  if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "no model in slot %d", obj);
+  if (!m->val_has_nrm) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp_plane: model slot %d was set without validation normals", obj);
+  if (!seg || ns <= 0 || !poses || k < 0) return pgp_fail(ctx, PGP_E_INVALID, "bad argument");
+  if (!(trim > 0.f) || !(ratio > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp_plane: trim and ratio must be > 0");
+  if (!tricp_inputs_finite(seg, ns, poses, k)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_tricp_plane: non-finite segment point or pose");
+  if (k == 0) return PGP_OK;
+  return k5_tricp(ctx, *m, seg, ns, poses, k, trim, ratio, max_iter, iters, energy, true);
 }
 
 }  // extern "C"
@@ -837,7 +850,7 @@ int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg, int ns, const double
     if (!flag[i]) { memcpy(&un[3 * (size_t)w], seg + 3 * (size_t)i, 12); ++w; }
   if (n_unexplained) *n_unexplained = kept;
   if (kept == 0) { for (int i = 0; i < k; ++i) { if (iters) iters[i] = 0; if (energy) energy[i] = 0.f; } return PGP_OK; }
-  return k5_tricp(ctx, *m, un.data(), kept, poses, k, trim, ratio, max_iter, iters, energy);
+  return k5_tricp(ctx, *m, un.data(), kept, poses, k, trim, ratio, max_iter, iters, energy, false);
 }
 
 int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, int class_id, const float* K9,

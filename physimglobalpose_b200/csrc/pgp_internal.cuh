@@ -114,6 +114,7 @@ struct Model {
   DevBuf val_groups;   // ceil(nv/32) x float4: bounding sphere {centre, radius} of each run of 32 points of `val` (K3 group cull)
   DevBuf val_orig;     // nv x float4 centred, ORIGINAL order (weighted mode with general priors, TrICP target)
   DevBuf val_nrm_orig;
+  bool val_has_nrm = false;   // pgp_set_model was given validation normals (the point-to-plane fit needs them)
   // model-space grid for TrICP (K5): nearest validation-model point of any query
   DevBuf val_raw;        // nv x float4, model frame as given (un-centred): the TrICP target
   float val_raw_lo[3] = {0, 0, 0}, val_raw_hi[3] = {0, 0, 0};
@@ -242,8 +243,9 @@ void k5_release(pgp_ctx* ctx);
 void k6_release(pgp_ctx* ctx);
 void k7_release(pgp_ctx* ctx);
 // k5_tricp.cu
+// plane: the point-to-plane fit (pgp_tricp_plane) instead of the point-to-point one (pgp_tricp)
 int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* poses16_host, int k, float trim, float ratio,
-             int max_iter, int* iters_out, float* energy_out);
+             int max_iter, int* iters_out, float* energy_out, bool plane);
 
 // ---------------------------------------------------------------------------------------------
 // fp32 arithmetic in the reference's association, every operation individually rounded

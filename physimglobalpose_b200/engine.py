@@ -387,6 +387,17 @@ class PoseEngine:
                                         _ptr(iters), _ptr(energy)))
         return P.reshape(-1, 4, 4), iters, energy
 
+    def tricp_plane(self, obj: int, segment_xyz, poses44, trim: float = 0.5, ratio: float = 0.99, max_iter: int = 100):
+        """Trimmed point-to-plane ICP (utilities::pointToPlaneICP): tricp's search, trim and stop, fitted to the validation normals
+        with 6x6 normal equations.  Returns (refined poses, iterations, point-to-plane trimmed energies)."""
+        seg = _f32(segment_xyz, 3)
+        P = np.ascontiguousarray(poses44, dtype=np.float64).reshape(-1, 16).copy()
+        iters = np.zeros(len(P), np.int32)
+        energy = np.zeros(len(P), np.float32)
+        self._check(self._lib.pgp_tricp_plane(self._ctx, obj, _ptr(seg), len(seg), _ptr(P), len(P), float(trim), float(ratio), int(max_iter),
+                                              _ptr(iters), _ptr(energy)))
+        return P.reshape(-1, 4, 4), iters, energy
+
     # ------------------------------------------------------------------ K6
     def remove_explained(self, obj: int, segment_xyz, placed_poses44, threshold: float = 0.008) -> np.ndarray:
         """Boolean mask of the segment points EXPLAINED by the placed objects (UCTState.cpp:149-174)."""
