@@ -122,8 +122,9 @@ PGP_API int pgp_centred_to_pose(pgp_ctx* ctx, int obj, const float* T12, double*
 PGP_API int pgp_grid_info(pgp_ctx* ctx, int* dims3, int64_t* n_cells, int64_t* n_occupied, float* cell, int64_t* bytes);
 
 /* Statistics of the tri-state label structure K1b builds over the grid (no reference counterpart; reports and
- * tuning): out8 = {cells whose 512 sub-voxels are all OUT, all IN, mixed; sub-voxels OUT, IN, AMBIG; words of
- * AMBIG candidate lists; entries of the nearest-candidate lists (0 until a WEIGHTED call built them)}. */
+ * tuning): out8 = {cells whose 512 sub-voxels are all OUT, all IN, mixed; sub-voxels OUT, IN, AMBIG; overflow
+ * records of the AMBIG candidate lists (candidates beyond the two each AMBIG voxel keeps inline); entries of the
+ * nearest-candidate lists (0 until a WEIGHTED call built them)}. */
 PGP_API int pgp_label_stats(pgp_ctx* ctx, int64_t* out8);
 
 /* ---------------------------------------------------------------- K3: LCP scoring ---------- */

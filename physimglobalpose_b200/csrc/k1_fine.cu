@@ -49,7 +49,8 @@ __global__ void k1f_bmrank(const uint32_t* __restrict__ bitmap, const uint32_t* 
 }
 
 // one CTA per block (= per cell with an occupied 27-neighbourhood): 4 sub-voxels per thread.
-// Pass A: labels + per-voxel number of "near" points (candidates of the exact test) + block header.
+// Pass A: labels + per-voxel number of "near" points (candidates of the exact test) + block header.  The block's record region is
+// sized for the OVERFLOW records only (beyond the two every AMBIG voxel keeps in its slot, see k1f_fill_lists).
 __global__ void __launch_bounds__(CLS_THREADS) k1f_classify(const uint32_t* __restrict__ block_cell, const uint32_t* __restrict__ cell_start,
                                                             const float4* __restrict__ pts, GridParams g, uint32_t* __restrict__ codes,
                                                             uint16_t* __restrict__ near_cnt, uint32_t* __restrict__ hdr,
@@ -114,7 +115,7 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_classify(const uint32_t* __re
     if (code == 2 && near[j] > 65535) atomicOr(overflow, 1);      // absurd density: the host drops the fine grid
     const int nn = code == 2 ? min(near[j], 65535) : 0;
     near_cnt[(size_t)b * 512 + v] = (uint16_t)nn;
-    my_list += (uint32_t)nn;
+    my_list += (uint32_t)max(nn - 2, 0);
   }
   my_list = __reduce_add_sync(0xffffffffu, my_list);
   if ((threadIdx.x & 31) == 0 && my_list) atomicAdd(&s_tot, my_list);
@@ -124,7 +125,7 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_classify(const uint32_t* __re
 #pragma unroll
     for (int k = 0; k < 16; ++k) w |= (uint32_t)s_code[threadIdx.x * 16 + k] << (2 * k);
     codes[(size_t)b * 32 + threadIdx.x] = w;
-    // header: ambig-rank prefix per group of 64 voxels (4 words), number of ambig voxels, list words
+    // header: ambig-rank prefix per group of 64 voxels (4 words), number of ambig voxels, overflow records
     const uint32_t amb = __popc(w & 0xAAAAAAAAu);
     uint32_t incl = amb;
 #pragma unroll
@@ -147,24 +148,25 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_classify(const uint32_t* __re
   }
 }
 
-// Pass B: candidate lists of the AMBIG voxels, laid out for K3's phase 2:
+// Pass B: candidate lists of the AMBIG voxels, laid out for K3's phase 2.  A voxel's candidates are every scene point whose distance
+// to the (inflated) voxel is <= delta (1 + 1e-5), minus the dominated ones, with the candidate closest to the voxel centre FIRST (the
+// most likely hit: K3's existence test stops at the first point within delta):
 //   hdrw[b * 32 + w]  = global rank of the first AMBIG voxel of label word w of block b (ranks run over all blocks, voxel order),
-//   adesc[rank]       = {first record, number of records} of that AMBIG voxel,
-//   arec[...]         = float4 COPIES {x, y, z, original index} of its candidates -- every scene point whose distance to the
-//                       (inflated) voxel is <= delta (1 + 1e-5) -- with the candidate closest to the voxel centre FIRST (the
-//                       most likely hit: K3's existence test stops at the first point within delta).
-// A query that fell into an AMBIG voxel reaches its candidates with two indexed loads (hdrw, adesc) and no second indirection.
+//   aslot[rank]       = one 32-byte slot per AMBIG voxel, two float4 {x0, y0, z0, n} {x1, y1, z1, first overflow record}: the first
+//                       two candidates (the second is a copy of the first when n = 1) and the number of candidates n >= 1,
+//   aovf[...]         = float4 copies {x, y, z, original index} of candidates 3 .. n, in list order.
+// A query that fell into an AMBIG voxel reads hdrw, then one sector; only when both inline candidates miss and n > 2 does it go on.
 __global__ void __launch_bounds__(CLS_THREADS) k1f_fill_lists(const uint32_t* __restrict__ block_cell, const uint32_t* __restrict__ cell_start,
                                                               const float4* __restrict__ pts, GridParams g, const uint32_t* __restrict__ codes,
                                                               const uint16_t* __restrict__ near_cnt, const uint32_t* __restrict__ hdr,
-                                                              const uint32_t* __restrict__ rec_base, const uint32_t* __restrict__ amb_base,
-                                                              uint32_t* __restrict__ hdrw, uint2* __restrict__ adesc, float4* __restrict__ arec) {
+                                                              const uint32_t* __restrict__ ovf_base, const uint32_t* __restrict__ amb_base,
+                                                              uint32_t* __restrict__ hdrw, float4* __restrict__ aslot, float4* __restrict__ aovf) {
   __shared__ float4 s_p[CLS_CHUNK];
   __shared__ uint16_t s_av[F * F * F];       // AMBIG voxels in rank order
-  __shared__ uint32_t s_off[F * F * F + 1];  // their list offsets within the block's record region
+  __shared__ uint32_t s_off[F * F * F + 1];  // their overflow offsets within the block's region
   const int b = blockIdx.x;
   const uint32_t n_amb = hdr[(size_t)b * 8 + 5];
-  const uint32_t abase = amb_base[b], rbase = rec_base[b];
+  const uint32_t abase = amb_base[b], obase = ovf_base[b];
   // rank order = voxel order; per-word rank prefixes + the compact voxel list from the code words
   if (threadIdx.x < 32) {
     const uint32_t w = codes[(size_t)b * 32 + threadIdx.x] & 0xAAAAAAAAu;
@@ -185,7 +187,7 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_fill_lists(const uint32_t* __
     uint32_t run = 0;
     for (uint32_t r0 = 0; r0 < n_amb; r0 += 32) {
       const uint32_t r = r0 + threadIdx.x;
-      uint32_t cnt = r < n_amb ? near_cnt[(size_t)b * 512 + s_av[r]] : 0u, incl = cnt;
+      uint32_t cnt = r < n_amb ? (uint32_t)max((int)near_cnt[(size_t)b * 512 + s_av[r]] - 2, 0) : 0u, incl = cnt;
 #pragma unroll
       for (int o = 1; o < 32; o <<= 1) { uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if ((int)threadIdx.x >= o) incl += t; }
       if (r < n_amb) s_off[r] = run + incl - cnt;
@@ -194,20 +196,26 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_fill_lists(const uint32_t* __
     if (threadIdx.x == 0) s_off[n_amb] = run;
   }
   __syncthreads();
-  // fill: thread t owns AMBIG voxels t, t+128, ... (up to 4)
+  // fill: thread t owns AMBIG voxels t, t+128, ... (up to 4).  Candidate k of the sweep goes to slot half k (k < 2) or to overflow
+  // record k - 2; afterwards the closest-to-centre candidate trades places with candidate 0.
   float vx[4], vy[4], vz[4], bd2[4], bx[4], by[4], bz[4];
   const float dom_margin = 1e-5f * g.dhi2;
-  uint32_t wr[4], first[4], bpos[4];
+  uint32_t n[4], ovf[4], bpos[4];
+  bool live[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const uint32_t r = threadIdx.x + CLS_THREADS * j;
-    const int v = r < n_amb ? s_av[r] : 0;
+    live[j] = r < n_amb;
+    const int v = live[j] ? s_av[r] : 0;
     vx[j] = __fmaf_rn((float)(cx * F + (v & 7)) + 0.5f, g.hf, g.lo[0]);
     vy[j] = __fmaf_rn((float)(cy * F + ((v >> 3) & 7)) + 0.5f, g.hf, g.lo[1]);
     vz[j] = __fmaf_rn((float)(cz * F + (v >> 6)) + 0.5f, g.hf, g.lo[2]);
-    wr[j] = r < n_amb ? rbase + s_off[r] : 0xffffffffu;
-    first[j] = wr[j]; bpos[j] = wr[j]; bd2[j] = INFINITY;
+    ovf[j] = live[j] ? obase + s_off[r] : 0u;
+    n[j] = 0; bpos[j] = 0; bd2[j] = INFINITY;
   }
+  auto rec = [&](int j, uint32_t k) -> float4* {
+    return k < 2 ? aslot + 2 * (size_t)(abase + threadIdx.x + CLS_THREADS * j) + k : aovf + ovf[j] + (k - 2);
+  };
   const uint32_t active_j = (n_amb + CLS_THREADS - 1) / CLS_THREADS;
   for (int row = 0; row < 9; ++row) {
     const int oy = row % 3 - 1, oz = row / 3 - 1;
@@ -222,7 +230,7 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_fill_lists(const uint32_t* __
         const float4 p = s_p[t];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          if ((uint32_t)j < active_j && wr[j] != 0xffffffffu) {
+          if ((uint32_t)j < active_j && live[j]) {
             const float dx = p.x - vx[j], dy = p.y - vy[j], dz = p.z - vz[j];
             const float ax = fabsf(dx), ay = fabsf(dy), az = fabsf(dz);
             const float lx = fmaxf(ax - hs, 0.f), ly = fmaxf(ay - hs, 0.f), lz = fmaxf(az - hs, 0.f);
@@ -230,23 +238,23 @@ __global__ void __launch_bounds__(CLS_THREADS) k1f_fill_lists(const uint32_t* __
             if (mind2 <= g.dhi2) {
               const float c2 = __fmaf_rn(dx, dx, __fmaf_rn(dy, dy, dz * dz));
               const bool keep = !(bd2[j] < INFINITY && dominated(p, bx[j], by[j], bz[j], hs, c2, bd2[j], dom_margin));   // as k1f_classify counted
-              if (c2 < bd2[j]) { bd2[j] = c2; bx[j] = p.x; by[j] = p.y; bz[j] = p.z; if (keep) bpos[j] = wr[j]; }    // strict <: first of equals
-              if (keep) arec[wr[j]++] = p;
+              if (c2 < bd2[j]) { bd2[j] = c2; bx[j] = p.x; by[j] = p.y; bz[j] = p.z; if (keep) bpos[j] = n[j]; }    // strict <: first of equals
+              if (keep) *rec(j, n[j]++) = p;
             }
           }
         }
       }
     }
   }
-  // the candidate closest to the voxel centre goes first (own writes, same thread: program order); descriptor = what was written
+  // closest candidate first, then the slot's count and overflow offset (own writes, same thread: program order)
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
-    if ((uint32_t)j < active_j && first[j] != 0xffffffffu) {
-      if (bpos[j] != first[j]) {
-        const float4 a = arec[first[j]], bb = arec[bpos[j]];
-        arec[first[j]] = bb; arec[bpos[j]] = a;
-      }
-      adesc[abase + threadIdx.x + CLS_THREADS * j] = make_uint2(first[j], wr[j] - first[j]);
+    if ((uint32_t)j < active_j && live[j]) {
+      float4 r0 = *rec(j, 0);
+      if (bpos[j] != 0) { float4* pb = rec(j, bpos[j]); const float4 t = *pb; *pb = r0; r0 = t; }
+      const float4 r1 = n[j] > 1 ? *rec(j, 1) : r0;
+      *rec(j, 0) = make_float4(r0.x, r0.y, r0.z, __uint_as_float(n[j]));
+      *rec(j, 1) = make_float4(r1.x, r1.y, r1.z, __uint_as_float(ovf[j]));
     }
   }
 }
@@ -580,7 +588,7 @@ int k1_build_fine(pgp_ctx* ctx) {
   g.dhi2 = (float)((d * (1.0 + 1e-5)) * (d * (1.0 + 1e-5)));
   // the OUT label also needs: everything within delta(1+1e-5) + inflate of a cell lies in its 27 cells
   if (!((double)g.h * (1.0 - 4e-4) >= d * (1.0 + 1e-5) + (double)g.inflate)) return PGP_OK;   // margins do not close: no fine grid
-  s.n_list_words = 0;
+  s.n_ovf_records = 0;
   if ((size_t)nb * 32 >= ((size_t)1 << 28)) return PGP_OK;          // K3 packs (label word index, rank) into one 32-bit queue entry
   if (nb > 0) {
     PGP_CUDA(ctx, s.near_cnt.reserve((size_t)nb * 512 * 2));
@@ -588,7 +596,7 @@ int k1_build_fine(pgp_ctx* ctx) {
     PGP_CUDA(ctx, s.hdrw.reserve((size_t)nb * 128));
     PGP_CUDA(ctx, s.region.reserve((size_t)(nb + 1) * 8));
     PGP_CUDA(ctx, s.scratch.reserve((size_t)((nb + 1) / 2048 + 4096) * 4));
-    uint32_t* region = s.region.as<uint32_t>();            // records per block -> first record of the block
+    uint32_t* region = s.region.as<uint32_t>();            // overflow records per block -> first overflow record of the block
     uint32_t* region_amb = region + (nb + 1);              // AMBIG voxels per block -> global rank of the block's first one
     unsigned long long* d_total = reinterpret_cast<unsigned long long*>(ctx->work.as<char>() + 192);
     PGP_CUDA(ctx, cudaMemsetAsync(region, 0, (size_t)(nb + 1) * 8, st));
@@ -611,14 +619,14 @@ int k1_build_fine(pgp_ctx* ctx) {
     if (overflow || total >= (1ull << 32) - 64) return PGP_OK;     // g.fine stays 0: scoring uses the 27-cell path
     size_t free_b = 0, total_b = 0;
     PGP_CUDA(ctx, cudaMemGetInfo(&free_b, &total_b));
-    if ((size_t)total * 16 + (size_t)n_amb_total * 8 + ((size_t)256 << 20) > free_b + s.arec.cap + s.adesc.cap) return PGP_OK;
-    PGP_CUDA(ctx, s.arec.reserve((size_t)total * 16 + 16));
-    PGP_CUDA(ctx, s.adesc.reserve((size_t)n_amb_total * 8 + 16));
+    if ((size_t)total * 16 + (size_t)n_amb_total * 32 + ((size_t)256 << 20) > free_b + s.aovf.cap + s.aslot.cap) return PGP_OK;
+    PGP_CUDA(ctx, s.aovf.reserve((size_t)total * 16 + 16));
+    PGP_CUDA(ctx, s.aslot.reserve((size_t)n_amb_total * 32 + 32));     // (cudaMalloc: 256-byte aligned, so every slot is one sector)
     k1f_fill_lists<<<nb, CLS_THREADS, 0, st>>>(s.block_cell.as<uint32_t>(), s.cell_start.as<uint32_t>(), s.pts.as<float4>(), g, s.codes.as<uint32_t>(),
                                                s.near_cnt.as<uint16_t>(), s.hdr.as<uint32_t>(), region, region_amb, s.hdrw.as<uint32_t>(),
-                                               s.adesc.as<uint2>(), s.arec.as<float4>());
+                                               s.aslot.as<float4>(), s.aovf.as<float4>());
     ctx->launches++;
-    s.n_list_words = (int64_t)total;
+    s.n_ovf_records = (int64_t)total;
     s.n_ambig_voxels = (int64_t)n_amb_total;
   }
   // K1d distance field on the R-times refined lattice (R = 2 unless the grid is huge)
@@ -709,7 +717,7 @@ int k1_fine_stats(pgp_ctx* ctx, int64_t* out8) {
   PGP_CUDA(ctx, cudaMemcpyAsync(h, d, 64, cudaMemcpyDeviceToHost, ctx->stream));
   PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   for (int i = 0; i < 6; ++i) out8[i] = (int64_t)h[i];
-  out8[6] = s.n_list_words;
+  out8[6] = s.n_ovf_records;
   out8[7] = s.wlists_ready ? s.n_wlist_entries : 0;
   return PGP_OK;
 }

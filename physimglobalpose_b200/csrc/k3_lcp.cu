@@ -58,8 +58,8 @@ struct LcpParams {
   const uint32_t* codes;     // n_blocks x 32 words
   int bmrank_words;          // words staged in smem (0: read from global/L1)
   const uint32_t* hdrw;      // n_blocks x 32: global rank of the first AMBIG voxel of each label word (K1b pass B)
-  const uint2* adesc;        // per AMBIG voxel: {first record, number of records}
-  const float4* arec;        // candidate records {x, y, z, original index}, closest to the voxel centre first
+  const float4* aslot;       // per AMBIG voxel, 32 bytes: {x0, y0, z0, n} {x1, y1, z1, first overflow record}, closest to the voxel centre first
+  const float4* aovf;        // candidates 3 .. n of every AMBIG voxel {x, y, z, original index}
   float model_rinf;          // max |coordinate| of the validation model (bounds the transform's intermediates)
   const unsigned char* wcnt; // K1c: per voxel candidate count (a byte)
   const uint32_t* wword;     // K1c: per label word (16 voxels) the first record
@@ -387,22 +387,38 @@ __device__ __forceinline__ const uint32_t* wlist_of(const LcpParams& p, const Fi
   return wlist_at(p, blk, ((iz & 7) << 6) | ((iy & 7) << 3) | (ix & 7), cnt);
 }
 
+// one 32-byte slot of K1b's aslot (32-byte aligned) in ONE 256-bit load (sm_100: LDG.256): a single request and a single sector per
+// lane.  (The .v8.f32 form of the same load crashes ptxas 12.9 in this file; .v4.u64 compiles to the same instruction.)
+__device__ __forceinline__ void load_slot(const float4* __restrict__ slot, float4& a, float4& b) {
+  unsigned long long u0, u1, u2, u3;
+  asm("ld.global.nc.v4.u64 {%0, %1, %2, %3}, [%4];" : "=l"(u0), "=l"(u1), "=l"(u2), "=l"(u3) : "l"(slot));
+  a = make_float4(__uint_as_float((uint32_t)u0), __uint_as_float((uint32_t)(u0 >> 32)), __uint_as_float((uint32_t)u1), __uint_as_float((uint32_t)(u1 >> 32)));
+  b = make_float4(__uint_as_float((uint32_t)u2), __uint_as_float((uint32_t)(u2 >> 32)), __uint_as_float((uint32_t)u3), __uint_as_float((uint32_t)(u3 >> 32)));
+}
+
 // phase 2 (count mode) for one queued query: the reference's exact test against the candidate records of its AMBIG voxel.
-// `e` = (label word index << 4) | rank of the voxel among the AMBIG voxels of that word, packed by phase 1.
+// `e` = (label word index << 4) | rank of the voxel among the AMBIG voxels of that word, packed by phase 1.  The voxel's slot holds
+// its first two candidates (most lists are 1-3 long and the first, closest to the voxel centre, is the likely hit); the overflow
+// records are read only when both miss.
 __device__ __forceinline__ int resolve_ambiguous(const LcpParams& p, const Xf& x, const float4 m, uint32_t e) {
   const uint32_t r = __ldg(p.hdrw + (e >> 4)) + (e & 15u);
-  const uint2 d = __ldg(p.adesc + r);
+  float4 s0, s1;
+  load_slot(p.aslot + 2 * (size_t)r, s0, s1);
   float tx, ty, tz;
   apply_xf(x, m, tx, ty, tz);
   const float r2 = p.g.r2;
-  const float4* __restrict__ rec = p.arec + d.x;
-  // two records per round (the second load is issued before the first is tested: lists are ~2 records, and the chain of
-  // dependent loads is what this path waits on)
-  for (uint32_t j = 0; j < d.y; j += 2) {
-    const float4 s0 = __ldg(rec + j);
-    const float4 s1 = __ldg(rec + min(j + 1u, d.y - 1u));
-    if (sqdist3(tx, ty, tz, s0.x, s0.y, s0.z) <= r2) return 1;
-    if (sqdist3(tx, ty, tz, s1.x, s1.y, s1.z) <= r2) return 1;
+  if (sqdist3(tx, ty, tz, s0.x, s0.y, s0.z) <= r2) return 1;
+  if (sqdist3(tx, ty, tz, s1.x, s1.y, s1.z) <= r2) return 1;
+  const uint32_t n = __float_as_uint(s0.w);
+  if (n <= 2u) return 0;
+  const float4* __restrict__ rec = p.aovf + __float_as_uint(s1.w);
+  // two records per round (the second load is issued before the first is tested: the chain of dependent loads is what this path
+  // waits on)
+  for (uint32_t j = 0; j < n - 2u; j += 2) {
+    const float4 t0 = __ldg(rec + j);
+    const float4 t1 = __ldg(rec + min(j + 1u, n - 3u));
+    if (sqdist3(tx, ty, tz, t0.x, t0.y, t0.z) <= r2) return 1;
+    if (sqdist3(tx, ty, tz, t1.x, t1.y, t1.z) <= r2) return 1;
   }
   return 0;
 }
@@ -979,7 +995,7 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
     p.n_tiles = (m.nv + tile_cap - 1) / tile_cap;
     if (p.n_tiles > 256) return pgp_fail(ctx, PGP_E_INVALID, "validation model too large (%d points)", m.nv);
     p.bmrank = s.bmrank.as<uint2>(); p.codes = s.codes.as<uint32_t>();
-    p.hdrw = s.hdrw.as<uint32_t>(); p.adesc = s.adesc.as<uint2>(); p.arec = s.arec.as<float4>();
+    p.hdrw = s.hdrw.as<uint32_t>(); p.aslot = s.aslot.as<float4>(); p.aovf = s.aovf.as<float4>();
     p.wcnt = s.wcnt.as<unsigned char>(); p.wword = s.wword.as<uint32_t>(); p.wlists = s.wlists.as<uint32_t>(); p.vrec = s.vrec.as<uint32_t>(); p.pts_orig = s.unsorted.as<float4>(); p.aux_orig = s.aux_orig.as<float4>();
     p.bmrank_words = (int)(bm / 8);
     p.model_rinf = m.val_rinf;

@@ -110,7 +110,7 @@ void pgp_destroy(pgp_ctx* ctx) {
   cudaDeviceSynchronize();
   Scene& s = ctx->scene;
   for (DevBuf* b : {&s.xyz_raw, &s.nrm_raw, &s.unsorted, &s.cursor, &s.pts, &s.aux, &s.cell_start, &s.cell_of, &s.bitmap, &s.bmrank,
-                    &s.block_cell, &s.codes, &s.near_cnt, &s.hdr, &s.region, &s.hdrw, &s.adesc, &s.arec, &s.wvox, &s.wbase, &s.wcnt, &s.wword, &s.wlists, &s.vrec, &s.aux_orig, &s.dist, &s.dist_tmp, &s.prior, &s.scratch, &ctx->work, &ctx->topk_out})
+                    &s.block_cell, &s.codes, &s.near_cnt, &s.hdr, &s.region, &s.hdrw, &s.aslot, &s.aovf, &s.wvox, &s.wbase, &s.wcnt, &s.wword, &s.wlists, &s.vrec, &s.aux_orig, &s.dist, &s.dist_tmp, &s.prior, &s.scratch, &ctx->work, &ctx->topk_out})
     b->release();
   for (BatchSlot& bs : ctx->batch) {
     bs.T.release(); bs.counts.release(); bs.scores.release();
@@ -399,7 +399,7 @@ int pgp_grid_info(pgp_ctx* ctx, int* dims3, int64_t* n_cells, int64_t* n_occupie
   if (cell) *cell = s.g.h;
   if (bytes) {
     *bytes = (int64_t)s.n * 32 + (s.g.n_cells + 1) * 4 + s.bitmap_words * 4;
-    if (s.g.fine) *bytes += s.bitmap_words * 8 + (int64_t)s.g.n_blocks * (128 + 128) + s.n_ambig_voxels * 8 + s.n_list_words * 16 + s.g.n_cells * 4 * s.dist_r * s.dist_r * s.dist_r;   // K1b: bmrank, codes, hdrw, adesc, arec; K1d: dist
+    if (s.g.fine) *bytes += s.bitmap_words * 8 + (int64_t)s.g.n_blocks * (128 + 128) + s.n_ambig_voxels * 32 + s.n_ovf_records * 16 + s.g.n_cells * 4 * s.dist_r * s.dist_r * s.dist_r;   // K1b: bmrank, codes, hdrw, aslot, aovf; K1d: dist
     if (s.wlists_ready) *bytes += (int64_t)s.g.n_blocks * (2052 + 640 + 2048) + s.n_wlist_entries * 4 + (int64_t)s.n * 16;       // K1c: wvox, wbase, wcnt, wword, vrec, wlists, aux_orig
   }
   return PGP_OK;

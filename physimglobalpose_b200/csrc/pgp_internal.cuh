@@ -72,12 +72,12 @@ struct Scene {
   DevBuf block_cell;   // n_blocks x u32: cell of block b
   DevBuf codes;        // n_blocks x 32 words: 512 2-bit voxel states, voxel v = (sz*8+sy)*8+sx at bits 2(v&15) of word v>>4
   DevBuf near_cnt;     // build scratch: n_blocks x 512 u16 candidate counts
-  DevBuf hdr;          // build scratch: n_blocks x 8 u32: {.., #ambig voxels at [5], #candidate records at [6], ..}
+  DevBuf hdr;          // build scratch: n_blocks x 8 u32: {.., #ambig voxels at [5], #overflow records at [6], ..}
   DevBuf region;       // build scratch: region sizes / bases
   DevBuf hdrw;         // n_blocks x 32 u32: global rank of the first AMBIG voxel of each label word
-  DevBuf adesc;        // per AMBIG voxel (rank order): {first record, number of records}
-  DevBuf arec;         // float4 copies {x, y, z, original index} of the AMBIG voxels' candidate points, closest to the voxel centre first
-  int64_t n_list_words = 0;    // records in arec
+  DevBuf aslot;        // per AMBIG voxel (rank order), 32 bytes: {x0, y0, z0, n} {x1, y1, z1, first overflow record}, candidate 0 closest to the voxel centre
+  DevBuf aovf;         // float4 copies {x, y, z, original index} of the AMBIG voxels' candidates beyond the second
+  int64_t n_ovf_records = 0;   // records in aovf
   int64_t n_ambig_voxels = 0;
   DevBuf wvox;         // K1c build scratch: n_blocks x 512 u32 counts / offsets
   DevBuf wbase;        // K1c build scratch: n_blocks u32: first wlists entry of the block's region

@@ -144,10 +144,11 @@ class PoseEngine:
         return dict(dims=tuple(dims), n_cells=nc.value, n_occupied=no.value, cell=cell.value, bytes=b.value)
 
     def label_stats(self) -> dict:
-        """Tri-state label structure of the current scene (pgp_label_stats)."""
+        """Tri-state label structure of the current scene (pgp_label_stats).  `ambig_overflow_records`: candidates of AMBIG voxels
+        beyond the two each voxel keeps inline in its 32-byte slot."""
         out = np.zeros(8, np.int64)
         self._check(self._lib.pgp_label_stats(self._ctx, _ptr(out)))
-        keys = ("cells_all_out", "cells_all_in", "cells_mixed", "voxels_out", "voxels_in", "voxels_ambig", "ambig_list_words", "nearest_list_entries")
+        keys = ("cells_all_out", "cells_all_in", "cells_mixed", "voxels_out", "voxels_in", "voxels_ambig", "ambig_overflow_records", "nearest_list_entries")
         return dict(zip(keys, (int(v) for v in out)))
 
     # ------------------------------------------------------------------ K3
