@@ -397,6 +397,57 @@ PGP_API int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int
                            float threshold, double* poses16_host, int k, float trim, float ratio, int max_iter, int* iters_out,
                            float* energy_out, int* n_unexplained);
 
+/* Many refinements in one call: the items of a frame (one per object) or of an expansion batch or rollouts (one per MCTS node
+ * or step), each with its own object, segment and placed set.  Explained-point removal runs as one launch sequence over every
+ * item with placed objects, the flags come back in one copy, and the trimmed ICP of every pose of every item is one K5 launch
+ * (one cluster of two CTAs per pose, the item's source, target grid and scratch rows read from a per-item descriptor).
+ *
+ * Item i refines rows [pose_offsets[i], pose_offsets[i + 1]) of poses16 (row-major 4x4 model->camera doubles, in place),
+ * iters_out and energy_out; k_i = 0 is allowed.  Its segment is points [seg_offsets[seg], seg_offsets[seg + 1]) of seg_xyz
+ * (camera frame, x 3); every segment goes up once however many items use it.  Its placed set is rows [placed_lo, placed_lo +
+ * n_placed) of placed16 (row-major 4x4 doubles); items may share rows.  n_unexplained_out: one entry per item, the points left
+ * after the removal (the segment size when n_placed = 0).  iters_out, energy_out and n_unexplained_out may be NULL.
+ *
+ * Each item's poses, iterations, energies and n_unexplained are bitwise those of the single calls on the same context:
+ *   PGP_ICP_POINT, n_placed > 0: pgp_mcts_tricp(obj, segment, placed rows, threshold, its poses, trim, ratio, max_iter);
+ *   PGP_ICP_POINT, n_placed = 0: pgp_tricp on the whole segment;
+ *   PGP_ICP_PLANE, n_placed > 0: pgp_remove_explained, the survivors in their original order, pgp_tricp_plane;
+ *   PGP_ICP_PLANE, n_placed = 0: pgp_tricp_plane on the whole segment.
+ * At the edges both metrics follow pgp_mcts_tricp: when no point survives, or n_keep < 3, the poses stay as given with
+ * iters_out = 0 and energy_out = 0; a pose whose result is not finite is returned as given with energy_out = +Inf.  No result
+ * depends on item order, on the other items or on earlier calls.
+ *
+ * PGP_E_INVALID, before anything runs and with every output untouched:
+ *   - metric not PGP_ICP_POINT / PGP_ICP_PLANE; n_items, n_segs or n_placed_rows < 0; a NULL array that has entries;
+ *   - seg_offsets or pose_offsets not non-decreasing from 0 (NULL reads as {0} when n_segs / n_items is 0);
+ *   - an item's seg outside [0, n_segs) or an empty segment; n_placed < 0 or placed rows outside [0, n_placed_rows);
+ *   - a segment coordinate, placed-pose entry or pose entry that is NaN or infinite;
+ *   - trim or ratio not > 0, threshold not >= 0 (NaN included);
+ *   - PGP_ICP_PLANE on a model slot set without validation normals;
+ *   - more than PGP_REFINE_MAX_POINTS segment points or PGP_REFINE_MAX_POSES poses in all; or scratch above PGP_REFINE_MAX_PAIRS,
+ *     counted in int64 as the sum over items of (k_i + (n_placed_i > 0)) x segment size -- the d2 / nn rows of the poses
+ *     (k_i x n_unexplained_i, bounded by the segment size since n_unexplained is not known before the call) and the flags.
+ * PGP_E_NO_MODEL: an item's slot has no model.  n_items = 0 is a valid no-op. */
+typedef struct pgp_refine_item {
+  int32_t obj;        /* model slot (pgp_set_model): its validation cloud is the ICP target and the explained cloud */
+  int32_t seg;        /* segment index: points seg_offsets[seg] .. seg_offsets[seg + 1] of seg_xyz */
+  int32_t placed_lo;  /* first row of placed16 */
+  int32_t n_placed;   /* number of placed poses (0: nothing is explained) */
+} pgp_refine_item;
+
+#define PGP_ICP_POINT 0   /* pgp_tricp's fit */
+#define PGP_ICP_PLANE 1   /* pgp_tricp_plane's fit */
+#define PGP_REFINE_MAX_POINTS (1ll << 30)
+#define PGP_REFINE_MAX_POSES (1ll << 20)
+#define PGP_REFINE_MAX_PAIRS (1ll << 30)
+
+PGP_API int pgp_refine_batch(pgp_ctx* ctx, int metric,
+                             const float* seg_xyz, const int64_t* seg_offsets, int n_segs,
+                             const double* placed16, int64_t n_placed_rows,
+                             const pgp_refine_item* items, const int64_t* pose_offsets, int n_items,
+                             double* poses16, float threshold, float trim, float ratio, int max_iter,
+                             int* iters_out, float* energy_out, int* n_unexplained_out);
+
 /* ---------------------------------------------------------------- K7: segment preparation -- */
 
 /* The step in front of the path, for one object of one RGB-D frame: depth decode (utilities::readDepthImage,

@@ -10,6 +10,8 @@ LIB_PATH = os.path.join(HERE, "libpgp.so")
 
 PGP_LCP_COUNT = 0
 PGP_LCP_WEIGHTED = 1
+PGP_ICP_POINT = 0
+PGP_ICP_PLANE = 1
 
 STATUS = {0: "PGP_OK", -1: "PGP_E_INVALID", -2: "PGP_E_CUDA", -3: "PGP_E_NO_SCENE", -4: "PGP_E_NO_MODEL",
           -5: "PGP_E_NO_SCORES", -6: "PGP_E_TOO_LARGE", -7: "PGP_E_NOMEM", -8: "PGP_E_CAPACITY", -9: "PGP_E_COMM"}
@@ -79,6 +81,7 @@ _SIGNATURES = {
     "pgp_get_bases": (_i, [_vp, _i, _vp, _vp, _vp, _i]),
     "pgp_remove_explained": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _vp]),
     "pgp_mcts_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _vp, _i, _f, _f, _i, _vp, _vp, _vp]),
+    "pgp_refine_batch": (_i, [_vp, _i, _vp, _vp, _i, _vp, _i64, _vp, _vp, _i, _vp, _f, _f, _f, _i, _vp, _vp, _vp]),
     "pgp_prepare_segment": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _f, _f, _f, _i, _vp, _vp, _i, _vp]),
     "pgp_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),
     "pgp_tricp_plane": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),

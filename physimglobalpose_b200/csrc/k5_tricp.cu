@@ -19,6 +19,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "pgp_internal.cuh"
@@ -39,6 +40,15 @@ struct TricpParams {
   int* iters; float* energy;
   const float4* nrm_orig;        // unit normals of tgt_orig, same order (point-to-plane fit)
 };
+
+// One item of a batched refinement (pgp_refine_batch): its own TricpParams -- source, target grid, n_keep, d2 / nn rows; T, iters
+// and energy point at its first pose -- and where its poses start in the launch.
+struct K5Item {
+  TricpParams p;
+  int pose_lo;
+};
+struct K5Batch { const K5Item* items; const int* pose_item; };   // pose_item: launch pose -> item
+template <bool BATCH> using K5Args = std::conditional_t<BATCH, K5Batch, TricpParams>;
 
 __global__ void k5_tgrid_count(const float4* __restrict__ pts, int n, TGrid tg, uint32_t* __restrict__ cell_of, uint32_t* __restrict__ counts) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -281,6 +291,8 @@ __host__ __device__ void euler_zyx(const double x[3], double R[3][3]) {
 
 // One Gauss-Newton step of the point-to-plane fit from the 28 sums S = {E, sum a r (6), H upper triangle row by row (21)}:
 // x = H^+ g with g = -sum a r, T <- fp32(dR R_T, ((dR_0 t_T + dR_1 t_T) + dR_2 t_T) + dt) in double from the fp32 T.
+// (one copy per kernel instance: a callee shared by the single and the batched kernel is register-allocated for both)
+template <bool BATCH>
 __device__ __noinline__ void plane_fit(const double* S, float* T) {
   double H[36], g[6], x[6], R[3][3];
   for (int i = 0, k = 7; i < 6; ++i)
@@ -381,11 +393,24 @@ __device__ __forceinline__ void plane_terms(const TricpParams& p, const float* s
 // PLANE = false: the point-to-point fit (16 sums, Horn).  PLANE = true: the point-to-plane fit; its 28 sums do not fit the
 // 64-register budget of a 1024-thread CTA next to the search, so they take two passes of 16 over the kept set (the second one
 // 12 sums and 4 zeros), each through the same butterfly into its own half of s_part.
-template <bool PLANE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kernel(const TricpParams p) {
+// BATCH = false: one item, its TricpParams in the kernel arguments.  BATCH = true (pgp_refine_batch): many items in one launch;
+// each cluster copies its item's K5Item into shared memory and runs the same code on it.
+template <bool PLANE, bool BATCH = false>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kernel(const K5Args<BATCH> a) {
   namespace cg = cooperative_groups;
   cg::cluster_group cl = cg::this_cluster();
   constexpr int NS = PLANE ? 32 : 16;    // sums exchanged between the CTAs
+  __shared__ K5Item s_item;
+  if constexpr (BATCH) {
+    static_assert(sizeof(K5Item) % 4 == 0 && sizeof(K5Item) / 4 <= TT, "K5Item is copied one word per thread");
+    const K5Item* src = a.items + a.pose_item[blockIdx.x >> 1];
+    if (threadIdx.x < sizeof(K5Item) / 4) reinterpret_cast<int*>(&s_item)[threadIdx.x] = reinterpret_cast<const int*>(src)[threadIdx.x];
+    __syncthreads();
+  }
+  const TricpParams* pp;
+  if constexpr (BATCH) pp = &s_item.p; else pp = &a;
+  const TricpParams& p = *pp;
+  const int pose = BATCH ? (int)(blockIdx.x >> 1) - s_item.pose_lo : (int)(blockIdx.x >> 1);
   __shared__ float sT[12];
   __shared__ uint32_t s_hist[2][256];    // double-buffered by pass parity: the partner may still read pass p while pass p+1 fills
   __shared__ uint32_t s_sel[4];          // prefix, remaining rank, CTA 0's count of values equal to tau
@@ -396,7 +421,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
   const unsigned cr = cl.block_rank();
   const uint32_t* r_hist = cl.map_shared_rank(&s_hist[0][0], cr ^ 1u);
   const double* r_part = cl.map_shared_rank(&s_part[0], cr ^ 1u);
-  const int pose = blockIdx.x >> 1, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int half = (p.ns + 1) >> 1;
   const int i_lo = cr ? half : 0, i_hi = cr ? p.ns : half;
   float* d2 = p.d2 + (size_t)pose * p.ns;
@@ -499,7 +524,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
       if (PLANE && !(energy <= FLT_MAX)) energy = INFINITY;      // (a NaN residual reports +Inf, as an overflowing one does)
       if (energy <= FLT_MAX) {                     // a kept squared distance overflowed: no fit, and the ratio test below stops
         if constexpr (PLANE) {
-          plane_fit(S, sT);
+          plane_fit<BATCH>(S, sT);
         } else {
           float Tn[12];
           rigid_fit((double)p.n_keep, S + 1, Tn);
@@ -521,7 +546,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
 
 // device scratch of the refinement: owned by the context (two contexts on one device must not share it), created on first
 // use, released by k5_release (pgp_destroy)
-struct TScratch { DevBuf seg, d2, nn, T, iters, energy, cell_of, cursor; };
+struct TScratch { DevBuf seg, d2, nn, T, iters, energy, cell_of, cursor, items, pose_item; };
 TScratch& tscratch_of(pgp_ctx* ctx) {
   if (!ctx->k5_scratch) ctx->k5_scratch = new TScratch();
   return *static_cast<TScratch*>(ctx->k5_scratch);
@@ -575,6 +600,83 @@ void invert_pose(const double* P, double* I) {
   I[12] = I[13] = I[14] = 0; I[15] = 1;
 }
 
+// The host half of one refinement, shared by pgp_tricp / pgp_tricp_plane / pgp_mcts_tricp (one item) and pgp_refine_batch (every
+// item): n_keep, the source in Morton order, the start transforms, and the poses from the refined transforms.
+
+int n_keep_of(float trim, int ns) {
+  const float keep_f = fabsf(trim * (float)ns);                          // abs(numPoints) on a float, UCTState.cpp:181,194
+  return keep_f < 2147483648.f ? std::min(ns, (int)keep_f) : ns;
+}
+
+// The source cloud goes up in Morton order of its own bounding box: a rigid transform keeps neighbours together, so the 32
+// queries of a warp walk the same few grid rows of the target in every iteration of every pose (the ring searches of unrelated
+// points diverge: 4 of 32 lanes were active in the distance loop).  Sums are order-free up to double rounding; ties at the trim
+// threshold are admitted in this order.  seg4: ns x float4 (w = 0).
+void morton_source(const float* seg_xyz_host, int ns, float* seg4) {
+  float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+  for (int i = 0; i < ns; ++i) for (int c = 0; c < 3; ++c) { lo[c] = std::min(lo[c], seg_xyz_host[3 * i + c]); hi[c] = std::max(hi[c], seg_xyz_host[3 * i + c]); }
+  const float ext = std::max(std::max(hi[0] - lo[0], hi[1] - lo[1]), std::max(hi[2] - lo[2], 1e-12f));
+  auto spread = [](uint32_t v) { uint64_t x = v & 0x1fffffu; x = (x | x << 32) & 0x1f00000000ffffull; x = (x | x << 16) & 0x1f0000ff0000ffull;
+                                 x = (x | x << 8) & 0x100f00f00f00f00full; x = (x | x << 4) & 0x10c30c30c30c30c3ull; x = (x | x << 2) & 0x1249249249249249ull; return x; };
+  std::vector<std::pair<uint64_t, int>> key((size_t)ns);
+  for (int i = 0; i < ns; ++i) {
+    uint64_t m = 0;
+    for (int c = 0; c < 3; ++c) {
+      const float u = (seg_xyz_host[3 * i + c] - lo[c]) / ext;
+      const uint32_t q = (uint32_t)std::min(1023.0f, std::max(0.0f, u * 1024.0f));     // (NaN -> 0)
+      m |= spread(q) << c;
+    }
+    key[(size_t)i] = std::make_pair(m, i);
+  }
+  std::sort(key.begin(), key.end());
+  for (int i = 0; i < ns; ++i) {
+    for (int c = 0; c < 3; ++c) seg4[4 * (size_t)i + c] = seg_xyz_host[3 * key[(size_t)i].second + c];
+    seg4[4 * (size_t)i + 3] = 0.f;
+  }
+}
+
+// T12: k x 12 fp32, the inverse of each pose (tform = inverse(object pose), UCTState.cpp:184-185)
+void start_transforms(const double* poses16_host, int k, float* T12) {
+  for (int i = 0; i < k; ++i) {
+    double inv[16];
+    invert_pose(poses16_host + 16 * (size_t)i, inv);
+    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) T12[12 * (size_t)i + 4 * r + c] = (float)inv[4 * r + c];
+  }
+}
+
+// pose = inverse(tform), UCTState.cpp:195-203; a non-finite energy leaves the pose as it was given
+void finish_poses(const float* T12, const int* it, const float* en, int k, double* poses16_host, int* iters_out, float* energy_out) {
+  for (int i = 0; i < k; ++i) {
+    if (en[i] <= FLT_MAX) {
+      double M[16] = {0}, inv[16];
+      for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) M[4 * r + c] = (double)T12[12 * (size_t)i + 4 * r + c];
+      M[15] = 1;
+      invert_pose(M, inv);
+      memcpy(poses16_host + 16 * (size_t)i, inv, sizeof(inv));
+    }
+    if (iters_out) iters_out[i] = it[i];
+    if (energy_out) energy_out[i] = en[i];
+  }
+}
+
+void zero_results(int k, int* iters_out, float* energy_out) {
+  for (int i = 0; i < k; ++i) { if (iters_out) iters_out[i] = 0; if (energy_out) energy_out[i] = 0.f; }
+}
+
+// the TricpParams of one item whose source, d2 / nn rows and pose rows start at the given device addresses
+TricpParams item_params(const Model& m, const float4* src, int ns, float* d2, int* nn, float* T, int* iters, float* energy, int n_keep, float ratio,
+                        int max_iter) {
+  TricpParams p{};
+  p.src = src; p.ns = ns;
+  p.tgt = m.tgrid_pts.as<float4>(); p.tstart = m.tgrid_start.as<uint32_t>(); p.nt = m.nv; p.tgt_orig = m.val_raw.as<float4>();
+  p.nrm_orig = m.val_nrm_orig.as<float4>();
+  memcpy(p.tg.lo, m.tg_lo, 12); p.tg.g = m.tg_g; p.tg.inv_g = 1.0f / m.tg_g; memcpy(p.tg.dim, m.tg_dim, 12);
+  p.d2 = d2; p.nn = nn; p.T = T;
+  p.n_keep = n_keep; p.ratio = ratio; p.max_iter = std::max(1, max_iter);
+  p.iters = iters; p.energy = energy;
+  return p;
+}
+
 }  // namespace
 
 // host-callable copy of max_eigvec4 for the CPU test-suite (tests/test_host_arithmetic.py): N16 row-major symmetric 4x4; returns 1
@@ -597,41 +699,11 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   TScratch& ts = tscratch_of(ctx);
   int rc = build_target_grid(ctx, m);
   if (rc) return rc;
-  const float keep_f = fabsf(trim * (float)ns);                          // abs(numPoints) on a float, UCTState.cpp:181,194
-  const int n_keep = keep_f < 2147483648.f ? std::min(ns, (int)keep_f) : ns;
-  if (n_keep < 3) {
-    for (int i = 0; i < k; ++i) { if (iters_out) iters_out[i] = 0; if (energy_out) energy_out[i] = 0.f; }
-    return PGP_OK;
-  }
-  // The source cloud goes up in Morton order of its own bounding box: a rigid transform keeps neighbours together, so the 32
-  // queries of a warp walk the same few grid rows of the target in every iteration of every pose (the ring searches of unrelated
-  // points diverge: 4 of 32 lanes were active in the distance loop).  Sums are order-free up to double rounding; ties at the trim
-  // threshold are admitted in this order.
-  std::vector<float> seg4((size_t)ns * 4, 0.f), T((size_t)k * 12);
-  {
-    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
-    for (int i = 0; i < ns; ++i) for (int c = 0; c < 3; ++c) { lo[c] = std::min(lo[c], seg_xyz_host[3 * i + c]); hi[c] = std::max(hi[c], seg_xyz_host[3 * i + c]); }
-    const float ext = std::max(std::max(hi[0] - lo[0], hi[1] - lo[1]), std::max(hi[2] - lo[2], 1e-12f));
-    auto spread = [](uint32_t v) { uint64_t x = v & 0x1fffffu; x = (x | x << 32) & 0x1f00000000ffffull; x = (x | x << 16) & 0x1f0000ff0000ffull;
-                                   x = (x | x << 8) & 0x100f00f00f00f00full; x = (x | x << 4) & 0x10c30c30c30c30c3ull; x = (x | x << 2) & 0x1249249249249249ull; return x; };
-    std::vector<std::pair<uint64_t, int>> key((size_t)ns);
-    for (int i = 0; i < ns; ++i) {
-      uint64_t m = 0;
-      for (int c = 0; c < 3; ++c) {
-        const float u = (seg_xyz_host[3 * i + c] - lo[c]) / ext;
-        const uint32_t q = (uint32_t)std::min(1023.0f, std::max(0.0f, u * 1024.0f));     // (NaN -> 0)
-        m |= spread(q) << c;
-      }
-      key[(size_t)i] = std::make_pair(m, i);
-    }
-    std::sort(key.begin(), key.end());
-    for (int i = 0; i < ns; ++i) for (int c = 0; c < 3; ++c) seg4[4 * (size_t)i + c] = seg_xyz_host[3 * key[(size_t)i].second + c];
-  }
-  for (int i = 0; i < k; ++i) {
-    double inv[16];
-    invert_pose(poses16_host + 16 * i, inv);                            // tform = inverse(object pose), UCTState.cpp:184-185
-    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) T[12 * (size_t)i + 4 * r + c] = (float)inv[4 * r + c];
-  }
+  const int n_keep = n_keep_of(trim, ns);
+  if (n_keep < 3) { zero_results(k, iters_out, energy_out); return PGP_OK; }
+  std::vector<float> seg4((size_t)ns * 4), T((size_t)k * 12);
+  morton_source(seg_xyz_host, ns, seg4.data());
+  start_transforms(poses16_host, k, T.data());
   PGP_CUDA(ctx, ts.seg.reserve((size_t)ns * 16));
   PGP_CUDA(ctx, ts.d2.reserve((size_t)k * ns * 4));
   PGP_CUDA(ctx, ts.nn.reserve((size_t)k * ns * 4));
@@ -640,14 +712,8 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   PGP_CUDA(ctx, ts.energy.reserve((size_t)k * 4));
   PGP_CUDA(ctx, cudaMemcpyAsync(ts.seg.p, seg4.data(), (size_t)ns * 16, cudaMemcpyHostToDevice, ctx->stream));
   PGP_CUDA(ctx, cudaMemcpyAsync(ts.T.p, T.data(), (size_t)k * 48, cudaMemcpyHostToDevice, ctx->stream));
-  TricpParams p{};
-  p.src = ts.seg.as<float4>(); p.ns = ns;
-  p.tgt = m.tgrid_pts.as<float4>(); p.tstart = m.tgrid_start.as<uint32_t>(); p.nt = m.nv; p.tgt_orig = m.val_raw.as<float4>();
-  p.nrm_orig = m.val_nrm_orig.as<float4>();
-  memcpy(p.tg.lo, m.tg_lo, 12); p.tg.g = m.tg_g; p.tg.inv_g = 1.0f / m.tg_g; memcpy(p.tg.dim, m.tg_dim, 12);
-  p.d2 = ts.d2.as<float>(); p.nn = ts.nn.as<int>(); p.T = ts.T.as<float>();
-  p.n_keep = n_keep; p.ratio = ratio; p.max_iter = std::max(1, max_iter);
-  p.iters = ts.iters.as<int>(); p.energy = ts.energy.as<float>();
+  const TricpParams p = item_params(m, ts.seg.as<float4>(), ns, ts.d2.as<float>(), ts.nn.as<int>(), ts.T.as<float>(), ts.iters.as<int>(),
+                                    ts.energy.as<float>(), n_keep, ratio, max_iter);
   if (plane) k5_tricp_kernel<true><<<2 * k, TT, 0, ctx->stream>>>(p);     // one cluster of two CTAs per pose
   else k5_tricp_kernel<false><<<2 * k, TT, 0, ctx->stream>>>(p);
   ctx->launches++;
@@ -658,16 +724,108 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   PGP_CUDA(ctx, cudaMemcpyAsync(it.data(), ts.iters.p, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream));
   PGP_CUDA(ctx, cudaMemcpyAsync(en.data(), ts.energy.p, (size_t)k * 4, cudaMemcpyDeviceToHost, ctx->stream));
   PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  for (int i = 0; i < k; ++i) {
-    if (en[i] <= FLT_MAX) {                                              // (non-finite energy: the pose stays as it was given)
-      double M[16] = {0}, inv[16];
-      for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) M[4 * r + c] = (double)T[12 * (size_t)i + 4 * r + c];
-      M[15] = 1;
-      invert_pose(M, inv);                                               // pose = inverse(tform), UCTState.cpp:195-203
-      memcpy(poses16_host + 16 * i, inv, sizeof(inv));
+  finish_poses(T.data(), it.data(), en.data(), k, poses16_host, iters_out, energy_out);
+  return PGP_OK;
+}
+
+// pgp_refine_batch after its checks (pgp_api.cu): K6 over every item with placed objects (one launch, one copy back), the host
+// half of every item (compaction, n_keep, Morton order, start transforms), then ONE K5 launch of 2 * sum(k) CTAs over the items
+// with n_keep >= 3.  Each item runs exactly the arithmetic of its single call: its own source, target grid and scratch rows.
+int k5_refine_batch(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16, int64_t n_placed_rows,
+                    const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold, float trim,
+                    float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out) {
+  if (n_items == 0) return PGP_OK;
+  TScratch& ts = tscratch_of(ctx);
+  for (int i = 0; i < n_items; ++i) {                                   // (cached per model: built once for each distinct obj)
+    int rc = build_target_grid(ctx, ctx->models[items[i].obj]);
+    if (rc) return rc;
+  }
+  // 1. explained points: every item with placed objects, flags in item order
+  std::vector<K6Job> jobs;
+  std::vector<int64_t> flag_lo((size_t)n_items, -1);
+  int64_t n_flags = 0;
+  for (int i = 0; i < n_items; ++i) {
+    const pgp_refine_item& it = items[i];
+    if (it.n_placed <= 0) continue;
+    const int ns = (int)(seg_offsets[it.seg + 1] - seg_offsets[it.seg]);
+    jobs.push_back(K6Job{&ctx->models[it.obj], seg_offsets[it.seg], ns, (int64_t)it.placed_lo, it.n_placed});
+    flag_lo[(size_t)i] = n_flags;
+    n_flags += ns;
+  }
+  std::vector<uint8_t> flags((size_t)n_flags);
+  if (!jobs.empty()) {
+    int rc = k6_flag_batch(ctx, seg_xyz, seg_offsets[n_segs], placed16, n_placed_rows, jobs, threshold, flags.data());
+    if (rc) return rc;
+  }
+  // 2. the host half of every item; items left out of the launch get their results here
+  struct Active { int item, ns, n_keep, k, pose_lo; int64_t src_lo, scr_lo; };
+  std::vector<Active> act;
+  std::vector<float> src4, T, un;
+  int64_t n_src = 0, n_scr = 0;
+  int n_poses = 0;
+  for (int i = 0; i < n_items; ++i) {
+    const pgp_refine_item& it = items[i];
+    const float* seg = seg_xyz + 3 * seg_offsets[it.seg];
+    const int ns = (int)(seg_offsets[it.seg + 1] - seg_offsets[it.seg]);
+    const int k = (int)(pose_offsets[i + 1] - pose_offsets[i]);
+    int kept = ns;
+    if (flag_lo[(size_t)i] >= 0) {                                      // extract.setNegative(true): the survivors in their original order
+      un.resize((size_t)ns * 3);
+      kept = k6_compact(seg, ns, flags.data() + flag_lo[(size_t)i], un.data());
+      seg = un.data();
     }
-    if (iters_out) iters_out[i] = it[i];
-    if (energy_out) energy_out[i] = en[i];
+    if (n_unexplained_out) n_unexplained_out[i] = kept;
+    if (k == 0) continue;
+    int* it_out = iters_out ? iters_out + pose_offsets[i] : nullptr;
+    float* en_out = energy_out ? energy_out + pose_offsets[i] : nullptr;
+    const int n_keep = n_keep_of(trim, kept);
+    if (n_keep < 3) { zero_results(k, it_out, en_out); continue; }     // (kept = 0 included)
+    act.push_back(Active{i, kept, n_keep, k, n_poses, n_src, n_scr});
+    src4.resize((size_t)(n_src + kept) * 4);
+    morton_source(seg, kept, src4.data() + 4 * n_src);
+    T.resize((size_t)(n_poses + k) * 12);
+    start_transforms(poses16 + 16 * pose_offsets[i], k, T.data() + 12 * (size_t)n_poses);
+    n_src += kept; n_scr += (int64_t)k * kept; n_poses += k;
+  }
+  if (act.empty()) return PGP_OK;
+  // 3. one launch: packed sources, start transforms, a descriptor per item and the pose -> item map, each up in one copy
+  PGP_CUDA(ctx, ts.seg.reserve((size_t)n_src * 16));
+  PGP_CUDA(ctx, ts.d2.reserve((size_t)n_scr * 4));
+  PGP_CUDA(ctx, ts.nn.reserve((size_t)n_scr * 4));
+  PGP_CUDA(ctx, ts.T.reserve((size_t)n_poses * 48));
+  PGP_CUDA(ctx, ts.iters.reserve((size_t)n_poses * 4));
+  PGP_CUDA(ctx, ts.energy.reserve((size_t)n_poses * 4));
+  PGP_CUDA(ctx, ts.items.reserve(act.size() * sizeof(K5Item)));
+  PGP_CUDA(ctx, ts.pose_item.reserve((size_t)n_poses * 4));
+  std::vector<K5Item> desc(act.size());
+  std::vector<int> pose_item((size_t)n_poses);
+  for (size_t a = 0; a < act.size(); ++a) {
+    const Active& A = act[a];
+    desc[a].p = item_params(ctx->models[items[A.item].obj], ts.seg.as<float4>() + A.src_lo, A.ns, ts.d2.as<float>() + A.scr_lo,
+                            ts.nn.as<int>() + A.scr_lo, ts.T.as<float>() + 12 * (size_t)A.pose_lo, ts.iters.as<int>() + A.pose_lo,
+                            ts.energy.as<float>() + A.pose_lo, A.n_keep, ratio, max_iter);
+    desc[a].pose_lo = A.pose_lo;
+    for (int j = 0; j < A.k; ++j) pose_item[(size_t)A.pose_lo + j] = (int)a;
+  }
+  PGP_CUDA(ctx, cudaMemcpyAsync(ts.seg.p, src4.data(), (size_t)n_src * 16, cudaMemcpyHostToDevice, ctx->stream));
+  PGP_CUDA(ctx, cudaMemcpyAsync(ts.T.p, T.data(), (size_t)n_poses * 48, cudaMemcpyHostToDevice, ctx->stream));
+  PGP_CUDA(ctx, cudaMemcpyAsync(ts.items.p, desc.data(), desc.size() * sizeof(K5Item), cudaMemcpyHostToDevice, ctx->stream));
+  PGP_CUDA(ctx, cudaMemcpyAsync(ts.pose_item.p, pose_item.data(), (size_t)n_poses * 4, cudaMemcpyHostToDevice, ctx->stream));
+  const K5Batch b{ts.items.as<K5Item>(), ts.pose_item.as<int>()};
+  if (plane) k5_tricp_kernel<true, true><<<2 * n_poses, TT, 0, ctx->stream>>>(b);
+  else k5_tricp_kernel<false, true><<<2 * n_poses, TT, 0, ctx->stream>>>(b);
+  ctx->launches++;
+  PGP_CUDA(ctx, cudaGetLastError());
+  std::vector<int> it((size_t)n_poses);
+  std::vector<float> en((size_t)n_poses);
+  PGP_CUDA(ctx, cudaMemcpyAsync(T.data(), ts.T.p, (size_t)n_poses * 48, cudaMemcpyDeviceToHost, ctx->stream));
+  PGP_CUDA(ctx, cudaMemcpyAsync(it.data(), ts.iters.p, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  PGP_CUDA(ctx, cudaMemcpyAsync(en.data(), ts.energy.p, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  for (const Active& A : act) {
+    const int64_t lo = pose_offsets[A.item];
+    finish_poses(T.data() + 12 * (size_t)A.pose_lo, it.data() + A.pose_lo, en.data() + A.pose_lo, A.k, poses16 + 16 * lo,
+                 iters_out ? iters_out + lo : nullptr, energy_out ? energy_out + lo : nullptr);
   }
   return PGP_OK;
 }
@@ -675,7 +833,7 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
 void k5_release(pgp_ctx* ctx) {
   if (!ctx->k5_scratch) return;
   TScratch* ts = static_cast<TScratch*>(ctx->k5_scratch);
-  for (DevBuf* b : {&ts->seg, &ts->d2, &ts->nn, &ts->T, &ts->iters, &ts->energy, &ts->cell_of, &ts->cursor}) b->release();
+  for (DevBuf* b : {&ts->seg, &ts->d2, &ts->nn, &ts->T, &ts->iters, &ts->energy, &ts->cell_of, &ts->cursor, &ts->items, &ts->pose_item}) b->release();
   delete ts;
   ctx->k5_scratch = nullptr;
 }

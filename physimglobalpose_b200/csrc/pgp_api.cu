@@ -845,12 +845,61 @@ int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg, int ns, const double
     if (rc) return rc;
   }
   std::vector<float> un((size_t)std::max(kept, 1) * 3);
-  int w = 0;
-  for (int i = 0; i < ns; ++i)                       // extract.setNegative(true): the survivors in their original order
-    if (!flag[i]) { memcpy(&un[3 * (size_t)w], seg + 3 * (size_t)i, 12); ++w; }
+  k6_compact(seg, ns, flag.data(), un.data());       // extract.setNegative(true): the survivors in their original order
   if (n_unexplained) *n_unexplained = kept;
   if (kept == 0) { for (int i = 0; i < k; ++i) { if (iters) iters[i] = 0; if (energy) energy[i] = 0.f; } return PGP_OK; }
   return k5_tricp(ctx, *m, un.data(), kept, poses, k, trim, ratio, max_iter, iters, energy, false);
+}
+
+static bool all_finite(const float* v, int64_t n) { for (int64_t i = 0; i < n; ++i) if (!std::isfinite(v[i])) return false; return true; }
+static bool all_finite(const double* v, int64_t n) { for (int64_t i = 0; i < n; ++i) if (!std::isfinite(v[i])) return false; return true; }
+// offsets[0] == 0 and offsets[i] <= offsets[i + 1] for the n + 1 entries
+static bool csr_offsets_ok(const int64_t* off, int n) {
+  if (off[0] != 0) return false;
+  for (int i = 0; i < n; ++i) if (off[i + 1] < off[i]) return false;
+  return true;
+}
+
+int pgp_refine_batch(pgp_ctx* ctx, int metric, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16,
+                     int64_t n_placed_rows, const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold,
+                     float trim, float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out) {
+  CHECK_CTX(ctx);
+  static const int64_t zero = 0;
+  if (metric != PGP_ICP_POINT && metric != PGP_ICP_PLANE) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: metric must be 0 or 1");
+  if (n_items < 0 || n_segs < 0 || n_placed_rows < 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: negative count");
+  if (!seg_offsets && n_segs > 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null seg_offsets");
+  if (!pose_offsets && n_items > 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null pose_offsets");
+  if (!seg_offsets) seg_offsets = &zero;
+  if (!pose_offsets) pose_offsets = &zero;
+  if (!csr_offsets_ok(seg_offsets, n_segs)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: seg_offsets must be non-decreasing from 0");
+  if (!csr_offsets_ok(pose_offsets, n_items)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: pose_offsets must be non-decreasing from 0");
+  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
+  if (n_pts > PGP_REFINE_MAX_POINTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: more than PGP_REFINE_MAX_POINTS segment points");
+  if (n_poses > PGP_REFINE_MAX_POSES) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: more than PGP_REFINE_MAX_POSES poses");
+  if ((n_pts > 0 && !seg_xyz) || (n_placed_rows > 0 && !placed16) || (n_items > 0 && !items) || (n_poses > 0 && !poses16))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null argument");
+  if (!all_finite(seg_xyz, 3 * n_pts) || !all_finite(placed16, 16 * n_placed_rows) || !all_finite(poses16, 16 * n_poses))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: non-finite segment point, placed pose or pose");
+  if (!(trim > 0.f) || !(ratio > 0.f) || !(threshold >= 0.f))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: trim and ratio must be > 0 and threshold >= 0");
+  int64_t pairs = 0;
+  for (int i = 0; i < n_items; ++i) {
+    const pgp_refine_item& it = items[i];
+    if (it.seg < 0 || it.seg >= n_segs) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: segment %d outside [0, %d)", i, it.seg, n_segs);
+    const int64_t ns = seg_offsets[it.seg + 1] - seg_offsets[it.seg];
+    if (ns == 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: segment %d is empty", i, it.seg);
+    if (it.n_placed < 0 || it.placed_lo < 0 || (int64_t)it.placed_lo + it.n_placed > n_placed_rows)
+      return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: placed rows outside [0, %lld)", i, (long long)n_placed_rows);
+    Model* m = get_model(ctx, it.obj);
+    if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "pgp_refine_batch: item %d: no model in slot %d", i, it.obj);
+    if (metric == PGP_ICP_PLANE && !m->val_has_nrm)
+      return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: model slot %d was set without validation normals", i, it.obj);
+    // d2 / nn rows of the poses, and the explained flags (each factor is at most 2^30 + 1: no overflow before the check)
+    pairs += (pose_offsets[i + 1] - pose_offsets[i] + (it.n_placed > 0 ? 1 : 0)) * ns;
+    if (pairs > PGP_REFINE_MAX_PAIRS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: scratch above PGP_REFINE_MAX_PAIRS");
+  }
+  return k5_refine_batch(ctx, metric == PGP_ICP_PLANE, seg_xyz, seg_offsets, n_segs, placed16, n_placed_rows, items, pose_offsets, n_items, poses16,
+                         threshold, trim, ratio, max_iter, iters_out, energy_out, n_unexplained_out);
 }
 
 int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, int class_id, const float* K9,

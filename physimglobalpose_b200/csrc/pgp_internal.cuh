@@ -246,6 +246,10 @@ void k7_release(pgp_ctx* ctx);
 // plane: the point-to-plane fit (pgp_tricp_plane) instead of the point-to-point one (pgp_tricp)
 int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* poses16_host, int k, float trim, float ratio,
              int max_iter, int* iters_out, float* energy_out, bool plane);
+// pgp_refine_batch after its argument checks
+int k5_refine_batch(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16, int64_t n_placed_rows,
+                    const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold, float trim,
+                    float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out);
 
 // ---------------------------------------------------------------------------------------------
 // fp32 arithmetic in the reference's association, every operation individually rounded
@@ -281,6 +285,14 @@ __device__ __forceinline__ bool depth_valid(float d) { return (double)d > 0.1 &&
 // k6_explained.cu
 int k6_remove_explained(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, const double* placed16_host, int n_placed, float threshold,
                         uint8_t* flags_host, int* n_unexplained);
+// One segment of a batch flagged against model m placed at rows [placed_lo, placed_lo + n_placed) (pgp_refine_batch).
+struct K6Job { const Model* m; int64_t seg_lo; int ns; int64_t placed_lo; int n_placed; };
+// The flags of every job in one launch and one copy back: job j's ns flags follow job j - 1's in flags_host, bit for bit those of
+// k6_remove_explained.  The n_seg_pts points of seg_xyz_host and the n_placed_rows placed rows go up once.
+int k6_flag_batch(pgp_ctx* ctx, const float* seg_xyz_host, int64_t n_seg_pts, const double* placed16_host, int64_t n_placed_rows,
+                  const std::vector<K6Job>& jobs, float threshold, uint8_t* flags_host);
+// the points with flag 0, in their original order (extract.setNegative(true), UCTState.cpp:170-174); returns their number
+int k6_compact(const float* seg_xyz_host, int ns, const uint8_t* flags, float* out_xyz);
 // k7_segment.cu
 int k7_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_host, const uint8_t* mask_host, int rows, int cols, int cls, const float* K9, float leaf,
                        float normal_r, float outlier_r, int min_nb, float* xyz_host, float* nrm_host, int cap, int* n_out, int* n_raw_out);

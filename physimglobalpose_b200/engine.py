@@ -421,6 +421,37 @@ class PoseEngine:
                                              _ptr(P), len(P), float(trim), float(ratio), int(max_iter), _ptr(iters), _ptr(energy), C.byref(nun)))
         return P.reshape(-1, 4, 4), iters, energy, nun.value
 
+    def refine_batch(self, segments, items, metric: str = "point", threshold: float = 0.008, trim: float = 0.5, ratio: float = 0.99,
+                     max_iter: int = 100):
+        """Many refinements in one call (pgp_refine_batch).  segments: list of (n, 3) clouds; items: list of
+        (obj, seg index, placed poses (m, 4, 4), candidate poses (k, 4, 4)); metric "point" (pgp_tricp's fit) or "plane"
+        (pgp_tricp_plane's).  Returns one (refined poses, iterations, energies, n_unexplained) per item, each equal to that
+        item's mcts_tricp (point) or remove_explained + tricp_plane (plane) result."""
+        icp = {"point": _lib.PGP_ICP_POINT, "plane": _lib.PGP_ICP_PLANE}[metric]
+        segs = [_f32(s, 3) for s in segments]
+        seg = np.ascontiguousarray(np.concatenate(segs) if segs else np.zeros((0, 3), np.float32))
+        seg_off = np.zeros(len(segs) + 1, np.int64)
+        seg_off[1:] = np.cumsum([len(s) for s in segs])
+        placed = [np.ascontiguousarray(it[2], dtype=np.float64).reshape(-1, 16) for it in items]
+        poses = [np.ascontiguousarray(it[3], dtype=np.float64).reshape(-1, 16) for it in items]
+        rec = np.zeros(len(items), np.dtype([("obj", "<i4"), ("seg", "<i4"), ("placed_lo", "<i4"), ("n_placed", "<i4")]))
+        lo = 0
+        for i, it in enumerate(items):
+            rec[i] = (int(it[0]), int(it[1]), lo, len(placed[i]))
+            lo += len(placed[i])
+        pl = np.ascontiguousarray(np.concatenate(placed) if placed else np.zeros((0, 16)))
+        P = np.ascontiguousarray(np.concatenate(poses) if poses else np.zeros((0, 16)))
+        pose_off = np.zeros(len(items) + 1, np.int64)
+        pose_off[1:] = np.cumsum([len(p) for p in poses])
+        iters = np.zeros(len(P), np.int32)
+        energy = np.zeros(len(P), np.float32)
+        nun = np.zeros(len(items), np.int32)
+        self._check(self._lib.pgp_refine_batch(self._ctx, icp, _ptr(seg), _ptr(seg_off), len(segs), _ptr(pl), len(pl), _ptr(rec), _ptr(pose_off),
+                                               len(items), _ptr(P), float(threshold), float(trim), float(ratio), int(max_iter), _ptr(iters),
+                                               _ptr(energy), _ptr(nun)))
+        return [(P[a:b].reshape(-1, 4, 4), iters[a:b], energy[a:b], int(nun[i]))
+                for i, (a, b) in enumerate(zip(pose_off[:-1], pose_off[1:]))]
+
     # ------------------------------------------------------------------ K7
     def prepare_segment(self, depth_raw_u16, class_mask_u8, class_id: int, K, leaf: float = 0.01, normal_radius: float = 0.02,
                         outlier_radius: float = 0.03, min_neighbors: int = 10, cap: int = 1 << 20):
