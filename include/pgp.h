@@ -398,9 +398,11 @@ PGP_API int pgp_mcts_tricp(pgp_ctx* ctx, int obj, const float* seg_xyz_host, int
                            float* energy_out, int* n_unexplained);
 
 /* Many refinements in one call: the items of a frame (one per object) or of an expansion batch or rollouts (one per MCTS node
- * or step), each with its own object, segment and placed set.  Explained-point removal runs as one launch sequence over every
- * item with placed objects, the flags come back in one copy, and the trimmed ICP of every pose of every item is one K5 launch
- * (one cluster of two CTAs per pose, the item's source, target grid and scratch rows read from a per-item descriptor).
+ * or step), each with its own object, segment and placed set.  The arrays go up once, the batch runs as the device pipeline of
+ * pgp_refine_batch_dev (explained-point removal over every item with placed objects in one launch, the survivors' count, n_keep
+ * and Morton order per item on the device, the trimmed ICP of every pose of every item in one K5 launch: one cluster of two CTAs
+ * per pose, the item's source, target grid and scratch rows read from a per-item descriptor), and the results come back with
+ * one synchronisation.
  *
  * Item i refines rows [pose_offsets[i], pose_offsets[i + 1]) of poses16 (row-major 4x4 model->camera doubles, in place),
  * iters_out and energy_out; k_i = 0 is allowed.  Its segment is points [seg_offsets[seg], seg_offsets[seg + 1]) of seg_xyz
@@ -447,6 +449,34 @@ PGP_API int pgp_refine_batch(pgp_ctx* ctx, int metric,
                              const pgp_refine_item* items, const int64_t* pose_offsets, int n_items,
                              double* poses16, float threshold, float trim, float ratio, int max_iter,
                              int* iters_out, float* energy_out, int* n_unexplained_out);
+
+/* pgp_refine_batch with the bulk data in device memory, asynchronous on the context's stream (pgp_set_stream): the form for a
+ * caller whose segments, placed poses or candidate poses already live on the GPU, or that queues the refinement behind other
+ * work.  pgp_refine_batch itself uploads its arguments, runs this pipeline and downloads the results.
+ *
+ * Arguments are those of pgp_refine_batch.  In device memory (of the context's device, or managed): seg_xyz_dev, placed16_dev,
+ * poses16_dev (refined in place), iters_dev, energy_dev and n_unexplained_dev (each may be NULL) and status_dev (one int32).
+ * On the host: seg_offsets, items and pose_offsets, so every launch size is known without reading anything back.  The call
+ * returns once the work is queued, and the host arrays may be reused at once.  Once the context's scratch has grown to the
+ * batch's size (a first call of that size), it makes no host synchronisation and no device-to-host copy; a call of a larger
+ * size grows the scratch, and cudaFree / cudaMalloc synchronise the device.
+ *
+ * Results: each item's poses, iterations, energies and n_unexplained are bitwise what pgp_refine_batch gives on the same inputs
+ * (so bitwise the single calls listed there), with the same edge cases.  The work is a fixed number of launches whatever the
+ * number of items: ingest (conversion, finiteness, start transforms), explained points, item preparation (survivor count,
+ * n_keep, Morton order), one K5 launch over every pose, and the final inversion.
+ *
+ * Returned at once, with nothing queued and every output untouched: every refusal of pgp_refine_batch that the host can decide
+ * (all but the value checks), status_dev == NULL, and a device argument that cudaPointerGetAttributes does not report as device
+ * or managed memory of the context's device.
+ * On the device: a NaN or infinite segment coordinate, placed-pose entry or pose entry sets *status_dev = PGP_E_INVALID and no
+ * output is written; otherwise *status_dev = PGP_OK.  Every call sets *status_dev afresh (n_items = 0 included). */
+PGP_API int pgp_refine_batch_dev(pgp_ctx* ctx, int metric,
+                                 const float* seg_xyz_dev, const int64_t* seg_offsets, int n_segs,
+                                 const double* placed16_dev, int64_t n_placed_rows,
+                                 const pgp_refine_item* items, const int64_t* pose_offsets, int n_items,
+                                 double* poses16_dev, float threshold, float trim, float ratio, int max_iter,
+                                 int* iters_dev, float* energy_dev, int* n_unexplained_dev, int32_t* status_dev);
 
 /* ---------------------------------------------------------------- K7: segment preparation -- */
 

@@ -82,6 +82,7 @@ _SIGNATURES = {
     "pgp_remove_explained": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _vp]),
     "pgp_mcts_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _vp, _i, _f, _f, _i, _vp, _vp, _vp]),
     "pgp_refine_batch": (_i, [_vp, _i, _vp, _vp, _i, _vp, _i64, _vp, _vp, _i, _vp, _f, _f, _f, _i, _vp, _vp, _vp]),
+    "pgp_refine_batch_dev": (_i, [_vp, _i, _vp, _vp, _i, _vp, _i64, _vp, _vp, _i, _vp, _f, _f, _f, _i, _vp, _vp, _vp, _vp]),
     "pgp_prepare_segment": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _f, _f, _f, _i, _vp, _vp, _i, _vp]),
     "pgp_tricp": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),
     "pgp_tricp_plane": (_i, [_vp, _i, _vp, _i, _vp, _i, _f, _f, _i, _vp, _vp]),

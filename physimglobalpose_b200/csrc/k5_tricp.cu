@@ -394,7 +394,9 @@ __device__ __forceinline__ void plane_terms(const TricpParams& p, const float* s
 // 64-register budget of a 1024-thread CTA next to the search, so they take two passes of 16 over the kept set (the second one
 // 12 sums and 4 zeros), each through the same butterfly into its own half of s_part.
 // BATCH = false: one item, its TricpParams in the kernel arguments.  BATCH = true (pgp_refine_batch): many items in one launch;
-// each cluster copies its item's K5Item into shared memory and runs the same code on it.
+// each cluster copies its item's K5Item into shared memory and runs the same code on it -- or returns at once when the item has
+// n_keep < 3 (set so by k5_prep_items, or left at 0 by a refused call), before any cluster barrier: both CTAs read the same
+// descriptor, so the pair leaves together and neither touches the other's shared memory.
 template <bool PLANE, bool BATCH = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kernel(const K5Args<BATCH> a) {
   namespace cg = cooperative_groups;
@@ -406,6 +408,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
     const K5Item* src = a.items + a.pose_item[blockIdx.x >> 1];
     if (threadIdx.x < sizeof(K5Item) / 4) reinterpret_cast<int*>(&s_item)[threadIdx.x] = reinterpret_cast<const int*>(src)[threadIdx.x];
     __syncthreads();
+    if (s_item.p.n_keep < 3) return;
   }
   const TricpParams* pp;
   if constexpr (BATCH) pp = &s_item.p; else pp = &a;
@@ -546,7 +549,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
 
 // device scratch of the refinement: owned by the context (two contexts on one device must not share it), created on first
 // use, released by k5_release (pgp_destroy)
-struct TScratch { DevBuf seg, d2, nn, T, iters, energy, cell_of, cursor, items, pose_item; };
+// The batch (pgp_refine_batch[_dev]) adds: in4 / placed_T (its segments and placed rows converted on the device), flags (K6),
+// keys (the sorts too large for shared memory), the host call's copies of its arguments (raw_*) and results (out), and pinned
+// staging for the one upload of its host-built tables: K5_STAGES buffers used in turn, each reused once its last copy has run.
+constexpr int K5_STAGES = 4;
+struct Staging { void* host = nullptr; size_t cap = 0; cudaEvent_t copied = nullptr; };
+struct TScratch {
+  DevBuf seg, d2, nn, T, iters, energy, cell_of, cursor, items;
+  DevBuf in4, placed_T, flags, keys, raw_seg, raw_placed, raw_poses, out;
+  Staging stage[K5_STAGES];
+  unsigned next_stage = 0;
+  bool prep_smem_set = false;
+};
 TScratch& tscratch_of(pgp_ctx* ctx) {
   if (!ctx->k5_scratch) ctx->k5_scratch = new TScratch();
   return *static_cast<TScratch*>(ctx->k5_scratch);
@@ -591,8 +605,8 @@ int build_target_grid(pgp_ctx* ctx, Model& m) {
   return PGP_OK;
 }
 
-// general 4x4 rigid inverse in double: [R t]^-1 = [R^T, -R^T t]
-void invert_pose(const double* P, double* I) {
+// general 4x4 rigid inverse in double: [R t]^-1 = [R^T, -R^T t] (the device copies run unfused like the host's: -fmad=false)
+__host__ __device__ void invert_pose(const double* P, double* I) {
   for (int r = 0; r < 3; ++r) {
     for (int c = 0; c < 3; ++c) I[4 * r + c] = P[4 * c + r];
     I[4 * r + 3] = -(P[0 * 4 + r] * P[3] + P[1 * 4 + r] * P[7] + P[2 * 4 + r] * P[11]);
@@ -600,33 +614,50 @@ void invert_pose(const double* P, double* I) {
   I[12] = I[13] = I[14] = 0; I[15] = 1;
 }
 
-// The host half of one refinement, shared by pgp_tricp / pgp_tricp_plane / pgp_mcts_tricp (one item) and pgp_refine_batch (every
-// item): n_keep, the source in Morton order, the start transforms, and the poses from the refined transforms.
+// The host half of one refinement of pgp_tricp / pgp_tricp_plane / pgp_mcts_tricp: n_keep, the source in Morton order, the start
+// transforms, and the poses from the refined transforms (the batch runs the same arithmetic on the device, k5_prep_items).
 
-int n_keep_of(float trim, int ns) {
+__host__ __device__ int n_keep_of(float trim, int ns) {
   const float keep_f = fabsf(trim * (float)ns);                          // abs(numPoints) on a float, UCTState.cpp:181,194
-  return keep_f < 2147483648.f ? std::min(ns, (int)keep_f) : ns;
+  return keep_f < 2147483648.f ? ((int)keep_f < ns ? (int)keep_f : ns) : ns;
 }
 
 // The source cloud goes up in Morton order of its own bounding box: a rigid transform keeps neighbours together, so the 32
 // queries of a warp walk the same few grid rows of the target in every iteration of every pose (the ring searches of unrelated
 // points diverge: 4 of 32 lanes were active in the distance loop).  Sums are order-free up to double rounding; ties at the trim
-// threshold are admitted in this order.  seg4: ns x float4 (w = 0).
+// threshold are admitted in this order.  The order is that of the (code, index) pairs; morton_source computes it on the host
+// for the single calls, k5_prep_items on the device for the batch, both with the two functions below.
+
+// edge of the bounding cube of the box [lo, hi]
+__host__ __device__ inline float morton_extent(const float lo[3], const float hi[3]) {
+  const float dx = hi[0] - lo[0], dy = hi[1] - lo[1], dz = hi[2] - lo[2];
+  const float a = dx < dy ? dy : dx, b = dz < 1e-12f ? 1e-12f : dz;                  // std::max(u, v) = u < v ? v : u
+  return a < b ? b : a;
+}
+// 30-bit code of p over the cube [lo, lo + ext]: per axis fp32 (p - lo) / ext, x 1024, clamped to [0, 1023] (NaN -> 0), the
+// axes' bits interleaved x lowest
+__host__ __device__ inline uint64_t morton_code(float x, float y, float z, const float lo[3], float ext) {
+  const float p[3] = {x, y, z};
+  uint64_t m = 0;
+  for (int c = 0; c < 3; ++c) {
+    const float v = (p[c] - lo[c]) / ext * 1024.0f;
+    uint64_t q = (uint32_t)(v > 0.0f ? (v < 1023.0f ? v : 1023.0f) : 0.0f);    // std::min(1023, std::max(0, v))
+    q = (q | q << 32) & 0x1f00000000ffffull; q = (q | q << 16) & 0x1f0000ff0000ffull; q = (q | q << 8) & 0x100f00f00f00f00full;
+    q = (q | q << 4) & 0x10c30c30c30c30c3ull; q = (q | q << 2) & 0x1249249249249249ull;
+    m |= q << c;
+  }
+  return m;
+}
+
+// seg4: ns x float4 (w = 0)
 void morton_source(const float* seg_xyz_host, int ns, float* seg4) {
   float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
   for (int i = 0; i < ns; ++i) for (int c = 0; c < 3; ++c) { lo[c] = std::min(lo[c], seg_xyz_host[3 * i + c]); hi[c] = std::max(hi[c], seg_xyz_host[3 * i + c]); }
-  const float ext = std::max(std::max(hi[0] - lo[0], hi[1] - lo[1]), std::max(hi[2] - lo[2], 1e-12f));
-  auto spread = [](uint32_t v) { uint64_t x = v & 0x1fffffu; x = (x | x << 32) & 0x1f00000000ffffull; x = (x | x << 16) & 0x1f0000ff0000ffull;
-                                 x = (x | x << 8) & 0x100f00f00f00f00full; x = (x | x << 4) & 0x10c30c30c30c30c3ull; x = (x | x << 2) & 0x1249249249249249ull; return x; };
+  const float ext = morton_extent(lo, hi);
   std::vector<std::pair<uint64_t, int>> key((size_t)ns);
   for (int i = 0; i < ns; ++i) {
-    uint64_t m = 0;
-    for (int c = 0; c < 3; ++c) {
-      const float u = (seg_xyz_host[3 * i + c] - lo[c]) / ext;
-      const uint32_t q = (uint32_t)std::min(1023.0f, std::max(0.0f, u * 1024.0f));     // (NaN -> 0)
-      m |= spread(q) << c;
-    }
-    key[(size_t)i] = std::make_pair(m, i);
+    const float* p = seg_xyz_host + 3 * (size_t)i;
+    key[(size_t)i] = std::make_pair(morton_code(p[0], p[1], p[2], lo, ext), i);
   }
   std::sort(key.begin(), key.end());
   for (int i = 0; i < ns; ++i) {
@@ -675,6 +706,145 @@ TricpParams item_params(const Model& m, const float4* src, int ns, float* d2, in
   p.n_keep = n_keep; p.ratio = ratio; p.max_iter = std::max(1, max_iter);
   p.iters = iters; p.energy = energy;
   return p;
+}
+
+// ---------------------------------------------------------------- the batch on the device (pgp_refine_batch[_dev])
+// ingest -> K6 -> k5_prep_items -> K5 -> k5_finish, a fixed number of launches and no read-back.  Every row of the packed source
+// and of the d2 / nn scratch is laid out by SEGMENT size (an upper bound of the survivors), so the host knows every offset.
+
+// The survivors of an item whose segment has at most K5_SORT_SHARED points are sorted in the dynamic shared memory of its CTA
+// (64 KB of keys at most); larger items sort in global memory (TScratch::keys), with the same code.
+constexpr int K5_SORT_SHARED = 8192;
+
+// One item as k5_prep_items reads it: its points in in4, its K6 flags (flag_lo < 0: nothing placed), its slot of the packed
+// source (src_lo < 0: k = 0) and of the global sort keys (key_lo < 0: sorted in shared memory).
+struct PrepItem { int64_t seg_lo, flag_lo, src_lo, key_lo; int ns, k; };
+
+__host__ __device__ inline int pow2_at_least(int n) { int p = 1; while (p < n) p <<= 1; return p; }
+
+// Step 1: segments to float4 (w = 0), placed rows to fp32 (pose16_to_f32x12, as K6 takes them), the start transforms (the fp32
+// inverse of every pose, as start_transforms), and the finiteness of every value: a NaN or Inf anywhere sets *status to
+// PGP_E_INVALID (PGP_OK was stored before the launch).  Index t < n_pts is a point, the next n_rows placed rows, then the poses.
+__global__ void k5_ingest(const float* __restrict__ seg_xyz, int64_t n_pts, const double* __restrict__ placed16, int64_t n_rows,
+                          const double* __restrict__ poses16, int64_t n_poses, float4* __restrict__ in4, float* __restrict__ placed_T,
+                          float* __restrict__ T, int32_t* __restrict__ status) {
+  bool ok = true;
+  const int64_t n = n_pts + n_rows + n_poses;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
+    if (t < n_pts) {
+      const float x = seg_xyz[3 * t], y = seg_xyz[3 * t + 1], z = seg_xyz[3 * t + 2];
+      ok &= isfinite(x) && isfinite(y) && isfinite(z);
+      in4[t] = make_float4(x, y, z, 0.f);
+      continue;
+    }
+    const bool placed = t < n_pts + n_rows;
+    const int64_t r = placed ? t - n_pts : t - n_pts - n_rows;
+    const double* src = (placed ? placed16 : poses16) + 16 * r;
+    double P[16];
+    for (int k = 0; k < 16; ++k) { P[k] = src[k]; ok &= isfinite(P[k]); }
+    if (placed) {
+      pose16_to_f32x12(P, placed_T + 12 * r);
+    } else {
+      double inv[16];
+      invert_pose(P, inv);
+      for (int k = 0; k < 12; ++k) T[12 * r + k] = (float)inv[k];
+    }
+  }
+  if (!ok) *status = PGP_E_INVALID;
+}
+
+// Step 3: the host half of one item, one CTA per item -- n_unexplained, n_keep and, for an item with k > 0 and n_keep >= 3, its
+// survivors in Morton order into its slot of the packed source, with ns and n_keep written into its K5 descriptor.  The bounding
+// box is exact (min / max), the codes are morton_code's.  A survivor keeps its segment index i, and the unique keys
+// (code << 32 | i) are sorted: compaction keeps the original order, so this is the order std::sort gives morton_source's
+// (code, survivor index) pairs.  Bitonic sort over the next power of two, with non-survivors and padding at ~0 (after every
+// code of 30 bits); __syncthreads orders the global-memory passes as it does the shared ones.
+__global__ void __launch_bounds__(TT) k5_prep_items(const float4* __restrict__ in4, const uint8_t* __restrict__ flags, const PrepItem* __restrict__ items,
+                                                    K5Item* __restrict__ desc, float4* __restrict__ src, uint64_t* __restrict__ gkeys, float trim,
+                                                    int* __restrict__ n_unexplained, const int32_t* __restrict__ status) {
+  extern __shared__ uint64_t s_keys[];
+  __shared__ float s_box[TT / 32][6];
+  __shared__ int s_cnt[TT / 32];
+  if (*status) return;
+  const PrepItem P = items[blockIdx.x];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const float4* seg = in4 + P.seg_lo;
+  const uint8_t* fl = P.flag_lo >= 0 ? flags + P.flag_lo : nullptr;
+  float b[6] = {INFINITY, INFINITY, INFINITY, -INFINITY, -INFINITY, -INFINITY};      // lo, hi of the survivors
+  int cnt = 0;
+  for (int i = tid; i < P.ns; i += TT)
+    if (!fl || !fl[i]) {
+      const float4 s = seg[i];
+      ++cnt;
+      b[0] = fminf(b[0], s.x); b[1] = fminf(b[1], s.y); b[2] = fminf(b[2], s.z);
+      b[3] = fmaxf(b[3], s.x); b[4] = fmaxf(b[4], s.y); b[5] = fmaxf(b[5], s.z);
+    }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      b[c] = fminf(b[c], __shfl_xor_sync(0xffffffffu, b[c], o));
+      b[3 + c] = fmaxf(b[3 + c], __shfl_xor_sync(0xffffffffu, b[3 + c], o));
+    }
+  }
+  if (lane == 0) { s_cnt[warp] = cnt; for (int c = 0; c < 6; ++c) s_box[warp][c] = b[c]; }
+  __syncthreads();
+  cnt = 0;
+  for (int w = 0; w < TT / 32; ++w) {
+    cnt += s_cnt[w];
+    for (int c = 0; c < 3; ++c) { b[c] = fminf(b[c], s_box[w][c]); b[3 + c] = fmaxf(b[3 + c], s_box[w][3 + c]); }
+  }
+  if (tid == 0 && n_unexplained) n_unexplained[blockIdx.x] = cnt;
+  if (P.k == 0) return;
+  const int n_keep = n_keep_of(trim, cnt);
+  if (tid == 0) { desc[blockIdx.x].p.ns = cnt; desc[blockIdx.x].p.n_keep = n_keep; }
+  if (n_keep < 3) return;
+  const float lo[3] = {b[0], b[1], b[2]}, hi[3] = {b[3], b[4], b[5]};
+  const float ext = morton_extent(lo, hi);
+  const int n2 = pow2_at_least(P.ns);
+  uint64_t* keys = P.key_lo >= 0 ? gkeys + P.key_lo : s_keys;
+  for (int i = tid; i < n2; i += TT) {
+    uint64_t key = ~0ull;
+    if (i < P.ns && (!fl || !fl[i])) { const float4 s = seg[i]; key = morton_code(s.x, s.y, s.z, lo, ext) << 32 | (uint32_t)i; }
+    keys[i] = key;
+  }
+  __syncthreads();
+  for (int k = 2; k <= n2; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int i = tid; i < n2; i += TT) {
+        const int l = i ^ j;
+        if (l > i) {
+          const uint64_t x = keys[i], y = keys[l];
+          if ((x > y) == ((i & k) == 0)) { keys[i] = y; keys[l] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  for (int r = tid; r < cnt; r += TT) src[P.src_lo + r] = seg[(uint32_t)keys[r]];
+}
+
+// Step 6, one thread per pose (finish_poses): pose = inverse(tform) when the energy is finite, and the iterations and energy; an
+// item that K5 skipped (n_keep < 3) keeps its poses and gets 0 / 0.  Nothing is written when the call was refused.
+__global__ void k5_finish(const K5Item* __restrict__ desc, const int* __restrict__ pose_item, const float* __restrict__ T, const int* __restrict__ it,
+                          const float* __restrict__ en, int n_poses, double* __restrict__ poses16, int* __restrict__ iters_out,
+                          float* __restrict__ energy_out, const int32_t* __restrict__ status) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_poses || *status) return;
+  int iv = 0;
+  float ev = 0.f;
+  if (desc[pose_item[i]].p.n_keep >= 3) {
+    iv = it[i]; ev = en[i];
+    if (ev <= FLT_MAX) {
+      double M[16] = {0}, inv[16];
+      for (int k = 0; k < 12; ++k) M[k] = (double)T[12 * (size_t)i + k];
+      M[15] = 1;
+      invert_pose(M, inv);
+      for (int k = 0; k < 16; ++k) poses16[16 * (size_t)i + k] = inv[k];
+    }
+  }
+  if (iters_out) iters_out[i] = iv;
+  if (energy_out) energy_out[i] = ev;
 }
 
 }  // namespace
@@ -728,112 +898,172 @@ int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* 
   return PGP_OK;
 }
 
-// pgp_refine_batch after its checks (pgp_api.cu): K6 over every item with placed objects (one launch, one copy back), the host
-// half of every item (compaction, n_keep, Morton order, start transforms), then ONE K5 launch of 2 * sum(k) CTAs over the items
-// with n_keep >= 3.  Each item runs exactly the arithmetic of its single call: its own source, target grid and scratch rows.
-int k5_refine_batch(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16, int64_t n_placed_rows,
-                    const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold, float trim,
-                    float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out) {
-  if (n_items == 0) return PGP_OK;
+static size_t align16(size_t n) { return (n + 15) & ~(size_t)15; }
+
+// pgp_refine_batch_dev after its checks (pgp_api.cu).  The host lays the batch out from the structure alone, builds the K5
+// descriptors, the item table of k5_prep_items, K6's job table and the pose -> item map, and sends them up in ONE copy from pinned
+// staging; the descriptors' ns and n_keep are filled in on the device.  Each item runs exactly the arithmetic of its single call.
+int k5_refine_batch_dev(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16,
+                        int64_t n_placed_rows, const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16,
+                        float threshold, float trim, float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out,
+                        int32_t* status) {
   TScratch& ts = tscratch_of(ctx);
+  cudaStream_t st = ctx->stream;
   for (int i = 0; i < n_items; ++i) {                                   // (cached per model: built once for each distinct obj)
     int rc = build_target_grid(ctx, ctx->models[items[i].obj]);
     if (rc) return rc;
   }
-  // 1. explained points: every item with placed objects, flags in item order
-  std::vector<K6Job> jobs;
-  std::vector<int64_t> flag_lo((size_t)n_items, -1);
-  int64_t n_flags = 0;
+  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
+  std::vector<PrepItem> prep((size_t)n_items);
+  std::vector<K6Dev> jobs;
+  int64_t n_flags = 0, n_blocks = 0, n_src = 0, n_keys = 0, n_scr = 0;
+  int smem_keys = 0;
   for (int i = 0; i < n_items; ++i) {
     const pgp_refine_item& it = items[i];
-    if (it.n_placed <= 0) continue;
-    const int ns = (int)(seg_offsets[it.seg + 1] - seg_offsets[it.seg]);
-    jobs.push_back(K6Job{&ctx->models[it.obj], seg_offsets[it.seg], ns, (int64_t)it.placed_lo, it.n_placed});
-    flag_lo[(size_t)i] = n_flags;
-    n_flags += ns;
-  }
-  std::vector<uint8_t> flags((size_t)n_flags);
-  if (!jobs.empty()) {
-    int rc = k6_flag_batch(ctx, seg_xyz, seg_offsets[n_segs], placed16, n_placed_rows, jobs, threshold, flags.data());
-    if (rc) return rc;
-  }
-  // 2. the host half of every item; items left out of the launch get their results here
-  struct Active { int item, ns, n_keep, k, pose_lo; int64_t src_lo, scr_lo; };
-  std::vector<Active> act;
-  std::vector<float> src4, T, un;
-  int64_t n_src = 0, n_scr = 0;
-  int n_poses = 0;
-  for (int i = 0; i < n_items; ++i) {
-    const pgp_refine_item& it = items[i];
-    const float* seg = seg_xyz + 3 * seg_offsets[it.seg];
     const int ns = (int)(seg_offsets[it.seg + 1] - seg_offsets[it.seg]);
     const int k = (int)(pose_offsets[i + 1] - pose_offsets[i]);
-    int kept = ns;
-    if (flag_lo[(size_t)i] >= 0) {                                      // extract.setNegative(true): the survivors in their original order
-      un.resize((size_t)ns * 3);
-      kept = k6_compact(seg, ns, flags.data() + flag_lo[(size_t)i], un.data());
-      seg = un.data();
+    PrepItem& P = prep[(size_t)i];
+    P = PrepItem{seg_offsets[it.seg], -1, -1, -1, ns, k};
+    if (it.n_placed > 0) {
+      const Model& m = ctx->models[it.obj];
+      jobs.push_back(K6Dev{m.val_raw.as<float4>(), m.nv, ns, it.n_placed, P.seg_lo, (int64_t)it.placed_lo, n_flags, n_blocks});
+      P.flag_lo = n_flags;
+      n_flags += ns; n_blocks += (ns + K6_T - 1) / K6_T;
     }
-    if (n_unexplained_out) n_unexplained_out[i] = kept;
-    if (k == 0) continue;
-    int* it_out = iters_out ? iters_out + pose_offsets[i] : nullptr;
-    float* en_out = energy_out ? energy_out + pose_offsets[i] : nullptr;
-    const int n_keep = n_keep_of(trim, kept);
-    if (n_keep < 3) { zero_results(k, it_out, en_out); continue; }     // (kept = 0 included)
-    act.push_back(Active{i, kept, n_keep, k, n_poses, n_src, n_scr});
-    src4.resize((size_t)(n_src + kept) * 4);
-    morton_source(seg, kept, src4.data() + 4 * n_src);
-    T.resize((size_t)(n_poses + k) * 12);
-    start_transforms(poses16 + 16 * pose_offsets[i], k, T.data() + 12 * (size_t)n_poses);
-    n_src += kept; n_scr += (int64_t)k * kept; n_poses += k;
+    if (k > 0) {
+      P.src_lo = n_src;
+      n_src += ns; n_scr += (int64_t)k * ns;
+      if (ns > K5_SORT_SHARED) { P.key_lo = n_keys; n_keys += pow2_at_least(ns); }
+      else smem_keys = std::max(smem_keys, pow2_at_least(ns));
+    }
   }
-  if (act.empty()) return PGP_OK;
-  // 3. one launch: packed sources, start transforms, a descriptor per item and the pose -> item map, each up in one copy
+  const size_t o_prep = align16((size_t)n_items * sizeof(K5Item)), o_jobs = o_prep + align16((size_t)n_items * sizeof(PrepItem));
+  const size_t o_map = o_jobs + align16(jobs.size() * sizeof(K6Dev)), blob = o_map + (size_t)n_poses * 4;
+  PGP_CUDA(ctx, ts.in4.reserve((size_t)n_pts * 16));
+  PGP_CUDA(ctx, ts.placed_T.reserve((size_t)n_placed_rows * 48));
+  PGP_CUDA(ctx, ts.flags.reserve((size_t)n_flags));
   PGP_CUDA(ctx, ts.seg.reserve((size_t)n_src * 16));
+  PGP_CUDA(ctx, ts.keys.reserve((size_t)n_keys * 8));
   PGP_CUDA(ctx, ts.d2.reserve((size_t)n_scr * 4));
   PGP_CUDA(ctx, ts.nn.reserve((size_t)n_scr * 4));
   PGP_CUDA(ctx, ts.T.reserve((size_t)n_poses * 48));
   PGP_CUDA(ctx, ts.iters.reserve((size_t)n_poses * 4));
   PGP_CUDA(ctx, ts.energy.reserve((size_t)n_poses * 4));
-  PGP_CUDA(ctx, ts.items.reserve(act.size() * sizeof(K5Item)));
-  PGP_CUDA(ctx, ts.pose_item.reserve((size_t)n_poses * 4));
-  std::vector<K5Item> desc(act.size());
-  std::vector<int> pose_item((size_t)n_poses);
-  for (size_t a = 0; a < act.size(); ++a) {
-    const Active& A = act[a];
-    desc[a].p = item_params(ctx->models[items[A.item].obj], ts.seg.as<float4>() + A.src_lo, A.ns, ts.d2.as<float>() + A.scr_lo,
-                            ts.nn.as<int>() + A.scr_lo, ts.T.as<float>() + 12 * (size_t)A.pose_lo, ts.iters.as<int>() + A.pose_lo,
-                            ts.energy.as<float>() + A.pose_lo, A.n_keep, ratio, max_iter);
-    desc[a].pose_lo = A.pose_lo;
-    for (int j = 0; j < A.k; ++j) pose_item[(size_t)A.pose_lo + j] = (int)a;
+  PGP_CUDA(ctx, ts.items.reserve(blob));
+  // 1. ingest (also for n_items = 0: the values are checked all the same)
+  PGP_CUDA(ctx, cudaMemsetAsync(status, 0, sizeof(int32_t), st));       // PGP_OK
+  const int64_t n_in = n_pts + n_placed_rows + n_poses;
+  if (n_in > 0) {
+    k5_ingest<<<(unsigned)std::min<int64_t>((n_in + 255) / 256, 16 * ctx->sm_count), 256, 0, st>>>(
+        seg_xyz, n_pts, placed16, n_placed_rows, poses16, n_poses, ts.in4.as<float4>(), ts.placed_T.as<float>(), ts.T.as<float>(), status);
+    ctx->launches++;
+    PGP_CUDA(ctx, cudaGetLastError());
   }
-  PGP_CUDA(ctx, cudaMemcpyAsync(ts.seg.p, src4.data(), (size_t)n_src * 16, cudaMemcpyHostToDevice, ctx->stream));
-  PGP_CUDA(ctx, cudaMemcpyAsync(ts.T.p, T.data(), (size_t)n_poses * 48, cudaMemcpyHostToDevice, ctx->stream));
-  PGP_CUDA(ctx, cudaMemcpyAsync(ts.items.p, desc.data(), desc.size() * sizeof(K5Item), cudaMemcpyHostToDevice, ctx->stream));
-  PGP_CUDA(ctx, cudaMemcpyAsync(ts.pose_item.p, pose_item.data(), (size_t)n_poses * 4, cudaMemcpyHostToDevice, ctx->stream));
-  const K5Batch b{ts.items.as<K5Item>(), ts.pose_item.as<int>()};
-  if (plane) k5_tricp_kernel<true, true><<<2 * n_poses, TT, 0, ctx->stream>>>(b);
-  else k5_tricp_kernel<false, true><<<2 * n_poses, TT, 0, ctx->stream>>>(b);
+  if (n_items == 0) return PGP_OK;
+  // the tables, staged in the next pinned buffer: its previous upload ran long ago unless K5_STAGES calls are still queued.  The
+  // buffers grow together, so that one call of a size readies every later call of that size.
+  if (ts.stage[0].cap < blob) {
+    const size_t cap = blob + blob / 4 + 256;
+    for (Staging& g : ts.stage) {
+      if (!g.copied) PGP_CUDA(ctx, cudaEventCreateWithFlags(&g.copied, cudaEventDisableTiming));
+      PGP_CUDA(ctx, cudaEventSynchronize(g.copied));
+      if (g.host) cudaFreeHost(g.host);
+      g.host = nullptr; g.cap = 0;
+      PGP_CUDA(ctx, cudaMallocHost(&g.host, cap));
+      g.cap = cap;
+    }
+  }
+  Staging& sg = ts.stage[ts.next_stage++ % K5_STAGES];
+  PGP_CUDA(ctx, cudaEventSynchronize(sg.copied));
+  char* h = static_cast<char*>(sg.host);
+  K5Item* desc = reinterpret_cast<K5Item*>(h);
+  int* pose_item = reinterpret_cast<int*>(h + o_map);
+  int64_t scr = 0;
+  for (int i = 0; i < n_items; ++i) {
+    const PrepItem& P = prep[(size_t)i];
+    const int64_t lo = pose_offsets[i];
+    desc[i] = K5Item{};
+    if (P.k == 0) continue;
+    desc[i].p = item_params(ctx->models[items[i].obj], ts.seg.as<float4>() + P.src_lo, 0, ts.d2.as<float>() + scr, ts.nn.as<int>() + scr,
+                            ts.T.as<float>() + 12 * lo, ts.iters.as<int>() + lo, ts.energy.as<float>() + lo, 0, ratio, max_iter);
+    desc[i].pose_lo = (int)lo;
+    for (int j = 0; j < P.k; ++j) pose_item[lo + j] = i;
+    scr += (int64_t)P.k * P.ns;
+  }
+  memcpy(h + o_prep, prep.data(), prep.size() * sizeof(PrepItem));
+  if (!jobs.empty()) memcpy(h + o_jobs, jobs.data(), jobs.size() * sizeof(K6Dev));
+  PGP_CUDA(ctx, cudaMemcpyAsync(ts.items.p, sg.host, blob, cudaMemcpyHostToDevice, st));
+  PGP_CUDA(ctx, cudaEventRecord(sg.copied, st));
+  const K5Item* desc_dev = ts.items.as<K5Item>();
+  const int* map_dev = reinterpret_cast<const int*>(ts.items.as<char>() + o_map);
+  // 2. explained points
+  int rc = k6_mark_batch_dev(ctx, ts.in4.as<float4>(), reinterpret_cast<const K6Dev*>(ts.items.as<char>() + o_jobs), (int)jobs.size(), n_blocks,
+                             ts.placed_T.as<float>(), threshold, ts.flags.as<uint8_t>());
+  if (rc) return rc;
+  // 3. compaction, n_keep, Morton order
+  if (!ts.prep_smem_set) {
+    PGP_CUDA(ctx, cudaFuncSetAttribute(k5_prep_items, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * K5_SORT_SHARED));
+    ts.prep_smem_set = true;
+  }
+  k5_prep_items<<<n_items, TT, (size_t)smem_keys * 8, st>>>(ts.in4.as<float4>(), ts.flags.as<uint8_t>(),
+                                                           reinterpret_cast<const PrepItem*>(ts.items.as<char>() + o_prep), ts.items.as<K5Item>(),
+                                                           ts.seg.as<float4>(), ts.keys.as<uint64_t>(), trim, n_unexplained_out, status);
   ctx->launches++;
   PGP_CUDA(ctx, cudaGetLastError());
-  std::vector<int> it((size_t)n_poses);
-  std::vector<float> en((size_t)n_poses);
-  PGP_CUDA(ctx, cudaMemcpyAsync(T.data(), ts.T.p, (size_t)n_poses * 48, cudaMemcpyDeviceToHost, ctx->stream));
-  PGP_CUDA(ctx, cudaMemcpyAsync(it.data(), ts.iters.p, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  PGP_CUDA(ctx, cudaMemcpyAsync(en.data(), ts.energy.p, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  PGP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  for (const Active& A : act) {
-    const int64_t lo = pose_offsets[A.item];
-    finish_poses(T.data() + 12 * (size_t)A.pose_lo, it.data() + A.pose_lo, en.data() + A.pose_lo, A.k, poses16 + 16 * lo,
-                 iters_out ? iters_out + lo : nullptr, energy_out ? energy_out + lo : nullptr);
+  if (n_poses == 0) return PGP_OK;
+  // 5. one cluster of two CTAs per pose of every item; 6. the poses back
+  const K5Batch b{desc_dev, map_dev};
+  if (plane) k5_tricp_kernel<true, true><<<2 * (unsigned)n_poses, TT, 0, st>>>(b);
+  else k5_tricp_kernel<false, true><<<2 * (unsigned)n_poses, TT, 0, st>>>(b);
+  k5_finish<<<(unsigned)((n_poses + 255) / 256), 256, 0, st>>>(desc_dev, map_dev, ts.T.as<float>(), ts.iters.as<int>(), ts.energy.as<float>(), (int)n_poses,
+                                                               poses16, iters_out, energy_out, status);
+  ctx->launches += 2;
+  PGP_CUDA(ctx, cudaGetLastError());
+  return PGP_OK;
+}
+
+// pgp_refine_batch after its checks: its arguments up, the device pipeline, the results down, one synchronisation.
+int k5_refine_batch(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16, int64_t n_placed_rows,
+                    const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold, float trim,
+                    float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out) {
+  if (n_items == 0) return PGP_OK;
+  TScratch& ts = tscratch_of(ctx);
+  cudaStream_t st = ctx->stream;
+  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
+  PGP_CUDA(ctx, ts.raw_seg.reserve((size_t)n_pts * 12));
+  PGP_CUDA(ctx, ts.raw_placed.reserve((size_t)n_placed_rows * 128));
+  PGP_CUDA(ctx, ts.raw_poses.reserve((size_t)n_poses * 128));
+  PGP_CUDA(ctx, ts.out.reserve((size_t)n_poses * 8 + (size_t)n_items * 4 + 4));
+  int* it_dev = ts.out.as<int>();
+  float* en_dev = reinterpret_cast<float*>(it_dev + n_poses);
+  int* nun_dev = it_dev + 2 * n_poses;
+  int32_t* status = nun_dev + n_items;
+  if (n_pts) PGP_CUDA(ctx, cudaMemcpyAsync(ts.raw_seg.p, seg_xyz, (size_t)n_pts * 12, cudaMemcpyHostToDevice, st));
+  if (n_placed_rows) PGP_CUDA(ctx, cudaMemcpyAsync(ts.raw_placed.p, placed16, (size_t)n_placed_rows * 128, cudaMemcpyHostToDevice, st));
+  if (n_poses) PGP_CUDA(ctx, cudaMemcpyAsync(ts.raw_poses.p, poses16, (size_t)n_poses * 128, cudaMemcpyHostToDevice, st));
+  int rc = k5_refine_batch_dev(ctx, plane, ts.raw_seg.as<float>(), seg_offsets, n_segs, ts.raw_placed.as<double>(), n_placed_rows, items, pose_offsets,
+                               n_items, ts.raw_poses.as<double>(), threshold, trim, ratio, max_iter, it_dev, en_dev, nun_dev, status);
+  if (rc) return rc;
+  if (n_poses) {
+    PGP_CUDA(ctx, cudaMemcpyAsync(poses16, ts.raw_poses.p, (size_t)n_poses * 128, cudaMemcpyDeviceToHost, st));
+    if (iters_out) PGP_CUDA(ctx, cudaMemcpyAsync(iters_out, it_dev, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, st));
+    if (energy_out) PGP_CUDA(ctx, cudaMemcpyAsync(energy_out, en_dev, (size_t)n_poses * 4, cudaMemcpyDeviceToHost, st));
   }
+  if (n_unexplained_out) PGP_CUDA(ctx, cudaMemcpyAsync(n_unexplained_out, nun_dev, (size_t)n_items * 4, cudaMemcpyDeviceToHost, st));
+  PGP_CUDA(ctx, cudaStreamSynchronize(st));
   return PGP_OK;
 }
 
 void k5_release(pgp_ctx* ctx) {
   if (!ctx->k5_scratch) return;
   TScratch* ts = static_cast<TScratch*>(ctx->k5_scratch);
-  for (DevBuf* b : {&ts->seg, &ts->d2, &ts->nn, &ts->T, &ts->iters, &ts->energy, &ts->cell_of, &ts->cursor, &ts->items, &ts->pose_item}) b->release();
+  for (DevBuf* b : {&ts->seg, &ts->d2, &ts->nn, &ts->T, &ts->iters, &ts->energy, &ts->cell_of, &ts->cursor, &ts->items, &ts->in4, &ts->placed_T,
+                    &ts->flags, &ts->keys, &ts->raw_seg, &ts->raw_placed, &ts->raw_poses, &ts->out})
+    b->release();
+  for (Staging& sg : ts->stage) {
+    if (sg.host) cudaFreeHost(sg.host);
+    if (sg.copied) cudaEventDestroy(sg.copied);
+  }
   delete ts;
   ctx->k5_scratch = nullptr;
 }

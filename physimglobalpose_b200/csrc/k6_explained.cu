@@ -22,8 +22,6 @@ __global__ void k6_transform(const float4* __restrict__ model, int nv, const flo
                        xf_row(T[8], T[9], T[10], T[11], p.x, p.y, p.z), 0.f);
 }
 
-constexpr int K6_T = 256;
-
 // whether any of the m tile points lies strictly within r of s
 __device__ __forceinline__ bool tile_hit(const float4 s, const float4* tile, int m, float r2) {
   for (int t = 0; t < m; ++t) {
@@ -50,9 +48,6 @@ __global__ void __launch_bounds__(K6_T) k6_mark(const float4* __restrict__ seg, 
   }
   if (i < ns) flag[i] = hit ? 1 : 0;
 }
-
-// k6_flag_batch's jobs on the device: block_lo = first block of the job (blocks map to (job, 256-point tile of its segment))
-struct K6Dev { const float4* model; int nv, ns, n_placed; int64_t seg_lo, placed_lo, flag_lo, block_lo; };
 
 // k6_mark for many (segment, placed set) jobs at once.  The explained cloud is not materialised: the tile loader transforms the
 // model point with k6_transform's arithmetic, in k6_transform's order (placed row major, model point minor), so every job gets
@@ -84,7 +79,7 @@ __global__ void __launch_bounds__(K6_T) k6_mark_batch(const float4* __restrict__
 }
 
 // owned by the context, released by k6_release (pgp_destroy)
-struct K6Scratch { DevBuf seg, expl, T, flag, jobs; };
+struct K6Scratch { DevBuf seg, expl, T, flag; };
 K6Scratch& k6_scratch_of(pgp_ctx* ctx) {
   if (!ctx->k6_scratch) ctx->k6_scratch = new K6Scratch();
   return *static_cast<K6Scratch*>(ctx->k6_scratch);
@@ -122,35 +117,12 @@ int k6_remove_explained(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int n
   return PGP_OK;
 }
 
-int k6_flag_batch(pgp_ctx* ctx, const float* seg_xyz_host, int64_t n_seg_pts, const double* placed16_host, int64_t n_placed_rows,
-                  const std::vector<K6Job>& jobs, float threshold, uint8_t* flags_host) {
-  K6Scratch& sc = k6_scratch_of(ctx);
-  cudaStream_t st = ctx->stream;
-  std::vector<float> seg4((size_t)n_seg_pts * 4, 0.f), T((size_t)n_placed_rows * 12);
-  for (int64_t i = 0; i < n_seg_pts; ++i) for (int c = 0; c < 3; ++c) seg4[4 * (size_t)i + c] = seg_xyz_host[3 * i + c];
-  for (int64_t k = 0; k < n_placed_rows; ++k) pose16_to_f32x12(placed16_host + 16 * (size_t)k, &T[12 * (size_t)k]);
-  std::vector<K6Dev> dev(jobs.size());
-  int64_t n_flags = 0, n_blocks = 0;
-  for (size_t j = 0; j < jobs.size(); ++j) {
-    const K6Job& J = jobs[j];
-    dev[j] = K6Dev{J.m->val_raw.as<float4>(), J.m->nv, J.ns, J.n_placed, J.seg_lo, J.placed_lo, n_flags, n_blocks};
-    n_flags += J.ns;
-    n_blocks += (J.ns + K6_T - 1) / K6_T;
-  }
+int k6_mark_batch_dev(pgp_ctx* ctx, const float4* seg4, const K6Dev* jobs_dev, int n_jobs, int64_t n_blocks, const float* T12, float threshold,
+                      uint8_t* flags_dev) {
   if (n_blocks == 0) return PGP_OK;                          // (pgp_refine_batch bounds the flags, so n_blocks < 2^31)
-  PGP_CUDA(ctx, sc.seg.reserve((size_t)n_seg_pts * 16));
-  PGP_CUDA(ctx, sc.T.reserve((size_t)n_placed_rows * 48));
-  PGP_CUDA(ctx, sc.jobs.reserve(dev.size() * sizeof(K6Dev)));
-  PGP_CUDA(ctx, sc.flag.reserve((size_t)n_flags));
-  PGP_CUDA(ctx, cudaMemcpyAsync(sc.seg.p, seg4.data(), (size_t)n_seg_pts * 16, cudaMemcpyHostToDevice, st));
-  PGP_CUDA(ctx, cudaMemcpyAsync(sc.T.p, T.data(), (size_t)n_placed_rows * 48, cudaMemcpyHostToDevice, st));
-  PGP_CUDA(ctx, cudaMemcpyAsync(sc.jobs.p, dev.data(), dev.size() * sizeof(K6Dev), cudaMemcpyHostToDevice, st));
-  k6_mark_batch<<<(unsigned)n_blocks, K6_T, 0, st>>>(sc.seg.as<float4>(), sc.jobs.as<K6Dev>(), (int)dev.size(), sc.T.as<float>(), threshold * threshold,
-                                                    sc.flag.as<uint8_t>());
+  k6_mark_batch<<<(unsigned)n_blocks, K6_T, 0, ctx->stream>>>(seg4, jobs_dev, n_jobs, T12, threshold * threshold, flags_dev);
   ctx->launches++;
   PGP_CUDA(ctx, cudaGetLastError());
-  PGP_CUDA(ctx, cudaMemcpyAsync(flags_host, sc.flag.p, (size_t)n_flags, cudaMemcpyDeviceToHost, st));
-  PGP_CUDA(ctx, cudaStreamSynchronize(st));
   return PGP_OK;
 }
 
@@ -164,7 +136,7 @@ int k6_compact(const float* seg_xyz_host, int ns, const uint8_t* flags, float* o
 void k6_release(pgp_ctx* ctx) {
   if (!ctx->k6_scratch) return;
   K6Scratch* sc = static_cast<K6Scratch*>(ctx->k6_scratch);
-  for (DevBuf* b : {&sc->seg, &sc->expl, &sc->T, &sc->flag, &sc->jobs}) b->release();
+  for (DevBuf* b : {&sc->seg, &sc->expl, &sc->T, &sc->flag}) b->release();
   delete sc;
   ctx->k6_scratch = nullptr;
 }

@@ -860,46 +860,85 @@ static bool csr_offsets_ok(const int64_t* off, int n) {
   return true;
 }
 
+// The checks of pgp_refine_batch (host_values: the arrays are host memory and their values are checked too) and of
+// pgp_refine_batch_dev (the device pointers are checked instead, the values on the device).
+static int refine_batch_checks(pgp_ctx* ctx, const char* fn, bool host_values, int metric, const float* seg_xyz, const int64_t*& seg_offsets,
+                               int n_segs, const double* placed16, int64_t n_placed_rows, const pgp_refine_item* items, const int64_t*& pose_offsets,
+                               int n_items, const double* poses16, float threshold, float trim, float ratio) {
+  static const int64_t zero = 0;
+  if (metric != PGP_ICP_POINT && metric != PGP_ICP_PLANE) return pgp_fail(ctx, PGP_E_INVALID, "%s: metric must be 0 or 1", fn);
+  if (n_items < 0 || n_segs < 0 || n_placed_rows < 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: negative count", fn);
+  if (!seg_offsets && n_segs > 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: null seg_offsets", fn);
+  if (!pose_offsets && n_items > 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: null pose_offsets", fn);
+  if (!seg_offsets) seg_offsets = &zero;
+  if (!pose_offsets) pose_offsets = &zero;
+  if (!csr_offsets_ok(seg_offsets, n_segs)) return pgp_fail(ctx, PGP_E_INVALID, "%s: seg_offsets must be non-decreasing from 0", fn);
+  if (!csr_offsets_ok(pose_offsets, n_items)) return pgp_fail(ctx, PGP_E_INVALID, "%s: pose_offsets must be non-decreasing from 0", fn);
+  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
+  if (n_pts > PGP_REFINE_MAX_POINTS) return pgp_fail(ctx, PGP_E_INVALID, "%s: more than PGP_REFINE_MAX_POINTS segment points", fn);
+  if (n_poses > PGP_REFINE_MAX_POSES) return pgp_fail(ctx, PGP_E_INVALID, "%s: more than PGP_REFINE_MAX_POSES poses", fn);
+  if ((n_pts > 0 && !seg_xyz) || (n_placed_rows > 0 && !placed16) || (n_items > 0 && !items) || (n_poses > 0 && !poses16))
+    return pgp_fail(ctx, PGP_E_INVALID, "%s: null argument", fn);
+  if (host_values && (!all_finite(seg_xyz, 3 * n_pts) || !all_finite(placed16, 16 * n_placed_rows) || !all_finite(poses16, 16 * n_poses)))
+    return pgp_fail(ctx, PGP_E_INVALID, "%s: non-finite segment point, placed pose or pose", fn);
+  if (!(trim > 0.f) || !(ratio > 0.f) || !(threshold >= 0.f))
+    return pgp_fail(ctx, PGP_E_INVALID, "%s: trim and ratio must be > 0 and threshold >= 0", fn);
+  int64_t pairs = 0;
+  for (int i = 0; i < n_items; ++i) {
+    const pgp_refine_item& it = items[i];
+    if (it.seg < 0 || it.seg >= n_segs) return pgp_fail(ctx, PGP_E_INVALID, "%s: item %d: segment %d outside [0, %d)", fn, i, it.seg, n_segs);
+    const int64_t ns = seg_offsets[it.seg + 1] - seg_offsets[it.seg];
+    if (ns == 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: item %d: segment %d is empty", fn, i, it.seg);
+    if (it.n_placed < 0 || it.placed_lo < 0 || (int64_t)it.placed_lo + it.n_placed > n_placed_rows)
+      return pgp_fail(ctx, PGP_E_INVALID, "%s: item %d: placed rows outside [0, %lld)", fn, i, (long long)n_placed_rows);
+    Model* m = get_model(ctx, it.obj);
+    if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "%s: item %d: no model in slot %d", fn, i, it.obj);
+    if (metric == PGP_ICP_PLANE && !m->val_has_nrm)
+      return pgp_fail(ctx, PGP_E_INVALID, "%s: item %d: model slot %d was set without validation normals", fn, i, it.obj);
+    // d2 / nn rows of the poses, and the explained flags (each factor is at most 2^30 + 1: no overflow before the check)
+    pairs += (pose_offsets[i + 1] - pose_offsets[i] + (it.n_placed > 0 ? 1 : 0)) * ns;
+    if (pairs > PGP_REFINE_MAX_PAIRS) return pgp_fail(ctx, PGP_E_INVALID, "%s: scratch above PGP_REFINE_MAX_PAIRS", fn);
+  }
+  return PGP_OK;
+}
+
 int pgp_refine_batch(pgp_ctx* ctx, int metric, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16,
                      int64_t n_placed_rows, const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold,
                      float trim, float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out) {
   CHECK_CTX(ctx);
-  static const int64_t zero = 0;
-  if (metric != PGP_ICP_POINT && metric != PGP_ICP_PLANE) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: metric must be 0 or 1");
-  if (n_items < 0 || n_segs < 0 || n_placed_rows < 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: negative count");
-  if (!seg_offsets && n_segs > 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null seg_offsets");
-  if (!pose_offsets && n_items > 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null pose_offsets");
-  if (!seg_offsets) seg_offsets = &zero;
-  if (!pose_offsets) pose_offsets = &zero;
-  if (!csr_offsets_ok(seg_offsets, n_segs)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: seg_offsets must be non-decreasing from 0");
-  if (!csr_offsets_ok(pose_offsets, n_items)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: pose_offsets must be non-decreasing from 0");
-  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
-  if (n_pts > PGP_REFINE_MAX_POINTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: more than PGP_REFINE_MAX_POINTS segment points");
-  if (n_poses > PGP_REFINE_MAX_POSES) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: more than PGP_REFINE_MAX_POSES poses");
-  if ((n_pts > 0 && !seg_xyz) || (n_placed_rows > 0 && !placed16) || (n_items > 0 && !items) || (n_poses > 0 && !poses16))
-    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: null argument");
-  if (!all_finite(seg_xyz, 3 * n_pts) || !all_finite(placed16, 16 * n_placed_rows) || !all_finite(poses16, 16 * n_poses))
-    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: non-finite segment point, placed pose or pose");
-  if (!(trim > 0.f) || !(ratio > 0.f) || !(threshold >= 0.f))
-    return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: trim and ratio must be > 0 and threshold >= 0");
-  int64_t pairs = 0;
-  for (int i = 0; i < n_items; ++i) {
-    const pgp_refine_item& it = items[i];
-    if (it.seg < 0 || it.seg >= n_segs) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: segment %d outside [0, %d)", i, it.seg, n_segs);
-    const int64_t ns = seg_offsets[it.seg + 1] - seg_offsets[it.seg];
-    if (ns == 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: segment %d is empty", i, it.seg);
-    if (it.n_placed < 0 || it.placed_lo < 0 || (int64_t)it.placed_lo + it.n_placed > n_placed_rows)
-      return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: placed rows outside [0, %lld)", i, (long long)n_placed_rows);
-    Model* m = get_model(ctx, it.obj);
-    if (!m) return pgp_fail(ctx, PGP_E_NO_MODEL, "pgp_refine_batch: item %d: no model in slot %d", i, it.obj);
-    if (metric == PGP_ICP_PLANE && !m->val_has_nrm)
-      return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: item %d: model slot %d was set without validation normals", i, it.obj);
-    // d2 / nn rows of the poses, and the explained flags (each factor is at most 2^30 + 1: no overflow before the check)
-    pairs += (pose_offsets[i + 1] - pose_offsets[i] + (it.n_placed > 0 ? 1 : 0)) * ns;
-    if (pairs > PGP_REFINE_MAX_PAIRS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_refine_batch: scratch above PGP_REFINE_MAX_PAIRS");
-  }
+  int rc = refine_batch_checks(ctx, "pgp_refine_batch", true, metric, seg_xyz, seg_offsets, n_segs, placed16, n_placed_rows, items, pose_offsets, n_items,
+                               poses16, threshold, trim, ratio);
+  if (rc) return rc;
   return k5_refine_batch(ctx, metric == PGP_ICP_PLANE, seg_xyz, seg_offsets, n_segs, placed16, n_placed_rows, items, pose_offsets, n_items, poses16,
                          threshold, trim, ratio, max_iter, iters_out, energy_out, n_unexplained_out);
+}
+
+// device or managed memory of the context's device (a host pointer, registered or not, is neither)
+static bool on_ctx_device(const pgp_ctx* ctx, const void* p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == ctx->device;
+}
+
+int pgp_refine_batch_dev(pgp_ctx* ctx, int metric, const float* seg_xyz_dev, const int64_t* seg_offsets, int n_segs, const double* placed16_dev,
+                         int64_t n_placed_rows, const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16_dev,
+                         float threshold, float trim, float ratio, int max_iter, int* iters_dev, float* energy_dev, int* n_unexplained_dev,
+                         int32_t* status_dev) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_refine_batch_dev";
+  if (!status_dev) return pgp_fail(ctx, PGP_E_INVALID, "%s: null status_dev", fn);
+  int rc = refine_batch_checks(ctx, fn, false, metric, seg_xyz_dev, seg_offsets, n_segs, placed16_dev, n_placed_rows, items, pose_offsets, n_items,
+                               poses16_dev, threshold, trim, ratio);
+  if (rc) return rc;
+  const int64_t n_pts = seg_offsets[n_segs], n_poses = pose_offsets[n_items];
+  const struct { const void* p; bool used; const char* name; } bufs[] = {
+      {status_dev, true, "status_dev"}, {seg_xyz_dev, n_pts > 0, "seg_xyz_dev"}, {placed16_dev, n_placed_rows > 0, "placed16_dev"},
+      {poses16_dev, n_poses > 0, "poses16_dev"}, {iters_dev, iters_dev != nullptr, "iters_dev"}, {energy_dev, energy_dev != nullptr, "energy_dev"},
+      {n_unexplained_dev, n_unexplained_dev != nullptr, "n_unexplained_dev"}};
+  for (const auto& b : bufs)
+    if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
+  return k5_refine_batch_dev(ctx, metric == PGP_ICP_PLANE, seg_xyz_dev, seg_offsets, n_segs, placed16_dev, n_placed_rows, items, pose_offsets, n_items,
+                             poses16_dev, threshold, trim, ratio, max_iter, iters_dev, energy_dev, n_unexplained_dev, status_dev);
 }
 
 int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, int class_id, const float* K9,

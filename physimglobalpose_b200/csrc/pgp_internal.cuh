@@ -246,10 +246,17 @@ void k7_release(pgp_ctx* ctx);
 // plane: the point-to-plane fit (pgp_tricp_plane) instead of the point-to-point one (pgp_tricp)
 int k5_tricp(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, double* poses16_host, int k, float trim, float ratio,
              int max_iter, int* iters_out, float* energy_out, bool plane);
-// pgp_refine_batch after its argument checks
+// pgp_refine_batch after its argument checks: uploads the host arrays, runs k5_refine_batch_dev, downloads, synchronises once
 int k5_refine_batch(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16, int64_t n_placed_rows,
                     const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16, float threshold, float trim,
                     float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out);
+// pgp_refine_batch_dev after its argument checks: the whole batch queued on ctx->stream (seg_xyz, placed16, poses16 and the outputs
+// in device memory, the structure on the host); *status_dev = PGP_OK, or PGP_E_INVALID with no output written when a value is
+// not finite
+int k5_refine_batch_dev(pgp_ctx* ctx, bool plane, const float* seg_xyz, const int64_t* seg_offsets, int n_segs, const double* placed16,
+                        int64_t n_placed_rows, const pgp_refine_item* items, const int64_t* pose_offsets, int n_items, double* poses16,
+                        float threshold, float trim, float ratio, int max_iter, int* iters_out, float* energy_out, int* n_unexplained_out,
+                        int32_t* status_dev);
 
 // ---------------------------------------------------------------------------------------------
 // fp32 arithmetic in the reference's association, every operation individually rounded
@@ -272,7 +279,7 @@ __device__ __forceinline__ float dot3_tree(float a0, float a1, float a2, float b
 __device__ __forceinline__ float cell_coord(float x, float lo, float inv_h) { return __fmul_rn(__fsub_rn(x, lo), inv_h); }
 // utilities::convertToMatrix (Isometry3d -> Matrix4f): the top 3x4 of a row-major 4x4 double pose, each entry rounded to fp32
 // (K6 placed poses, K8 rendered poses)
-inline void pose16_to_f32x12(const double* pose16, float* T12) {
+__host__ __device__ inline void pose16_to_f32x12(const double* pose16, float* T12) {
   for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) T12[4 * r + c] = (float)pose16[4 * r + c];
 }
 // utilities::readDepthImage (PPE/src/misc/utilities.cpp:47-61): ((d << 13) | (d >> 3)) as u16, / 10000 (K7 segments, K8 observations)
@@ -285,12 +292,14 @@ __device__ __forceinline__ bool depth_valid(float d) { return (double)d > 0.1 &&
 // k6_explained.cu
 int k6_remove_explained(pgp_ctx* ctx, Model& m, const float* seg_xyz_host, int ns, const double* placed16_host, int n_placed, float threshold,
                         uint8_t* flags_host, int* n_unexplained);
-// One segment of a batch flagged against model m placed at rows [placed_lo, placed_lo + n_placed) (pgp_refine_batch).
-struct K6Job { const Model* m; int64_t seg_lo; int ns; int64_t placed_lo; int n_placed; };
-// The flags of every job in one launch and one copy back: job j's ns flags follow job j - 1's in flags_host, bit for bit those of
-// k6_remove_explained.  The n_seg_pts points of seg_xyz_host and the n_placed_rows placed rows go up once.
-int k6_flag_batch(pgp_ctx* ctx, const float* seg_xyz_host, int64_t n_seg_pts, const double* placed16_host, int64_t n_placed_rows,
-                  const std::vector<K6Job>& jobs, float threshold, uint8_t* flags_host);
+// One segment of a batch flagged against a model placed at rows [placed_lo, placed_lo + n_placed) of the placed transforms
+// (pgp_refine_batch): its flags start at flag_lo, its blocks of K6_T points at block_lo.
+constexpr int K6_T = 256;
+struct K6Dev { const float4* model; int nv, ns, n_placed; int64_t seg_lo, placed_lo, flag_lo, block_lo; };
+// The flags of every job in one launch on ctx->stream, bit for bit those of k6_remove_explained: seg4 is every segment point
+// (w = 0), T12 every placed row (pose16_to_f32x12), n_blocks the sum over the jobs of ceil(ns / K6_T).
+int k6_mark_batch_dev(pgp_ctx* ctx, const float4* seg4, const K6Dev* jobs_dev, int n_jobs, int64_t n_blocks, const float* T12, float threshold,
+                      uint8_t* flags_dev);
 // the points with flag 0, in their original order (extract.setNegative(true), UCTState.cpp:170-174); returns their number
 int k6_compact(const float* seg_xyz_host, int ns, const uint8_t* flags, float* out_xyz);
 // k7_segment.cu

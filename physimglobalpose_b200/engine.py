@@ -452,6 +452,30 @@ class PoseEngine:
         return [(P[a:b].reshape(-1, 4, 4), iters[a:b], energy[a:b], int(nun[i]))
                 for i, (a, b) in enumerate(zip(pose_off[:-1], pose_off[1:]))]
 
+    def refine_batch_device(self, seg_xyz, seg_offsets, placed, items, pose_offsets, poses, status, iters=None, energy=None,
+                            n_unexplained=None, metric: str = "point", threshold: float = 0.008, trim: float = 0.5, ratio: float = 0.99,
+                            max_iter: int = 100):
+        """pgp_refine_batch_dev: refine_batch on device data, asynchronous on the context's stream (set_stream).
+        Device data, torch CUDA tensors: seg_xyz (n, 3) f32; placed (m, 4, 4) or (m, 16) f64; poses (p, 4, 4) or (p, 16) f64,
+        refined in place; status (1,) i32, PGP_OK or PGP_E_INVALID once the work has run; optional outputs iters (p,) i32,
+        energy (p,) f32, n_unexplained (len(items),) i32.  Structure, numpy: seg_offsets (n_segs + 1,) int64; items (n, 4) int32
+        rows (obj, seg, placed_lo, n_placed); pose_offsets (len(items) + 1,) int64.  The tensors are kept alive until the next call."""
+        import torch
+        icp = {"point": _lib.PGP_ICP_POINT, "plane": _lib.PGP_ICP_PLANE}[metric]
+        want = {"seg_xyz": (seg_xyz, torch.float32), "placed": (placed, torch.float64), "poses": (poses, torch.float64), "status": (status, torch.int32),
+                "iters": (iters, torch.int32), "energy": (energy, torch.float32), "n_unexplained": (n_unexplained, torch.int32)}
+        for name, (t, dt) in want.items():
+            if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of {dt}")
+        seg_off = np.ascontiguousarray(seg_offsets, np.int64)
+        rec = np.ascontiguousarray(items, np.int32).reshape(-1, 4)
+        pose_off = np.ascontiguousarray(pose_offsets, np.int64)
+        self._keep["refine_batch"] = (seg_xyz, placed, poses, status, iters, energy, n_unexplained)
+        dp = lambda t: None if t is None or t.numel() == 0 else t.data_ptr()
+        self._check(self._lib.pgp_refine_batch_dev(self._ctx, icp, dp(seg_xyz), _ptr(seg_off), len(seg_off) - 1, dp(placed), placed.numel() // 16,
+                                                   _ptr(rec) if len(rec) else None, _ptr(pose_off), len(rec), dp(poses), float(threshold), float(trim),
+                                                   float(ratio), int(max_iter), dp(iters), dp(energy), dp(n_unexplained), status.data_ptr()))
+
     # ------------------------------------------------------------------ K7
     def prepare_segment(self, depth_raw_u16, class_mask_u8, class_id: int, K, leaf: float = 0.01, normal_radius: float = 0.02,
                         outlier_radius: float = 0.03, min_neighbors: int = 10, cap: int = 1 << 20):
