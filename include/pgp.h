@@ -535,7 +535,8 @@ PGP_API int pgp_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, c
 PGP_API int pgp_set_depth_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols,
                                       const float* K9, int64_t* class_pixels_out);
 
-/* One state rendered in full: depth_out rows x cols fp32 metres (0 = nothing), slot_out rows x cols (-1 = nothing; NULL allowed). */
+/* One state rendered in full: depth_out rows x cols fp32 metres (0 = nothing), slot_out rows x cols (-1 = nothing; NULL allowed).
+ * PGP_E_TOO_LARGE: the state covers more than 2^31 - 1 (triangle, tile) entries; depth_out and slot_out then hold an empty frame. */
 PGP_API int pgp_render_depth(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n, float* depth_out, int32_t* slot_out);
 
 typedef struct pgp_depth_counts { int32_t rendered, agree, in_front, behind, on_segment; } pgp_depth_counts;
@@ -547,6 +548,33 @@ typedef struct pgp_depth_counts { int32_t rendered, agree, in_front, behind, on_
  * PGP_E_NO_MODEL: an object without a mesh.  n_states = 0 and empty states are valid. */
 PGP_API int pgp_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16,
                            float tau, pgp_depth_counts* out);
+
+/* pgp_depth_cost with the poses and counts in device memory, asynchronous on the context's stream (pgp_set_stream): the form for an
+ * MCTS driver whose refined poses are already on the GPU (pgp_refine_batch_dev), so that refinement, rendering and cost run as one
+ * stream of work.  pgp_depth_cost and pgp_render_depth run this pipeline themselves: they upload, run it, download and
+ * synchronise once.
+ *
+ * Arguments are those of pgp_depth_cost.  On the host: state_offsets and obj_ids (the tree structure; with them every mesh and
+ * every chunk of the work is known without reading anything back).  In device memory (of the context's device, or managed):
+ * poses16_dev (one row-major 4x4 double per record), out_dev (one pgp_depth_counts per record) and status_dev (one int32).  The
+ * call returns once the work is queued, and the host arrays may be reused at once.  Once the context's scratch has grown to the
+ * call's size (a first call of that size), it makes no host synchronisation and no device-to-host copy; a call of a larger size
+ * grows the scratch, and cudaFree / cudaMalloc synchronise the device.
+ *
+ * Results: bitwise those of pgp_depth_cost on the same inputs.  The states are rasterized in chunks cut on the host by triangles,
+ * vertices and (state, tile) bins; each chunk reserves min(2^25, its triangles x the image's 16 x 16 tiles) (triangle, tile) entries.
+ *
+ * Returned at once, with nothing queued and every output untouched: every refusal of pgp_depth_cost that the host can decide (all
+ * but the pose values), status_dev == NULL, and a device argument that cudaPointerGetAttributes does not report as device or
+ * managed memory of the context's device.
+ * On the device, every call sets *status_dev afresh (n_states = 0 included):
+ *   PGP_OK;
+ *   PGP_E_INVALID: a pose entry is NaN or infinite;
+ *   PGP_E_CAPACITY: a chunk needs more (triangle, tile) entries than it reserved (pgp_depth_cost evaluates such states in
+ *     smaller chunks).
+ * On either error out_dev is not written. */
+PGP_API int pgp_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids,
+                               const double* poses16_dev, float tau, pgp_depth_counts* out_dev, int32_t* status_dev);
 
 #define PGP_MAX_OBJECTS 64
 #define PGP_MAX_CELLS (1ll << 29)

@@ -551,14 +551,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TT, 1) k5_tricp_kern
 // use, released by k5_release (pgp_destroy)
 // The batch (pgp_refine_batch[_dev]) adds: in4 / placed_T (its segments and placed rows converted on the device), flags (K6),
 // keys (the sorts too large for shared memory), the host call's copies of its arguments (raw_*) and results (out), and pinned
-// staging for the one upload of its host-built tables: K5_STAGES buffers used in turn, each reused once its last copy has run.
-constexpr int K5_STAGES = 4;
-struct Staging { void* host = nullptr; size_t cap = 0; cudaEvent_t copied = nullptr; };
+// staging for the one upload of its host-built tables.
 struct TScratch {
   DevBuf seg, d2, nn, T, iters, energy, cell_of, cursor, items;
   DevBuf in4, placed_T, flags, keys, raw_seg, raw_placed, raw_poses, out;
-  Staging stage[K5_STAGES];
-  unsigned next_stage = 0;
+  StagingRing staging;
   bool prep_smem_set = false;
 };
 TScratch& tscratch_of(pgp_ctx* ctx) {
@@ -960,22 +957,10 @@ int k5_refine_batch_dev(pgp_ctx* ctx, bool plane, const float* seg_xyz, const in
     PGP_CUDA(ctx, cudaGetLastError());
   }
   if (n_items == 0) return PGP_OK;
-  // the tables, staged in the next pinned buffer: its previous upload ran long ago unless K5_STAGES calls are still queued.  The
-  // buffers grow together, so that one call of a size readies every later call of that size.
-  if (ts.stage[0].cap < blob) {
-    const size_t cap = blob + blob / 4 + 256;
-    for (Staging& g : ts.stage) {
-      if (!g.copied) PGP_CUDA(ctx, cudaEventCreateWithFlags(&g.copied, cudaEventDisableTiming));
-      PGP_CUDA(ctx, cudaEventSynchronize(g.copied));
-      if (g.host) cudaFreeHost(g.host);
-      g.host = nullptr; g.cap = 0;
-      PGP_CUDA(ctx, cudaMallocHost(&g.host, cap));
-      g.cap = cap;
-    }
-  }
-  Staging& sg = ts.stage[ts.next_stage++ % K5_STAGES];
-  PGP_CUDA(ctx, cudaEventSynchronize(sg.copied));
-  char* h = static_cast<char*>(sg.host);
+  // the tables, staged in the next pinned buffer
+  StagingRing::Stage* sg = nullptr;
+  PGP_CUDA(ctx, ts.staging.acquire(blob, &sg));
+  char* h = static_cast<char*>(sg->host);
   K5Item* desc = reinterpret_cast<K5Item*>(h);
   int* pose_item = reinterpret_cast<int*>(h + o_map);
   int64_t scr = 0;
@@ -992,8 +977,7 @@ int k5_refine_batch_dev(pgp_ctx* ctx, bool plane, const float* seg_xyz, const in
   }
   memcpy(h + o_prep, prep.data(), prep.size() * sizeof(PrepItem));
   if (!jobs.empty()) memcpy(h + o_jobs, jobs.data(), jobs.size() * sizeof(K6Dev));
-  PGP_CUDA(ctx, cudaMemcpyAsync(ts.items.p, sg.host, blob, cudaMemcpyHostToDevice, st));
-  PGP_CUDA(ctx, cudaEventRecord(sg.copied, st));
+  PGP_CUDA(ctx, StagingRing::upload(sg, ts.items.p, blob, st));
   const K5Item* desc_dev = ts.items.as<K5Item>();
   const int* map_dev = reinterpret_cast<const int*>(ts.items.as<char>() + o_map);
   // 2. explained points
@@ -1060,10 +1044,7 @@ void k5_release(pgp_ctx* ctx) {
   for (DevBuf* b : {&ts->seg, &ts->d2, &ts->nn, &ts->T, &ts->iters, &ts->energy, &ts->cell_of, &ts->cursor, &ts->items, &ts->in4, &ts->placed_T,
                     &ts->flags, &ts->keys, &ts->raw_seg, &ts->raw_placed, &ts->raw_poses, &ts->out})
     b->release();
-  for (Staging& sg : ts->stage) {
-    if (sg.host) cudaFreeHost(sg.host);
-    if (sg.copied) cudaEventDestroy(sg.copied);
-  }
+  ts->staging.release();
   delete ts;
   ctx->k5_scratch = nullptr;
 }

@@ -984,11 +984,11 @@ int pgp_set_depth_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uin
   return k8_set_observation(ctx, depth_raw, class_mask, rows, cols, K9, class_pixels_out);
 }
 
-// the checks shared by the two depth calls: objects with meshes, finite poses
+// the checks shared by the depth calls: objects with meshes, finite poses (poses16 nullptr: in device memory, checked there)
 static int check_placed(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int64_t n) {
   for (int64_t i = 0; i < n; ++i)
     if (obj_ids[i] < 0 || obj_ids[i] >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "object id %d out of range", obj_ids[i]);
-  for (int64_t i = 0; i < n * 16; ++i)
+  for (int64_t i = 0; poses16 && i < n * 16; ++i)
     if (!std::isfinite(poses16[i])) return pgp_fail(ctx, PGP_E_INVALID, "pose %lld is not finite", (long long)(i / 16));
   for (int64_t i = 0; i < n; ++i)
     if (!k8_has_mesh(ctx, obj_ids[i])) return pgp_fail(ctx, PGP_E_NO_MODEL, "no mesh in slot %d (pgp_set_mesh)", obj_ids[i]);
@@ -1004,22 +1004,47 @@ int pgp_render_depth(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16
   return rc ? rc : k8_render(ctx, obj_ids, poses16, n, depth_out, slot_out);
 }
 
+// The checks of pgp_depth_cost (host_values: the poses are host memory and their values are checked too) and of pgp_depth_cost_dev
+// (the values are checked on the device); *n_rec: the number of records.
+static int depth_cost_checks(pgp_ctx* ctx, const char* fn, bool host_values, const int64_t* state_offsets, int n_states, const int32_t* obj_ids,
+                             const double* poses16, float tau, const void* out, int64_t* n_rec) {
+  *n_rec = 0;
+  if (!k8_has_observation(ctx)) return pgp_fail(ctx, PGP_E_INVALID, "%s: pgp_set_depth_observation first", fn);
+  if (n_states < 0 || (n_states > 0 && !state_offsets)) return pgp_fail(ctx, PGP_E_INVALID, "%s: bad state list", fn);
+  if (!std::isfinite(tau) || !(tau >= 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "%s: tau must be finite and >= 0", fn);
+  if (n_states == 0) return PGP_OK;
+  if (state_offsets[0] != 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: state_offsets[0] must be 0", fn);
+  for (int s = 0; s < n_states; ++s) {
+    const int64_t k = state_offsets[s + 1] - state_offsets[s];
+    if (k < 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: state_offsets decrease at state %d", fn, s);
+    if (k > PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "%s: state %d places %lld objects (at most %d)", fn, s, (long long)k, PGP_MAX_OBJECTS);
+  }
+  const int64_t n = state_offsets[n_states];
+  if (n > INT32_MAX) return pgp_fail(ctx, PGP_E_INVALID, "%s: more than 2^31 - 1 placed objects", fn);
+  if (n > 0 && (!obj_ids || !poses16 || !out)) return pgp_fail(ctx, PGP_E_INVALID, "%s: null argument", fn);
+  *n_rec = n;
+  return check_placed(ctx, obj_ids, host_values ? poses16 : nullptr, n);
+}
+
 int pgp_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16, float tau,
                    pgp_depth_counts* out) {
   CHECK_CTX(ctx);
-  if (!k8_has_observation(ctx)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: pgp_set_depth_observation first");
-  if (n_states < 0 || (n_states > 0 && !state_offsets)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: bad state list");
-  if (!std::isfinite(tau) || !(tau >= 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: tau must be finite and >= 0");
-  if (n_states == 0) return PGP_OK;
-  if (state_offsets[0] != 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state_offsets[0] must be 0");
-  for (int s = 0; s < n_states; ++s) {
-    const int64_t k = state_offsets[s + 1] - state_offsets[s];
-    if (k < 0) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state_offsets decrease at state %d", s);
-    if (k > PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: state %d places %lld objects (at most %d)", s, (long long)k, PGP_MAX_OBJECTS);
-  }
-  const int64_t n = state_offsets[n_states];
-  if (n > INT32_MAX) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: more than 2^31 - 1 placed objects");
-  if (n > 0 && (!obj_ids || !poses16 || !out)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_depth_cost: null argument");
-  int rc = check_placed(ctx, obj_ids, poses16, n);
+  int64_t n_rec = 0;
+  int rc = depth_cost_checks(ctx, "pgp_depth_cost", true, state_offsets, n_states, obj_ids, poses16, tau, out, &n_rec);
   return rc ? rc : k8_depth_cost(ctx, state_offsets, n_states, obj_ids, poses16, tau, out);
+}
+
+int pgp_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16_dev, float tau,
+                       pgp_depth_counts* out_dev, int32_t* status_dev) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_depth_cost_dev";
+  if (!status_dev) return pgp_fail(ctx, PGP_E_INVALID, "%s: null status_dev", fn);
+  int64_t n_rec = 0;
+  int rc = depth_cost_checks(ctx, fn, false, state_offsets, n_states, obj_ids, poses16_dev, tau, out_dev, &n_rec);
+  if (rc) return rc;
+  const struct { const void* p; bool used; const char* name; } bufs[] = {
+      {status_dev, true, "status_dev"}, {poses16_dev, n_rec > 0, "poses16_dev"}, {out_dev, n_rec > 0, "out_dev"}};
+  for (const auto& b : bufs)
+    if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
+  return k8_depth_cost_dev(ctx, state_offsets, n_states, obj_ids, poses16_dev, tau, out_dev, status_dev);
 }

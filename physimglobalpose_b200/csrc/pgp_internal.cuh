@@ -30,6 +30,47 @@ struct DevBuf {
   template <class T> T* as() const { return static_cast<T*>(p); }
 };
 
+// Pinned staging for the one host -> device upload of a call's host-built tables (K5 and K8 device pipelines): PGP_STAGES buffers
+// used in turn, each reused once its last copy has run, so that a call queues without waiting unless PGP_STAGES calls are still
+// queued.  The buffers grow together, so that one call of a size readies every later call of that size.
+constexpr int PGP_STAGES = 4;
+struct StagingRing {
+  struct Stage { void* host = nullptr; size_t cap = 0; cudaEvent_t copied = nullptr; };
+  Stage stage[PGP_STAGES];
+  unsigned next = 0;
+  // the next buffer, at least `bytes` long and free to be written
+  cudaError_t acquire(size_t bytes, Stage** out) {
+    cudaError_t e = cudaSuccess;
+    if (stage[0].cap < bytes) {
+      const size_t cap = bytes + bytes / 4 + 256;
+      for (Stage& g : stage) {
+        if (!g.copied && (e = cudaEventCreateWithFlags(&g.copied, cudaEventDisableTiming)) != cudaSuccess) return e;
+        if ((e = cudaEventSynchronize(g.copied)) != cudaSuccess) return e;
+        if (g.host) cudaFreeHost(g.host);
+        g.host = nullptr; g.cap = 0;
+        if ((e = cudaMallocHost(&g.host, cap)) != cudaSuccess) return e;
+        g.cap = cap;
+      }
+    }
+    Stage& g = stage[next++ % PGP_STAGES];
+    if ((e = cudaEventSynchronize(g.copied)) != cudaSuccess) return e;
+    *out = &g;
+    return cudaSuccess;
+  }
+  // queues the copy of the buffer's first `bytes` to dev on st, and marks the buffer busy until it has run
+  static cudaError_t upload(Stage* g, void* dev, size_t bytes, cudaStream_t st) {
+    cudaError_t e = cudaMemcpyAsync(dev, g->host, bytes, cudaMemcpyHostToDevice, st);
+    return e != cudaSuccess ? e : cudaEventRecord(g->copied, st);
+  }
+  void release() {
+    for (Stage& g : stage) {
+      if (g.host) cudaFreeHost(g.host);
+      if (g.copied) cudaEventDestroy(g.copied);
+      g = Stage{};
+    }
+  }
+};
+
 // Scene voxel grid ("K1").  Cell edge h = delta * (1 + 2^-8) so that every scene point that can
 // pass the fp32 test d2 <= delta^2 lies in the 27 cells around the query's cell (DESIGN.md).
 // Two empty apron cells on every side: a query in cells 1..dim-2 never indexes out of range.
@@ -310,6 +351,12 @@ int k8_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, const int3
 bool k8_has_mesh(pgp_ctx* ctx, int obj);
 bool k8_has_observation(pgp_ctx* ctx);
 int k8_set_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, const float* K9, int64_t* class_pixels_out);
+// the host forms: the poses up, the device pipeline, the results down, one synchronisation (one more, and a second run, when a
+// chunk's (triangle, tile) pairs exceeded its reservation)
 int k8_render(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n, float* depth_out, int32_t* slot_out);
 int k8_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16, float tau, pgp_depth_counts* out);
+// pgp_depth_cost_dev after its checks: the pipeline queued on ctx->stream; *status_dev = PGP_OK, PGP_E_INVALID (a pose entry not
+// finite) or PGP_E_CAPACITY (a chunk's pairs exceeded its reservation), out_dev written only on PGP_OK
+int k8_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16_dev, float tau,
+                      pgp_depth_counts* out_dev, int32_t* status_dev);
 void k8_release(pgp_ctx* ctx);

@@ -534,6 +534,30 @@ class PoseEngine:
         self._check(self._lib.pgp_depth_cost(self._ctx, _ptr(offs), len(states), _ptr(flat_ids), _ptr(flat_P), float(tau), _ptr(out)))
         return out
 
+    def depth_cost_device(self, states_ids, poses, out, status, tau: float):
+        """pgp_depth_cost_dev: depth_cost on device data, asynchronous on the context's stream (set_stream).
+        Structure, numpy: states_ids, one int array of object ids per state.  Device data, torch CUDA tensors, one row per placed
+        object in state order: poses (n, 4, 4) or (n, 16) f64; out (n, 5) i32 {rendered, agree, in_front, behind, on_segment},
+        written once the work has run with status PGP_OK; status (1,) i32: PGP_OK, PGP_E_INVALID (a pose entry is not finite) or
+        PGP_E_CAPACITY (a chunk needed more (triangle, tile) entries than it reserved; depth_cost evaluates such states).  The
+        tensors are kept alive until the next call."""
+        import torch
+        want = {"poses": (poses, torch.float64), "out": (out, torch.int32), "status": (status, torch.int32)}
+        for name, (t, dt) in want.items():
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of {dt}")
+        ids = [np.asarray(i, np.int32).reshape(-1) for i in states_ids]
+        offs = np.zeros(len(ids) + 1, np.int64)
+        offs[1:] = np.cumsum([len(i) for i in ids])
+        n = int(offs[-1])
+        if poses.numel() != 16 * n or out.numel() != 5 * n or status.numel() != 1:
+            raise ValueError(f"{n} placed objects: poses needs {n} x 16 entries, out {n} x 5, status 1")
+        flat_ids = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32), np.int32)
+        self._keep["depth_cost"] = (poses, out, status)
+        dp = lambda t: None if t.numel() == 0 else t.data_ptr()   # noqa: E731
+        self._check(self._lib.pgp_depth_cost_dev(self._ctx, _ptr(offs), len(ids), _ptr(flat_ids), dp(poses), float(tau), dp(out),
+                                                 status.data_ptr()))
+
 
 class PoseGroup:
     """One process, n GPUs (pgp_group_*): replicated scene / models, bases or hypotheses sharded over the devices, NCCL
