@@ -576,6 +576,32 @@ PGP_API int pgp_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_sta
 PGP_API int pgp_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids,
                                const double* poses16_dev, float tau, pgp_depth_counts* out_dev, int32_t* status_dev);
 
+/* n_states states in CSR form, as pgp_depth_cost_dev, rendered into device memory on the context's stream: the form for a caller that
+ * composes its own per-pixel cost on the GPU from the rendered frames.  depth_dev: n_states x rows x cols fp32 metres, state s at
+ * offset s x rows x cols (0 = nothing); slot_dev: the same layout in int32 (-1 = nothing), or NULL.  Frame s is bitwise
+ * pgp_render_depth of state s alone; an empty state gives an empty frame.  Offsets are 64-bit: n_states x rows x cols may exceed 2^31.
+ *
+ * Structure, asynchrony, device memory and refusals are those of pgp_depth_cost_dev (tau aside): the call is queued and returns,
+ * and once the scratch has grown to the call's size it makes no host synchronisation and no device-to-host copy.  Returned at once,
+ * with nothing queued and every frame untouched: every refusal the host can decide, status_dev == NULL, and a depth_dev, slot_dev,
+ * poses16_dev or status_dev that is not device or managed memory of the context's device.  *status_dev, set afresh by every call
+ * (n_states = 0 included):
+ *   PGP_OK: every frame is written;
+ *   PGP_E_INVALID: a pose entry is NaN or infinite; no frame is written;
+ *   PGP_E_CAPACITY: a chunk needs more (triangle, tile) entries than it reserved; the frames' contents are then unspecified, and
+ *     pgp_render_depth renders those states (it re-cuts the chunks). */
+PGP_API int pgp_render_depth_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids,
+                                 const double* poses16_dev, float* depth_dev, int32_t* slot_dev, int32_t* status_dev);
+
+/* pgp_set_depth_observation on device data (of the context's device, or managed): depth_raw_dev rows x cols uint16 in the stored
+ * encoding, class_mask_dev rows x cols uint8 or NULL, K9 on the host, class_pixels_dev 256 x int64 or NULL (zeroed, then the pixels
+ * of each label with valid depth; all 0 without a mask).  Queued on the context's stream with no host synchronisation: the raw depth
+ * is decoded into the context's frame and the mask copied into the context's buffer, so the caller's buffers are read only by work
+ * ordered at this call, and every call queued after it on the stream sees this observation.  Refusals: those of
+ * pgp_set_depth_observation, and a device argument that is not device or managed memory of the context's device. */
+PGP_API int pgp_set_depth_observation_dev(pgp_ctx* ctx, const uint16_t* depth_raw_dev, const uint8_t* class_mask_dev, int rows,
+                                          int cols, const float* K9, int64_t* class_pixels_dev);
+
 #define PGP_MAX_OBJECTS 64
 #define PGP_MAX_CELLS (1ll << 29)
 

@@ -91,6 +91,8 @@ _SIGNATURES = {
     "pgp_render_depth": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "pgp_depth_cost": (_i, [_vp, _vp, _i, _vp, _vp, _f, _vp]),
     "pgp_depth_cost_dev": (_i, [_vp, _vp, _i, _vp, _vp, _f, _vp, _vp]),
+    "pgp_render_depth_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "pgp_set_depth_observation_dev": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp]),
     # multi-GPU
     "pgp_generate_pcs_range": (_i, [_vp, _i, _vp, C.c_uint64, _i, _i, _i64, _vp]),
     "pgp_topk_begin": (_i, [_vp, _i, _i, _i64]),

@@ -4,8 +4,10 @@
 // and computeCost's formula is not available; K8 follows its own exact contract (include/pgp.h, DESIGN.md 3), restated in numpy
 // in oracle/render_port.py and matched bit for bit.
 //
-// One device pipeline for pgp_depth_cost_dev, pgp_depth_cost and pgp_render_depth, queued on the context's stream with no host stop:
+// One device pipeline for pgp_depth_cost_dev, pgp_render_depth_dev, pgp_depth_cost and pgp_render_depth, queued on the context's
+// stream with no host stop:
 //   k8_ingest  per placed object: pose -> fp32 3x4, finiteness (status PGP_E_INVALID)
+//   k8_clear   render mode: every frame of the call emptied, only when the status is still PGP_OK
 // then per chunk of states, the chunks cut on the host from the mesh sizes alone and queued back to back on the same scratch:
 //   k8_vertex  per (state, slot, vertex): transform, project, snap to 1/256 px
 //   k8_setup   per triangle: cull, orient, pixel bounding box clipped to the image, count its (state, 16x16 tile) bins; the chunk's
@@ -13,12 +15,12 @@
 //   scan -> k8_list (non-empty bins, their number on the device) -> k8_fill (bin lists, when the chunk's pairs fit the entries
 //              reserved for it; otherwise status PGP_E_CAPACITY and the chunk's fill and tiles do nothing)
 //   k8_tiles   a persistent grid that takes the non-empty (state, tile) bins in turn: 64-bit (depth bits, slot) z-buffer in shared
-//              memory with atomicMin, then either the frame written out (pgp_render_depth) or the fused comparison with the
-//              observation, summed per slot in shared memory and added to the state's records.
+//              memory with atomicMin, then either the tile written out to its state's frame (render mode) or the fused comparison
+//              with the observation, summed per slot in shared memory and added to the state's records.
 // and k8_finish copies the counts out when the status is PGP_OK.  The host forms upload, run the pipeline, download and synchronise
 // once; on PGP_E_CAPACITY they re-cut the chunks from the per-state pair counts the device wrote and run again.
-// Work scales with triangles and covered tiles; no per-state frame reaches HBM.  Every count is an integer and every depth is a
-// deterministic function of one triangle and one sample, so results depend neither on scheduling nor on chunking.
+// Work scales with triangles and covered tiles; in the cost mode no per-state frame reaches HBM.  Every count is an integer and every
+// depth is a deterministic function of one triangle and one sample, so results depend neither on scheduling nor on chunking.
 #include <math.h>
 #include <string.h>
 
@@ -74,6 +76,16 @@ __global__ void __launch_bounds__(T) k8_ingest(const double* __restrict__ poses1
     pose16_to_f32x12(P, pose12 + 12 * i);
   }
   if (!ok) *status = PGP_E_INVALID;
+}
+
+// render mode: the call's n frame pixels emptied (depth 0.0f, slot -1: nothing; slot nullptr: no slot frames), queued after k8_ingest
+// so that a call whose poses it refused writes no frame; k8_tiles then writes the pixels of every non-empty tile
+__global__ void __launch_bounds__(T) k8_clear(size_t n, float* __restrict__ depth, int* __restrict__ slot, const int32_t* __restrict__ status) {
+  if (*status != PGP_OK) return;
+  for (size_t i = blockIdx.x * (size_t)T + threadIdx.x; i < n; i += (size_t)gridDim.x * T) {
+    depth[i] = 0.f;
+    if (slot) slot[i] = -1;
+  }
 }
 
 // vertex v0 + i of the call -> {snapped x, snapped y, Z bits, ok} at i
@@ -209,8 +221,9 @@ struct ChunkCounters {
 };
 
 // A persistent grid: each CTA takes the next non-empty bin (list position from counters->next) until none is left, and resets its
-// z-buffer, queue and accumulators per bin.  RENDER: write the frame (one state);  else: compare with the observation and add the
-// per-slot counts to out.  Nothing when the status is not PGP_OK (an earlier refusal, or this chunk's bins did not fit).
+// z-buffer, queue and accumulators per bin.  RENDER: write the tile into frame key / ntiles of depth_out / slot_out (the chunk's
+// first frame; slot_out nullptr: no slot frames);  else: compare with the observation and add the per-slot counts to out.  Nothing
+// when the status is not PGP_OK (an earlier refusal, or this chunk's bins did not fit).
 template <bool RENDER>
 __global__ void __launch_bounds__(TT) k8_tiles(const Tri* __restrict__ tris, const uint32_t* __restrict__ off, const uint32_t* __restrict__ bins,
                                                const uint32_t* __restrict__ list, ChunkCounters* __restrict__ counters, int ntx, int ntiles,
@@ -273,8 +286,9 @@ __global__ void __launch_bounds__(TT) k8_tiles(const Tri* __restrict__ tris, con
     const size_t p = (size_t)mr * obs.cols + mc;
     if (RENDER) {
       if (in_img) {
-        depth_out[p] = k == ~0ull ? 0.f : __uint_as_float((unsigned)(k >> 32));
-        if (slot_out) slot_out[p] = k == ~0ull ? -1 : (int)(unsigned)k;
+        const size_t q = (size_t)(*vkey / (uint32_t)ntiles) * ((size_t)obs.rows * obs.cols) + p;
+        depth_out[q] = k == ~0ull ? 0.f : __uint_as_float((unsigned)(k >> 32));
+        if (slot_out) slot_out[q] = k == ~0ull ? -1 : (int)(unsigned)k;
       }
       continue;
     }
@@ -368,11 +382,13 @@ int cut_chunks(pgp_ctx* ctx, const K8Scratch& sc, const int64_t* offs, int n_sta
 // The device pipeline of one call, queued on ctx->stream (see the top of the file): the records of offs[0 .. n_states] with their
 // poses in device memory (poses16), the given chunks.  *status: PGP_OK, PGP_E_INVALID (a pose entry is not finite; nothing runs)
 // or PGP_E_CAPACITY (a chunk's pairs exceeded its reservation; its fill and tiles and those of every later chunk did nothing).
-// Counts: summed in sc.out, then copied to out_dev when the status is PGP_OK (out_dev nullptr: left in sc.out).  render: the one
-// state's frame to sc.frame_d / sc.frame_s.  Makes no host synchronisation once the scratch has grown to the call's size.
-int run_pipeline(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, int n_states, const int32_t* obj_ids, const double* poses16,
-                 float tau, const std::vector<Chunk>& chunks, int* out_dev, int32_t* status) {
+// Counts: summed in sc.out, then copied to out_dev when the status is PGP_OK (out_dev nullptr: left in sc.out).  Render mode
+// (frame_d not nullptr): state s's frame to frame_d / frame_s + s x rows x cols (frame_s nullptr: no slot frames), and no counts.
+// Makes no host synchronisation once the scratch has grown to the call's size.
+int run_pipeline(pgp_ctx* ctx, K8Scratch& sc, const int64_t* offs, int n_states, const int32_t* obj_ids, const double* poses16, float tau,
+                 const std::vector<Chunk>& chunks, int* out_dev, float* frame_d, int* frame_s, int32_t* status) {
   cudaStream_t st = ctx->stream;
+  const bool render = frame_d != nullptr;
   const int ntx = (sc.cols + TILE - 1) / TILE, ntiles = (int)ntiles_of(sc);
   const int64_t n_rec = n_states > 0 ? offs[n_states] : 0;
   // sizes: every reservation before the first launch (a growing buffer's cudaFree synchronises the device)
@@ -397,25 +413,25 @@ int run_pipeline(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, 
   PGP_CUDA(ctx, sc.bins.reserve((size_t)max_cap * 4));
   PGP_CUDA(ctx, sc.misc.reserve(sizeof(ChunkCounters)));
   PGP_CUDA(ctx, ctx->scene.scratch.reserve((size_t)((max_keys + 1) / 2048 + 4096) * 4));
-  if (render) {
-    PGP_CUDA(ctx, sc.frame_d.reserve(npx * 4));
-    PGP_CUDA(ctx, sc.frame_s.reserve(npx * 4));
-  }
   for (int r = 0; r < 2; ++r)
     if (!sc.tiles_grid[r]) {
       int per_sm = 0;
       PGP_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, r ? k8_tiles<true> : k8_tiles<false>, TT, 0));
       sc.tiles_grid[r] = std::max(per_sm, 1) * ctx->sm_count;
     }
-  // ingest
+  // ingest, then the frames emptied unless a pose was refused
   PGP_CUDA(ctx, cudaMemsetAsync(status, 0, sizeof(int32_t), st));     // PGP_OK
-  if (render) {
-    PGP_CUDA(ctx, cudaMemsetAsync(sc.frame_d.p, 0, npx * 4, st));      // 0.0f: nothing
-    PGP_CUDA(ctx, cudaMemsetAsync(sc.frame_s.p, 0xff, npx * 4, st));   // -1: nothing
+  if (n_rec > 0) {
+    k8_ingest<<<(unsigned)std::min<int64_t>((n_rec + T - 1) / T, 4 * ctx->sm_count), T, 0, st>>>(poses16, n_rec, sc.pose12.as<float>(), status);
+    ctx->launches++;
   }
+  if (render && n_states > 0) {
+    const size_t n = (size_t)n_states * npx;
+    k8_clear<<<(unsigned)std::min<size_t>((n + T - 1) / T, (size_t)8 * ctx->sm_count), T, 0, st>>>(n, frame_d, frame_s, status);
+    ctx->launches++;
+  }
+  PGP_CUDA(ctx, cudaGetLastError());
   if (n_rec == 0) return PGP_OK;
-  k8_ingest<<<(unsigned)std::min<int64_t>((n_rec + T - 1) / T, 4 * ctx->sm_count), T, 0, st>>>(poses16, n_rec, sc.pose12.as<float>(), status);
-  ctx->launches++;
   PGP_CUDA(ctx, cudaMemsetAsync(sc.out.p, 0, (size_t)n_rec * sizeof(pgp_depth_counts), st));
   PGP_CUDA(ctx, cudaMemsetAsync(sc.state_pairs.p, 0, (size_t)n_states * 8, st));
   // the tables, in one copy from the next pinned buffer: every record's instance, each state's first record, each record's class
@@ -463,7 +479,8 @@ int run_pipeline(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, 
     const unsigned grid = (unsigned)std::min<int64_t>(sc.tiles_grid[render], n_keys);
     if (render)
       k8_tiles<true><<<grid, TT, 0, st>>>(sc.tris.as<Tri>(), sc.cnt.as<uint32_t>(), sc.bins.as<uint32_t>(), sc.list.as<uint32_t>(), ctr, ntx, ntiles,
-                                          obs, tau, first_dev + c.s, cls_dev, nullptr, sc.frame_d.as<float>(), sc.frame_s.as<int>(), status);
+                                          obs, tau, first_dev + c.s, cls_dev, nullptr, frame_d + (size_t)c.s * npx,
+                                          frame_s ? frame_s + (size_t)c.s * npx : nullptr, status);
     else
       k8_tiles<false><<<grid, TT, 0, st>>>(sc.tris.as<Tri>(), sc.cnt.as<uint32_t>(), sc.bins.as<uint32_t>(), sc.list.as<uint32_t>(), ctr, ntx, ntiles,
                                            obs, tau, first_dev + c.s, cls_dev, sc.out.as<int>(), nullptr, nullptr, status);
@@ -482,8 +499,8 @@ int run_pipeline(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, 
 // The host forms: the poses up, the pipeline, the results down (fetch: queues their copies), one synchronisation.  When a chunk's
 // pairs did not fit, the per-state pair counts come back and the pipeline runs again on chunks cut to fit them.
 template <class Fetch>
-int run_host(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, int n_states, const int32_t* obj_ids, const double* poses16, float tau,
-             Fetch fetch) {
+int run_host(pgp_ctx* ctx, K8Scratch& sc, const int64_t* offs, int n_states, const int32_t* obj_ids, const double* poses16, float tau,
+             float* frame_d, int* frame_s, Fetch fetch) {
   cudaStream_t st = ctx->stream;
   const int64_t n_rec = n_states > 0 ? offs[n_states] : 0;
   PGP_CUDA(ctx, sc.raw_poses.reserve((size_t)n_rec * 128));
@@ -493,7 +510,7 @@ int run_host(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, int 
   std::vector<unsigned long long> pairs;
   for (int pass = 0;; ++pass) {
     int rc = cut_chunks(ctx, sc, offs, n_states, obj_ids, pass ? pairs.data() : nullptr, chunks);
-    if (!rc) rc = run_pipeline(ctx, sc, render, offs, n_states, obj_ids, sc.raw_poses.as<double>(), tau, chunks, nullptr, sc.status.as<int32_t>());
+    if (!rc) rc = run_pipeline(ctx, sc, offs, n_states, obj_ids, sc.raw_poses.as<double>(), tau, chunks, nullptr, frame_d, frame_s, sc.status.as<int32_t>());
     if (rc) return rc;
     int32_t status = PGP_OK;
     PGP_CUDA(ctx, cudaMemcpyAsync(&status, sc.status.p, sizeof(status), cudaMemcpyDeviceToHost, st));
@@ -505,6 +522,14 @@ int run_host(pgp_ctx* ctx, K8Scratch& sc, bool render, const int64_t* offs, int 
     PGP_CUDA(ctx, cudaMemcpyAsync(pairs.data(), sc.state_pairs.p, (size_t)n_states * 8, cudaMemcpyDeviceToHost, st));
     PGP_CUDA(ctx, cudaStreamSynchronize(st));
   }
+}
+
+// the observation's frame size, intrinsics and mask flag, once its decode and mask are queued
+void observed(K8Scratch& sc, int rows, int cols, const float* K9, bool has_mask) {
+  sc.rows = rows; sc.cols = cols;
+  sc.fx = K9[0]; sc.fy = K9[4]; sc.cx = K9[2]; sc.cy = K9[5];
+  sc.has_mask = has_mask;
+  sc.has_obs = true;
 }
 
 }  // namespace
@@ -551,10 +576,31 @@ int k8_set_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* c
   if (hist_wanted) PGP_CUDA(ctx, cudaMemcpyAsync(hist, sc.misc.p, sizeof(hist), cudaMemcpyDeviceToHost, st));
   PGP_CUDA(ctx, cudaStreamSynchronize(st));
   if (class_pixels_out) for (int i = 0; i < 256; ++i) class_pixels_out[i] = (int64_t)hist[i];
-  sc.rows = rows; sc.cols = cols;
-  sc.fx = K9[0]; sc.fy = K9[4]; sc.cx = K9[2]; sc.cy = K9[5];
-  sc.has_mask = class_mask != nullptr;
-  sc.has_obs = true;
+  observed(sc, rows, cols, K9, class_mask != nullptr);
+  return PGP_OK;
+}
+
+// k8_set_observation on device data, queued on ctx->stream with no synchronisation: the caller's raw depth decoded straight into the
+// context's frame and its mask copied into the context's buffer (later calls read them), so the caller's buffers are read only by
+// work ordered at this call.  A call queued earlier on the stream still reads the observation it was queued with.
+int k8_set_observation_dev(pgp_ctx* ctx, const uint16_t* depth_raw_dev, const uint8_t* class_mask_dev, int rows, int cols, const float* K9,
+                           int64_t* class_pixels_dev) {
+  K8Scratch& sc = k8_scratch_of(ctx);
+  cudaStream_t st = ctx->stream;
+  const int npx = rows * cols;
+  unsigned long long* hist = reinterpret_cast<unsigned long long*>(class_pixels_dev);
+  sc.has_obs = false;
+  PGP_CUDA(ctx, sc.depth.reserve((size_t)npx * 4));
+  if (class_mask_dev) {
+    PGP_CUDA(ctx, sc.mask.reserve((size_t)npx));
+    PGP_CUDA(ctx, cudaMemcpyAsync(sc.mask.p, class_mask_dev, (size_t)npx, cudaMemcpyDeviceToDevice, st));
+  }
+  if (hist) PGP_CUDA(ctx, cudaMemsetAsync(hist, 0, 256 * 8, st));
+  k8_observe<<<std::min((npx + T - 1) / T, ctx->sm_count * 4), T, 0, st>>>(depth_raw_dev, sc.mask.as<uint8_t>(), npx, sc.depth.as<float>(),
+                                                                           class_mask_dev ? hist : nullptr);
+  ctx->launches++;
+  PGP_CUDA(ctx, cudaGetLastError());
+  observed(sc, rows, cols, K9, class_mask_dev != nullptr);
   return PGP_OK;
 }
 
@@ -563,7 +609,9 @@ int k8_render(pgp_ctx* ctx, const int32_t* obj_ids, const double* poses16, int n
   cudaStream_t st = ctx->stream;
   const size_t npx = (size_t)sc.rows * sc.cols;
   const int64_t offs[2] = {0, n};
-  return run_host(ctx, sc, true, offs, 1, obj_ids, poses16, 0.f, [&]() {
+  PGP_CUDA(ctx, sc.frame_d.reserve(npx * 4));
+  PGP_CUDA(ctx, sc.frame_s.reserve(npx * 4));
+  return run_host(ctx, sc, offs, 1, obj_ids, poses16, 0.f, sc.frame_d.as<float>(), sc.frame_s.as<int>(), [&]() {
     cudaError_t e = cudaMemcpyAsync(depth_out, sc.frame_d.p, npx * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess && slot_out) e = cudaMemcpyAsync(slot_out, sc.frame_s.p, npx * 4, cudaMemcpyDeviceToHost, st);
     return e;
@@ -575,7 +623,7 @@ int k8_depth_cost(pgp_ctx* ctx, const int64_t* offs, int n_states, const int32_t
   const int64_t n_rec = n_states > 0 ? offs[n_states] : 0;
   if (n_rec == 0) return PGP_OK;
   std::vector<pgp_depth_counts> counts((size_t)n_rec);         // out is written only once the status is PGP_OK
-  int rc = run_host(ctx, sc, false, offs, n_states, obj_ids, poses16, tau, [&]() {
+  int rc = run_host(ctx, sc, offs, n_states, obj_ids, poses16, tau, nullptr, nullptr, [&]() {
     return cudaMemcpyAsync(counts.data(), sc.out.p, (size_t)n_rec * sizeof(pgp_depth_counts), cudaMemcpyDeviceToHost, ctx->stream);
   });
   if (rc) return rc;
@@ -588,7 +636,16 @@ int k8_depth_cost_dev(pgp_ctx* ctx, const int64_t* offs, int n_states, const int
   K8Scratch& sc = k8_scratch_of(ctx);
   std::vector<Chunk> chunks;
   int rc = cut_chunks(ctx, sc, offs, n_states, obj_ids, nullptr, chunks);
-  return rc ? rc : run_pipeline(ctx, sc, false, offs, n_states, obj_ids, poses16_dev, tau, chunks, reinterpret_cast<int*>(out_dev), status_dev);
+  return rc ? rc : run_pipeline(ctx, sc, offs, n_states, obj_ids, poses16_dev, tau, chunks, reinterpret_cast<int*>(out_dev), nullptr, nullptr,
+                                status_dev);
+}
+
+int k8_render_dev(pgp_ctx* ctx, const int64_t* offs, int n_states, const int32_t* obj_ids, const double* poses16_dev, float* depth_dev,
+                  int32_t* slot_dev, int32_t* status_dev) {
+  K8Scratch& sc = k8_scratch_of(ctx);
+  std::vector<Chunk> chunks;
+  int rc = cut_chunks(ctx, sc, offs, n_states, obj_ids, nullptr, chunks);
+  return rc ? rc : run_pipeline(ctx, sc, offs, n_states, obj_ids, poses16_dev, 0.f, chunks, nullptr, depth_dev, slot_dev, status_dev);
 }
 
 void k8_release(pgp_ctx* ctx) {

@@ -973,15 +973,21 @@ int pgp_set_mesh(pgp_ctx* ctx, int obj, const float* vert_xyz, int nv, const int
   return k8_set_mesh(ctx, obj, vert_xyz, nv, tri3, nt, class_id);
 }
 
+// the checks of both observation forms: frame size and intrinsics
+static int observation_checks(pgp_ctx* ctx, const char* fn, const void* depth_raw, int rows, int cols, const float* K9) {
+  if (!depth_raw || !K9 || rows < 1 || cols < 1 || rows > K8_MAX_SIDE || cols > K8_MAX_SIDE)
+    return pgp_fail(ctx, PGP_E_INVALID, "%s: need a depth frame of 1 .. %d px per side and K9", fn, K8_MAX_SIDE);
+  for (int i = 0; i < 9; ++i)
+    if (!std::isfinite(K9[i])) return pgp_fail(ctx, PGP_E_INVALID, "%s: K[%d] is not finite", fn, i);
+  if (!(K9[0] > 0.f) || !(K9[4] > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "%s: fx and fy must be > 0", fn);
+  return PGP_OK;
+}
+
 int pgp_set_depth_observation(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, const float* K9,
                               int64_t* class_pixels_out) {
   CHECK_CTX(ctx);
-  if (!depth_raw || !K9 || rows < 1 || cols < 1 || rows > K8_MAX_SIDE || cols > K8_MAX_SIDE)
-    return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: need a depth frame of 1 .. %d px per side and K9", K8_MAX_SIDE);
-  for (int i = 0; i < 9; ++i)
-    if (!std::isfinite(K9[i])) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: K[%d] is not finite", i);
-  if (!(K9[0] > 0.f) || !(K9[4] > 0.f)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_depth_observation: fx and fy must be > 0");
-  return k8_set_observation(ctx, depth_raw, class_mask, rows, cols, K9, class_pixels_out);
+  int rc = observation_checks(ctx, "pgp_set_depth_observation", depth_raw, rows, cols, K9);
+  return rc ? rc : k8_set_observation(ctx, depth_raw, class_mask, rows, cols, K9, class_pixels_out);
 }
 
 // the checks shared by the depth calls: objects with meshes, finite poses (poses16 nullptr: in device memory, checked there)
@@ -1047,4 +1053,34 @@ int pgp_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states,
   for (const auto& b : bufs)
     if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
   return k8_depth_cost_dev(ctx, state_offsets, n_states, obj_ids, poses16_dev, tau, out_dev, status_dev);
+}
+
+int pgp_render_depth_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16_dev,
+                         float* depth_dev, int32_t* slot_dev, int32_t* status_dev) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_render_depth_dev";
+  if (!status_dev) return pgp_fail(ctx, PGP_E_INVALID, "%s: null status_dev", fn);
+  int64_t n_rec = 0;
+  int rc = depth_cost_checks(ctx, fn, false, state_offsets, n_states, obj_ids, poses16_dev, 0.f, depth_dev, &n_rec);
+  if (rc) return rc;
+  const struct { const void* p; bool used; const char* name; } bufs[] = {
+      {status_dev, true, "status_dev"}, {poses16_dev, n_rec > 0, "poses16_dev"}, {depth_dev, n_states > 0, "depth_dev"},
+      {slot_dev, n_states > 0 && slot_dev != nullptr, "slot_dev"}};
+  for (const auto& b : bufs)
+    if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
+  return k8_render_dev(ctx, state_offsets, n_states, obj_ids, poses16_dev, depth_dev, slot_dev, status_dev);
+}
+
+int pgp_set_depth_observation_dev(pgp_ctx* ctx, const uint16_t* depth_raw_dev, const uint8_t* class_mask_dev, int rows, int cols, const float* K9,
+                                  int64_t* class_pixels_dev) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_set_depth_observation_dev";
+  int rc = observation_checks(ctx, fn, depth_raw_dev, rows, cols, K9);
+  if (rc) return rc;
+  const struct { const void* p; bool used; const char* name; } bufs[] = {
+      {depth_raw_dev, true, "depth_raw_dev"}, {class_mask_dev, class_mask_dev != nullptr, "class_mask_dev"},
+      {class_pixels_dev, class_pixels_dev != nullptr, "class_pixels_dev"}};
+  for (const auto& b : bufs)
+    if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
+  return k8_set_observation_dev(ctx, depth_raw_dev, class_mask_dev, rows, cols, K9, class_pixels_dev);
 }

@@ -359,4 +359,11 @@ int k8_depth_cost(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, cons
 // finite) or PGP_E_CAPACITY (a chunk's pairs exceeded its reservation), out_dev written only on PGP_OK
 int k8_depth_cost_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16_dev, float tau,
                       pgp_depth_counts* out_dev, int32_t* status_dev);
+// pgp_render_depth_dev after its checks: the same pipeline in render mode, state s's frame to depth_dev / slot_dev + s x rows x cols;
+// the status as k8_depth_cost_dev, the frames cleared and written only while it is PGP_OK
+int k8_render_dev(pgp_ctx* ctx, const int64_t* state_offsets, int n_states, const int32_t* obj_ids, const double* poses16_dev, float* depth_dev,
+                  int32_t* slot_dev, int32_t* status_dev);
+// pgp_set_depth_observation_dev after its checks: decode, mask copy and histogram queued on ctx->stream, no synchronisation
+int k8_set_observation_dev(pgp_ctx* ctx, const uint16_t* depth_raw_dev, const uint8_t* class_mask_dev, int rows, int cols, const float* K9,
+                           int64_t* class_pixels_dev);
 void k8_release(pgp_ctx* ctx);

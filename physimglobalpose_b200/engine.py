@@ -558,6 +558,51 @@ class PoseEngine:
         self._check(self._lib.pgp_depth_cost_dev(self._ctx, _ptr(offs), len(ids), _ptr(flat_ids), dp(poses), float(tau), dp(out),
                                                  status.data_ptr()))
 
+    def render_depth_device(self, states_ids, poses, depth, status, slot=None):
+        """pgp_render_depth_dev: every state rendered into device frames, asynchronous on the context's stream (set_stream).
+        Structure, numpy: states_ids, one int array of object ids per state.  Device data, torch CUDA tensors: poses (n, 4, 4) or
+        (n, 16) f64, one row per placed object in state order; depth (n_states, rows, cols) f32 metres (0 = nothing) and slot
+        (n_states, rows, cols) i32 (-1 = nothing) or None, frame s equal to render_depth of state s; status (1,) i32: PGP_OK,
+        PGP_E_INVALID (a pose entry is not finite; no frame written) or PGP_E_CAPACITY (a chunk needed more (triangle, tile) entries
+        than it reserved; the frames are unspecified and render_depth renders such states).  The tensors are kept alive until the
+        next call."""
+        import torch
+        want = {"poses": (poses, torch.float64), "depth": (depth, torch.float32), "status": (status, torch.int32), "slot": (slot, torch.int32)}
+        for name, (t, dt) in want.items():
+            if (t is not None or name != "slot") and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of {dt}")
+        ids = [np.asarray(i, np.int32).reshape(-1) for i in states_ids]
+        offs = np.zeros(len(ids) + 1, np.int64)
+        offs[1:] = np.cumsum([len(i) for i in ids])
+        n, px = int(offs[-1]), len(ids) * int(np.prod(getattr(self, "_frame", (1, 1))))
+        if poses.numel() != 16 * n or depth.numel() != px or (slot is not None and slot.numel() != px) or status.numel() != 1:
+            raise ValueError(f"{n} placed objects in {len(ids)} states: poses needs {n} x 16 entries, depth and slot {px}, status 1")
+        flat_ids = np.ascontiguousarray(np.concatenate(ids) if ids else np.zeros(0, np.int32), np.int32)
+        self._keep["render_depth"] = (poses, depth, slot, status)
+        dp = lambda t: None if t is None or t.numel() == 0 else t.data_ptr()   # noqa: E731
+        self._check(self._lib.pgp_render_depth_dev(self._ctx, _ptr(offs), len(ids), _ptr(flat_ids), dp(poses), dp(depth), dp(slot),
+                                                   status.data_ptr()))
+
+    def set_depth_observation_device(self, depth_raw, class_mask, K, class_pixels=None):
+        """pgp_set_depth_observation_dev: set_depth_observation on device data, asynchronous on the context's stream (set_stream).
+        Torch CUDA tensors: depth_raw (rows, cols) u16 or i16 (the same bits) as stored; class_mask (rows, cols) u8 or None;
+        class_pixels (256,) i64 or None, the pixels of each label with valid depth once the work has run.  K: 3x3 intrinsics on the
+        host.  Calls queued after this one on the stream see this observation.  The tensors are kept alive until the next call."""
+        import torch
+        if not (isinstance(depth_raw, torch.Tensor) and depth_raw.is_cuda and depth_raw.dtype in (torch.uint16, torch.int16)
+                and depth_raw.is_contiguous() and depth_raw.dim() == 2):
+            raise ValueError("depth_raw must be a contiguous 2-D CUDA tensor of torch.uint16 or torch.int16")
+        want = {"class_mask": (class_mask, torch.uint8, depth_raw.numel()), "class_pixels": (class_pixels, torch.int64, 256)}
+        for name, (t, dt, numel) in want.items():
+            if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() == numel):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of {numel} {dt}")
+        K = _f32(K).reshape(9)
+        self._keep["observation"] = (depth_raw, class_mask, class_pixels)
+        dp = lambda t: None if t is None else t.data_ptr()   # noqa: E731
+        self._check(self._lib.pgp_set_depth_observation_dev(self._ctx, dp(depth_raw), dp(class_mask), depth_raw.shape[0], depth_raw.shape[1],
+                                                            _ptr(K), dp(class_pixels)))
+        self._frame = tuple(depth_raw.shape)
+
 
 class PoseGroup:
     """One process, n GPUs (pgp_group_*): replicated scene / models, bases or hypotheses sharded over the devices, NCCL
