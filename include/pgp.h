@@ -491,7 +491,15 @@ PGP_API int pgp_refine_batch_dev(pgp_ctx* ctx, int metric,
  * PPE/src/hypothesis_generation/ObjectPoseCandidateSet.cpp:28-51).  pgp_set_option("k7_mls", 0) selects plain PCA normals on the
  * un-projected centroids instead (round 1's stand-in).
  * depth_raw: rows x cols uint16 as stored in frame-*.depth.png; class_mask: rows x cols uint8; K9 row-major intrinsics.
- * xyz_out / nrm_out: cap x 3 camera-frame points / unit normals, ready for pgp_set_scene.  Returns the number of points. */
+ * xyz_out / nrm_out: cap x 3 camera-frame points / unit normals, ready for pgp_set_scene.  Returns the number of points.
+ * A centroid q is a neighbour of p when ((dx*dx + dy*dy) + dz*dz) <= r*r, in double from the fp32 coordinates, with r the fp32
+ * radius promoted to double.  A 6x6 polynomial system whose Cholesky pivot falls to 1e-10 of its diagonal or below (neighbours
+ * on one or two lines) is not solved: the point stays on the PCA plane with the plane's normal.
+ * PGP_E_INVALID, before anything runs and with every output untouched: a NULL pointer, rows or cols < 1, rows x cols > 2^30, cap < 0,
+ * a NaN or infinite K9 entry, fx or fy = 0, leaf not finite and > 0, a radius not > 0, a radius above 16 x leaf, or a leaf so
+ * small that a voxel index could exceed 2^30 (coordinates bounded by depth < 2 m over the frame: max(2, 2 |v - cx| / |fx|,
+ * 2 |u - cy| / |fy|) / leaf > 2^30).  PGP_E_TOO_LARGE: the voxel table over the segment's extent needs more than 2.5e8 cells.
+ * PGP_E_CAPACITY: more than cap points survive; xyz_out and nrm_out are then not written. */
 PGP_API int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, int class_id,
                                 const float* K9, float leaf, float normal_radius, float outlier_radius, int min_neighbors,
                                 float* xyz_out, float* nrm_out, int cap, int* n_valid_pixels);

@@ -45,11 +45,25 @@ def voxel_centroids(pts: np.ndarray, leaf: float = 0.01) -> np.ndarray:
     return (np.add.reduceat(pts.astype(np.float64), starts, axis=0) / cnt[:, None]).astype(np.float32)
 
 
-def pca_normals(cen: np.ndarray, radius: float = 0.02) -> np.ndarray:
+def neighbours(cen: np.ndarray, radius: float) -> list:
+    """Per point, the ascending indices of the points q with ((dx*dx + dy*dy) + dz*dz) <= r*r: the kernel's predicate, in double
+    from the fp32 coordinates, each operation rounded, with r the fp32 radius the C ABI receives promoted to double (0.02f, not 0.02).
+    The kd-tree only proposes candidates, within a slightly larger radius; the predicate decides."""
     from scipy.spatial import cKDTree
-    tree = cKDTree(cen)
+    r = float(np.float32(radius))
+    c64 = cen.astype(np.float64)
+    out = []
+    for i, cand in enumerate(cKDTree(cen).query_ball_point(cen, r * (1.0 + 1e-6), return_sorted=True)):
+        cand = np.asarray(cand, np.int64)
+        d = c64[cand] - c64[i]
+        d2 = (d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2]
+        out.append(cand[d2 <= r * r].tolist())
+    return out
+
+
+def pca_normals(cen: np.ndarray, radius: float = 0.02) -> np.ndarray:
     nrm = np.zeros_like(cen)
-    for i, nb in enumerate(tree.query_ball_point(cen, radius)):
+    for i, nb in enumerate(neighbours(cen, radius)):
         q = cen[nb].astype(np.float64)
         if len(nb) >= 3:
             w, vec = np.linalg.eigh(np.cov((q - q.mean(axis=0)).T))
@@ -72,6 +86,42 @@ def _unit_orthogonal(n: np.ndarray) -> np.ndarray:
     return np.array([0.0, -z * inv, y * inv])
 
 
+CHOL6_REL_PIVOT = 1e-10
+
+
+def chol6_solve(A: np.ndarray, b: np.ndarray):
+    """k7_segment.cu::chol6_solve, operation for operation in Python floats (IEEE double, no fused multiply-add): Cholesky of the
+    lower triangle, then the two triangular solves.  None when a pivot is not above CHOL6_REL_PIVOT times its column's diagonal --
+    a system singular up to rounding (neighbours on one or two lines) is not solved, on both sides, whatever the rounding."""
+    n = len(b)
+    L = [[float(A[i][j]) for j in range(n)] for i in range(n)]
+    x = [float(v) for v in b]
+    for j in range(n):
+        d = L[j][j]
+        for k in range(j):
+            d -= L[j][k] * L[j][k]
+        if not (d > CHOL6_REL_PIVOT * L[j][j]):
+            return None
+        d = float(np.sqrt(d))
+        L[j][j] = d
+        for i in range(j + 1, n):
+            v = L[i][j]
+            for k in range(j):
+                v -= L[i][k] * L[j][k]
+            L[i][j] = v / d
+    for i in range(n):
+        v = x[i]
+        for k in range(i):
+            v -= L[i][k] * x[k]
+        x[i] = v / L[i][i]
+    for i in range(n - 1, -1, -1):
+        v = x[i]
+        for k in range(i + 1, n):
+            v -= L[k][i] * x[k]
+        x[i] = v / L[i][i]
+    return np.array(x)
+
+
 def mls_project(cen: np.ndarray, radius: float = 0.02, order: int = 2):
     """pcl::MovingLeastSquares with setPolynomialFit(true), setComputeNormals(true), no upsampling, as the reference configures it
     (PPE/src/segmentation/Segmentation.cpp:231-238): per point, the (unweighted) PCA plane of its neighbours within `radius`, the
@@ -80,16 +130,14 @@ def mls_project(cen: np.ndarray, radius: float = 0.02, order: int = 2):
     normal tilted by its gradient there.  Restated from PCL's published algorithm (mls.hpp, computeMLSPointNormal): PCL is not
     available here, PARITY UNPINNED.  Returns (points, unit normals oriented to the camera at the origin, valid mask): points
     with fewer than 3 neighbours are dropped by PCL (valid = False)."""
-    from scipy.spatial import cKDTree
-    tree = cKDTree(cen)
     n_coef = (order + 1) * (order + 2) // 2
+    r = float(np.float32(radius))                                    # the weights use the fp32 radius, as the kernel does
     out_p = cen.astype(np.float64).copy()
     out_n = np.zeros((len(cen), 3))
     valid = np.zeros(len(cen), dtype=bool)
-    for i, nb in enumerate(tree.query_ball_point(cen, radius)):
+    for i, nb in enumerate(neighbours(cen, radius)):
         if len(nb) < 3:
             continue
-        nb = sorted(nb)
         q = cen[nb].astype(np.float64)
         c = cen[i].astype(np.float64)
         mean = q.mean(axis=0)
@@ -99,20 +147,17 @@ def mls_project(cen: np.ndarray, radius: float = 0.02, order: int = 2):
         normal = n.copy()
         if len(nb) >= n_coef:
             de = q - point
-            wgt = np.exp(-np.einsum("ij,ij->i", de, de) / (radius * radius))
+            wgt = np.exp(-np.einsum("ij,ij->i", de, de) / (r * r))
             v_axis = _unit_orthogonal(n)
             u_axis = np.cross(n, v_axis)
             u, v, f = de @ u_axis, de @ v_axis, de @ n
             P = np.stack([u ** ui * v ** vi for ui in range(order + 1) for vi in range(order + 1 - ui)])     # [1, v, v^2, u, uv, u^2]
             A = (P * wgt) @ P.T
             b = (P * wgt) @ f
-            try:
-                L = np.linalg.cholesky(A)
-                coef = np.linalg.solve(L.T, np.linalg.solve(L, b))
+            coef = chol6_solve(A, b)
+            if coef is not None:
                 point = point + coef[0] * n
                 normal = n - coef[order + 1] * u_axis - coef[1] * v_axis
-            except np.linalg.LinAlgError:
-                pass
         if np.dot(normal, point) > 0:
             normal = -normal
         out_p[i] = point
@@ -122,9 +167,7 @@ def mls_project(cen: np.ndarray, radius: float = 0.02, order: int = 2):
 
 
 def radius_outlier_keep(cen: np.ndarray, radius: float = 0.03, min_neighbors: int = 10) -> np.ndarray:
-    from scipy.spatial import cKDTree
-    tree = cKDTree(cen)
-    return np.array([len(nb) >= min_neighbors for nb in tree.query_ball_point(cen, radius)])       # the point itself counts, as in PCL
+    return np.array([len(nb) >= min_neighbors for nb in neighbours(cen, radius)], dtype=bool)      # the point itself counts, as in PCL
 
 
 def prepare_segment(depth_m, mask, cls, K, leaf=0.01, normal_radius=0.02, outlier_radius=0.03, min_neighbors=10, mls=False):

@@ -21,6 +21,7 @@
 namespace {
 
 constexpr int T = 256;
+constexpr int64_t K7_MAX_CELLS = 250000000;            // dense voxel table: 2.5e8 cells, 1 GB per uint32 array
 
 // pass 1: validity flag per pixel; pass 2 (after the scan): emit points in row-major pixel order
 __global__ void k7_flags(const uint16_t* __restrict__ depth, const uint8_t* __restrict__ mask, int n, int cls, uint32_t* __restrict__ flag) {
@@ -127,12 +128,17 @@ __device__ void unit_orthogonal(const double n[3], double v[3]) {
   }
 }
 
-// A x = b for a symmetric positive definite 6x6 A (lower triangle read), Cholesky in place; false if a pivot is not positive
+// A x = b for a symmetric positive definite 6x6 A (lower triangle read), Cholesky in place.  False if a pivot is not above
+// CHOL6_REL_PIVOT times its column's own diagonal: such a system is singular up to rounding (neighbours on one line or on two lines,
+// as thin strips and mask edges give), and whether its rounding-level pivot comes out positive is an accident of summation order.
+// The threshold makes the decision a property of the geometry, so oracle/segment_port.py::chol6_solve (this function, operation
+// for operation) decides the same.
+constexpr double CHOL6_REL_PIVOT = 1e-10;
 __device__ bool chol6_solve(double A[6][6], double b[6]) {
   for (int j = 0; j < 6; ++j) {
     double d = A[j][j];
     for (int k = 0; k < j; ++k) d -= A[j][k] * A[j][k];
-    if (!(d > 0.0)) return false;
+    if (!(d > CHOL6_REL_PIVOT * A[j][j])) return false;
     d = sqrt(d);
     A[j][j] = d;
     for (int i = j + 1; i < 6; ++i) {
@@ -154,7 +160,8 @@ __device__ bool chol6_solve(double A[6][6], double b[6]) {
 // the plane normal by its value at (0, 0) and the normal tilts by its gradient there; points with fewer than 3 neighbours are
 // dropped (proj.w = 0), as PCL drops them.  Restated from PCL's published algorithm (mls.hpp): PARITY UNPINNED, == oracle/segment_port.py.
 __global__ void k7_normals(const float4* __restrict__ cen, int nc, VoxGrid g, const int* __restrict__ vox_to_cen, double normal_r, double outlier_r,
-                           int min_nb, int mls, float4* __restrict__ nrm, float4* __restrict__ proj, uint32_t* __restrict__ keep) {
+                           int min_nb, int mls, float4* __restrict__ nrm, float4* __restrict__ proj, uint32_t* __restrict__ keep,
+                           float* __restrict__ max_disp) {
   const int i = blockIdx.x * T + threadIdx.x;
   if (i >= nc) return;
   const float4 c = cen[i];
@@ -251,16 +258,25 @@ __global__ void k7_normals(const float4* __restrict__ cen, int nc, VoxGrid g, co
       if (n[0] * pt[0] + n[1] * pt[1] + n[2] * pt[2] > 0) { n[0] = -n[0]; n[1] = -n[1]; n[2] = -n[2]; }
       const double l = sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
       nrm[i] = make_float4((float)(n[0] / l), (float)(n[1] / l), (float)(n[2] / l), 0.f);
-      proj[i] = make_float4((float)pt[0], (float)pt[1], (float)pt[2], 1.f);
+      const float4 out = make_float4((float)pt[0], (float)pt[1], (float)pt[2], 1.f);
+      proj[i] = out;
       keep[i] = cnt_o >= min_nb ? 1u : 0u;                   // (mls: overwritten by k7_outlier_count on the projected cloud)
+      if (mls) {                                             // |proj - cen| of the stored floats, rounded up: k7_outlier_count's window
+        const double ex = (double)out.x - (double)c.x, ey = (double)out.y - (double)c.y, ez = (double)out.z - (double)c.z;
+        const float disp = __double2float_ru(sqrt(ex * ex + ey * ey + ez * ez));
+        atomicMax(reinterpret_cast<int*>(max_disp), __float_as_int(disp));      // non-negative floats order as their bits
+      }
     }
   }
 }
 
-// mls = 1: the radius-outlier filter runs on the PROJECTED cloud (ObjectPoseCandidateSet.cpp:28-32 filters what MLS returned).  A
-// projected point lies within `slack` voxels of its centroid's voxel (checked: the displacement is bounded by the fit's radius).
+// mls = 1: the radius-outlier filter runs on the PROJECTED cloud (ObjectPoseCandidateSet.cpp:28-32 filters what MLS returned), but
+// the voxel table holds the centroids.  Two projected points within outlier_r have centroids within outlier_r + 2 * max_disp (the
+// largest |proj - cen| of the call, recorded by k7_normals), so a window of ceil((outlier_r + 2 * max_disp) / leaf) + 1 voxels
+// around the centroid's voxel holds every neighbour; the + 1 absorbs the rounding of the voxel indices.  The displacement is not
+// bounded by normal_r (the polynomial's value at the origin is not), hence the measured bound.  Clamped to the table.
 __global__ void k7_outlier_count(const float4* __restrict__ cen, const float4* __restrict__ proj, int nc, VoxGrid g, const int* __restrict__ vox_to_cen,
-                                 double outlier_r, int min_nb, uint32_t* __restrict__ keep) {
+                                 double outlier_r, int min_nb, const float* __restrict__ max_disp, uint32_t* __restrict__ keep) {
   const int i = blockIdx.x * T + threadIdx.x;
   if (i >= nc) return;
   const float4 me = proj[i];
@@ -268,7 +284,9 @@ __global__ void k7_outlier_count(const float4* __restrict__ cen, const float4* _
   const float4 c = cen[i];
   const int ci = (int)floorf(__fdiv_rn(c.x, g.leaf)) - g.mn[0], cj = (int)floorf(__fdiv_rn(c.y, g.leaf)) - g.mn[1],
             ck = (int)floorf(__fdiv_rn(c.z, g.leaf)) - g.mn[2];
-  const int R = (int)ceil(outlier_r / (double)g.leaf) + 5;           // + 2 x 2 voxels: both points may have moved by up to normal_r
+  const int span = max(g.dim[0], max(g.dim[1], g.dim[2]));
+  const double Rd = ceil((outlier_r + 2.0 * (double)*max_disp) / (double)g.leaf) + 1.0;
+  const int R = Rd < (double)span ? (int)Rd : span;
   const double or2 = outlier_r * outlier_r;
   int cnt = 0;
   for (int dk = -R; dk <= R; ++dk) {
@@ -301,7 +319,7 @@ __global__ void k7_keep(const float4* __restrict__ cen, const float4* __restrict
 }
 
 // device scratch of the segment preparation: owned by the context (k7_release)
-struct K7Scratch { DevBuf depth, mask, flag, pts, key_of, cnt, cursor, sorted, occ, cen, vox_to_cen, nrm, proj, keep, xyz, nxyz; };
+struct K7Scratch { DevBuf depth, mask, flag, pts, key_of, cnt, cursor, sorted, occ, cen, vox_to_cen, nrm, proj, keep, xyz, nxyz, max_disp; };
 K7Scratch& k7_scratch_of(pgp_ctx* ctx) {
   if (!ctx->k7_scratch) ctx->k7_scratch = new K7Scratch();
   return *static_cast<K7Scratch*>(ctx->k7_scratch);
@@ -349,12 +367,22 @@ int k7_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_host, const uint8_t* 
   int mm[6];
   PGP_CUDA(ctx, cudaMemcpyAsync(mm, d_mm, sizeof(mm), cudaMemcpyDeviceToHost, st));
   PGP_CUDA(ctx, cudaStreamSynchronize(st));
+  // the index span in int64: max - min + 1 of two ints can exceed INT_MAX (the leaf refusal of pgp_prepare_segment keeps every index
+  // within +-2^30, this keeps the table size honest regardless); each factor is checked before the next multiplication, so the
+  // product never exceeds 2.5e8 * 2^32
   VoxGrid g{};
   g.leaf = leaf;
-  double cells = 1;
-  for (int k = 0; k < 3; ++k) { g.mn[k] = mm[k]; g.dim[k] = mm[3 + k] - mm[k] + 1; cells *= g.dim[k]; }
-  if (cells > 2.5e8) return pgp_fail(ctx, PGP_E_TOO_LARGE, "segment voxel table needs %.3g cells", cells);
-  const int n_vox = g.dim[0] * g.dim[1] * g.dim[2];
+  int64_t dim[3], cells = 1;
+  for (int k = 0; k < 3; ++k) {
+    g.mn[k] = mm[k];
+    dim[k] = (int64_t)mm[3 + k] - (int64_t)mm[k] + 1;
+    cells *= dim[k];
+    if (cells > K7_MAX_CELLS)
+      return pgp_fail(ctx, PGP_E_TOO_LARGE, "segment voxel table needs more than %lld cells (span %lld x %lld x %lld voxels so far)", (long long)K7_MAX_CELLS,
+                      (long long)dim[0], (long long)(k > 0 ? dim[1] : 1), (long long)(k > 1 ? dim[2] : 1));
+  }
+  for (int k = 0; k < 3; ++k) g.dim[k] = (int)dim[k];
+  const int n_vox = (int)cells;
   PGP_CUDA(ctx, sc.key_of.reserve((size_t)n_raw * 4));
   PGP_CUDA(ctx, sc.cnt.reserve((size_t)(n_vox + 1) * 4));
   PGP_CUDA(ctx, sc.cursor.reserve((size_t)(n_vox + 1) * 4));
@@ -384,12 +412,14 @@ int k7_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_host, const uint8_t* 
   PGP_CUDA(ctx, sc.nxyz.reserve((size_t)nc * 12));
   k7_compact<<<vb, T, 0, st>>>(sc.sorted.as<float4>(), sc.cnt.as<uint32_t>(), sc.occ.as<uint32_t>(), n_vox, sc.cen.as<float4>(), sc.vox_to_cen.as<int>());
   PGP_CUDA(ctx, cudaMemsetAsync(sc.keep.as<uint32_t>() + nc, 0, 4, st));
+  PGP_CUDA(ctx, sc.max_disp.reserve(4));
+  PGP_CUDA(ctx, cudaMemsetAsync(sc.max_disp.p, 0, 4, st));                // +0.0f: the atomicMax identity of non-negative float bits
   k7_normals<<<((int)nc + T - 1) / T, T, 0, st>>>(sc.cen.as<float4>(), (int)nc, g, sc.vox_to_cen.as<int>(), (double)normal_r, (double)outlier_r, min_nb,
-                                                 ctx->k7_mls, sc.nrm.as<float4>(), sc.proj.as<float4>(), sc.keep.as<uint32_t>());
+                                                 ctx->k7_mls, sc.nrm.as<float4>(), sc.proj.as<float4>(), sc.keep.as<uint32_t>(), sc.max_disp.as<float>());
   ctx->launches += 2;
   if (ctx->k7_mls) {
     k7_outlier_count<<<((int)nc + T - 1) / T, T, 0, st>>>(sc.cen.as<float4>(), sc.proj.as<float4>(), (int)nc, g, sc.vox_to_cen.as<int>(), (double)outlier_r, min_nb,
-                                                         sc.keep.as<uint32_t>());
+                                                         sc.max_disp.as<float>(), sc.keep.as<uint32_t>());
     ctx->launches++;
   }
   uint32_t n_keep = 0;
@@ -412,7 +442,7 @@ void k7_release(pgp_ctx* ctx) {
   if (!ctx->k7_scratch) return;
   K7Scratch* sc = static_cast<K7Scratch*>(ctx->k7_scratch);
   for (DevBuf* b : {&sc->depth, &sc->mask, &sc->flag, &sc->pts, &sc->key_of, &sc->cnt, &sc->cursor, &sc->sorted, &sc->occ, &sc->cen, &sc->vox_to_cen, &sc->nrm,
-                    &sc->proj, &sc->keep, &sc->xyz, &sc->nxyz})
+                    &sc->proj, &sc->keep, &sc->xyz, &sc->nxyz, &sc->max_disp})
     b->release();
   delete sc;
   ctx->k7_scratch = nullptr;

@@ -941,16 +941,28 @@ int pgp_refine_batch_dev(pgp_ctx* ctx, int metric, const float* seg_xyz_dev, con
                              poses16_dev, threshold, trim, ratio, max_iter, iters_dev, energy_dev, n_unexplained_dev, status_dev);
 }
 
+#define K7_MAX_PIXELS (1ll << 30)   // rows x cols: every pixel index, scan length and grid size of K7 stays far from INT_MAX
+
 int pgp_prepare_segment(pgp_ctx* ctx, const uint16_t* depth_raw, const uint8_t* class_mask, int rows, int cols, int class_id, const float* K9,
                         float leaf, float normal_radius, float outlier_radius, int min_neighbors, float* xyz_out, float* nrm_out, int cap,
                         int* n_valid_pixels) {
   CHECK_CTX(ctx);
   if (!depth_raw || !class_mask || rows <= 0 || cols <= 0 || !K9 || !xyz_out || !nrm_out || cap < 0)
     return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: bad argument");
-  if (!(leaf > 0.f) || !(normal_radius > 0.f) || !(outlier_radius > 0.f) || !(K9[0] != 0.f) || !(K9[4] != 0.f))
-    return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: leaf, radii and focal lengths must be non-zero");
+  if ((int64_t)rows * cols > K7_MAX_PIXELS)
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: %d x %d pixels, at most %lld", rows, cols, (long long)K7_MAX_PIXELS);
+  for (int i = 0; i < 9; ++i)
+    if (!std::isfinite(K9[i])) return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: K[%d] is not finite", i);
+  if (!(leaf > 0.f) || !std::isfinite(leaf) || !(normal_radius > 0.f) || !(outlier_radius > 0.f) || !(K9[0] != 0.f) || !(K9[4] != 0.f))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: leaf must be finite and > 0, radii > 0, focal lengths non-zero");
   if ((double)normal_radius / leaf > 16.0 || (double)outlier_radius / leaf > 16.0)
     return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: radius / leaf > 16");
+  // voxel indices floor(coordinate / leaf) are ints: bound |coordinate| over the frame (valid depth < 2 m) and keep every index
+  // within 2^30, so that an index span max - min + 1 stays representable
+  const double du = std::max(std::fabs((double)K9[2]), std::fabs((double)(cols - 1) - K9[2])), dv = std::max(std::fabs((double)K9[5]), std::fabs((double)(rows - 1) - K9[5]));
+  const double coord = std::max(2.0, 2.0 * std::max(du / std::fabs((double)K9[0]), dv / std::fabs((double)K9[4])));
+  if (coord / leaf > 1073741824.0)
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_prepare_segment: leaf %g too small for coordinates up to %g m (index above 2^30)", (double)leaf, coord);
   int n = 0;
   int rc = k7_prepare_segment(ctx, depth_raw, class_mask, rows, cols, class_id, K9, leaf, normal_radius, outlier_radius, min_neighbors, xyz_out, nrm_out,
                               cap, &n, n_valid_pixels);
