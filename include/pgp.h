@@ -203,6 +203,59 @@ PGP_API int pgp_topk_merge(const pgp_hyp* lists, int n_lists, int k_each, int k,
  * ranks' batches in rank order (each rank may contribute at most PGP_CHAIN_EXCHANGE_CAP elements). */
 PGP_API int pgp_improving_chain(pgp_ctx* ctx, int obj, int64_t index_base, pgp_hyp* out_host, int cap);
 
+/* ---------------------------------------------------------------- K4d: pose-distinct candidates */
+
+/* Greedy non-maximum suppression in pose space: which hypotheses of an object become MCTS candidates when many of the best ones
+ * are the same placement with millimetre and sub-degree jitter (congruent sets of different bases agree, LCP is smooth in the
+ * pose).  No live reference counterpart: the reference's pose-space clustering (greedyClustering) is commented out
+ * (PPE/src/hypothesis_generation/HypothesisSelection.cpp:161) and its only CUDA kernel is a box NMS.  RESTATED, exact contract
+ * (oracle/select_port.py restates it in float64):
+ *
+ *  Pool: m records (pgp_hyp) of one object, 1 <= m <= 4096, processed in the order given (pgp_topk's order is what callers pass).
+ *    Records with index < 0 (pgp_topk_dev's padding) are skipped: they neither keep nor suppress.
+ *  Greedy rule: record i is kept iff no earlier KEPT record suppresses it; the walk stops once k records are kept.  Kept records
+ *    keep their pool order and are copied bit for bit.
+ *  A kept record a suppresses a later record b when both tests pass, every step in double from the fp32 entries of the centred
+ *  row-major 3x4 T, each operation rounded on its own (no FMA):
+ *    translation: dx = (double)a.T[3] - (double)b.T[3], dy (entries 7), dz (entries 11); d2 = (dx*dx + dy*dy) + dz*dz;
+ *      passes when d2 <= max_dist * max_dist (one rounded product).  In the centred frame this is the distance between the
+ *      points where the model's search centroid lands.
+ *    rotation: for S in {I} and the object's symmetries, G = R_b S entry by entry ((R_b[r][0] S[0][c] + R_b[r][1] S[1][c]) +
+ *      R_b[r][2] S[2][c]) (for S = I, G = R_b promoted to double; the identity is not multiplied in); tr = sum R_a[r][c] G[r][c]
+ *      left to right in row-major order; passes when tr >= 1.0 + 2.0 * cos_angle for some S.
+ *  NaN follows the IEEE comparisons: a record with a NaN entry in T never suppresses and is never suppressed (it is kept when
+ *  reached, and suppresses nothing).
+ *  Camera-frame output row j = pgp_centred_to_pose(obj, kept[j].T), bitwise (same double expression and order). */
+#define PGP_MAX_SYMMETRIES 23
+/* Discrete symmetries of model slot obj: n row-major 3x3 rotations R9 (n x 9 doubles) in the centred model frame; the identity is
+ * implied.  n = 0 clears the set.  A property of the model, like pgp_set_mesh: pgp_set_model leaves it alone.  The matrices need not
+ * be orthonormal (the contract is the arithmetic above).  PGP_E_INVALID: obj out of range, n < 0 or n > PGP_MAX_SYMMETRIES, a
+ * NULL R9 with n > 0, a non-finite entry. */
+PGP_API int pgp_set_symmetries(pgp_ctx* ctx, int obj, const double* R9, int n);
+/* Many pools at once on device data, asynchronous on the context's stream, in two launches whatever n_lists is.  On the host:
+ * objs (n_lists model slots), pool_offsets (n_lists + 1, non-decreasing from 0, each list 1 .. 4096 records) and k (1 .. 4096), so
+ * every launch size is known and nothing is read back.  In device memory (of the context's device, or managed):
+ *   pool_dev  the concatenated pools (pool_offsets[n_lists] records);
+ *   out_dev   n_lists x k records: list l's kept records at l x k, the slots after them index = -1 and zero elsewhere (as pgp_topk_dev pads);
+ *   poses16_dev (NULL allowed) n_lists x k row-major 4x4 doubles, the kept records' camera-frame poses, the rows after them the
+ *     identity: with pose_offsets = {0, k, 2k, ...} they go straight to pgp_refine_batch_dev (a padding row is finite, refines to
+ *     something finite and is ignored by its record's index);
+ *   n_kept_dev (NULL allowed) one int32 per list.
+ * The call returns once the work is queued; once the context's scratch has grown to the call's size (one 2 MB suppression mask per
+ * 4096-pool) it makes no host synchronisation.  Returned at once with nothing queued and every output untouched: n_lists < 0, bad
+ * offsets or list sizes, k outside 1 .. 4096, max_dist not finite or < 0, cos_angle NaN, a NULL objs / pool_dev / out_dev with
+ * lists, an obj out of range (PGP_E_INVALID) or without a model (PGP_E_NO_MODEL), no scene when poses16_dev is requested
+ * (PGP_E_NO_SCENE), a device argument that is not device or managed memory of the context's device.  No value is refused on the
+ * device (there is no status word).  n_lists = 0 is a no-op. */
+PGP_API int pgp_distinct_dev(pgp_ctx* ctx, const int32_t* objs, const int64_t* pool_offsets, int n_lists, const pgp_hyp* pool_dev, int k,
+                             double max_dist, double cos_angle, pgp_hyp* out_dev, double* poses16_dev, int32_t* n_kept_dev);
+/* The host convenience: the pool is pgp_topk(obj, m, PGP_INDEX_AUTO), K4d runs on it, out_host (room for k records) receives the
+ * kept ones; returns their number.  On a communicator context the call is COLLECTIVE because pgp_topk is: every rank selects from
+ * the same merged pool, so the answer does not depend on the number of GPUs (greedy suppression over the global top m depends on
+ * that list alone).  PGP_E_INVALID: m or k outside 1 .. 4096, max_dist not finite or < 0, cos_angle NaN, out_host NULL; the
+ * refusals of pgp_topk. */
+PGP_API int pgp_topk_distinct(pgp_ctx* ctx, int obj, int m, int k, double max_dist, double cos_angle, pgp_hyp* out_host);
+
 /* ---------------------------------------------------------------- K2: PCS generation ------- */
 
 PGP_API void pgp_pcs_default_opts(pgp_pcs_opts* o);
@@ -324,6 +377,10 @@ PGP_API int pgp_group_score_lcp(pgp_group* g, int obj, const float* T_host, int6
 /* K4 on every device -> one grouped ncclAllGather -> merge: the global answers, independent of the device count */
 PGP_API int pgp_group_topk(pgp_group* g, int obj, int k, pgp_hyp* out_host);
 PGP_API int pgp_group_improving_chain(pgp_group* g, int obj, pgp_hyp* out_host, int cap);
+/* pgp_set_symmetries on every device; pgp_topk_distinct over pgp_group_topk's merged pool (run on device 0): the same answer as one
+ * context on the concatenated batch. */
+PGP_API int pgp_group_set_symmetries(pgp_group* g, int obj, const double* R9, int n);
+PGP_API int pgp_group_topk_distinct(pgp_group* g, int obj, int m, int k, double max_dist, double cos_angle, pgp_hyp* out_host);
 
 /* Random 32-byte-sector gather micro-benchmark (SURVEY.md 8d: the denominator of K3's moved-bytes roofline): every thread chases
  * `loads_per_thread` pseudo-random 32-byte sectors of a `footprint_bytes` buffer (L2-resident when below ~100 MB), four

@@ -65,6 +65,9 @@ _SIGNATURES = {
     "pgp_topk_dev": (_i, [_vp, _i, _i, _i64, _vp]),
     "pgp_topk_merge": (_i, [_vp, _i, _i, _i, _vp]),
     "pgp_improving_chain": (_i, [_vp, _i, _i64, _vp, _i]),
+    "pgp_set_symmetries": (_i, [_vp, _i, _vp, _i]),
+    "pgp_distinct_dev": (_i, [_vp, _vp, _vp, _i, _vp, _i, C.c_double, C.c_double, _vp, _vp, _vp]),
+    "pgp_topk_distinct": (_i, [_vp, _i, _i, _i, C.c_double, C.c_double, _vp]),
     "pgp_pcs_default_opts": (None, [_vp]),
     "pgp_extract_pairs": (_i, [_vp, _i, _f, _f, _vp, _i64, _vp]),
     "pgp_find_quads": (_i, [_vp, _i, _vp, _f, _f, _f, _vp, _i64, _vp, _i64, _vp, _i64, _vp]),
@@ -122,6 +125,8 @@ _SIGNATURES = {
     "pgp_group_score_lcp": (_i, [_vp, _i, _vp, _i64, _i, _vp, _vp]),
     "pgp_group_topk": (_i, [_vp, _i, _i, _vp]),
     "pgp_group_improving_chain": (_i, [_vp, _i, _vp, _i]),
+    "pgp_group_set_symmetries": (_i, [_vp, _i, _vp, _i]),
+    "pgp_group_topk_distinct": (_i, [_vp, _i, _i, _i, C.c_double, C.c_double, _vp]),
     "pgp_bench_sector_gather": (_i, [_vp, _i64, _i, _vp]),
     "pgp_generated_cap_split": (_i, [_vp, _i, _i64, _i, _vp, _vp, _vp]),
     "pgp_host_chain_sum_equal": (C.c_float, [C.c_float, C.c_longlong]),

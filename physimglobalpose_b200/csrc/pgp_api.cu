@@ -126,6 +126,7 @@ void pgp_destroy(pgp_ctx* ctx) {
   k6_release(ctx);
   k7_release(ctx);
   k8_release(ctx);
+  k4d_release(ctx);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   cudaStreamDestroy(ctx->own_stream);
   cudaStreamDestroy(ctx->copy_stream);
@@ -1095,4 +1096,61 @@ int pgp_set_depth_observation_dev(pgp_ctx* ctx, const uint16_t* depth_raw_dev, c
   for (const auto& b : bufs)
     if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
   return k8_set_observation_dev(ctx, depth_raw_dev, class_mask_dev, rows, cols, K9, class_pixels_dev);
+}
+
+// ---------------------------------------------------------------- K4d: pose-distinct candidates
+int pgp_set_symmetries(pgp_ctx* ctx, int obj, const double* R9, int n) {
+  CHECK_CTX(ctx);
+  if (obj < 0 || obj >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_symmetries: object slot %d out of range", obj);
+  if (n < 0 || n > PGP_MAX_SYMMETRIES || (n > 0 && !R9))
+    return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_symmetries: need 0 .. %d matrices (n = %d)", PGP_MAX_SYMMETRIES, n);
+  if (!all_finite(R9, (int64_t)9 * n)) return pgp_fail(ctx, PGP_E_INVALID, "pgp_set_symmetries: a matrix entry is not finite");
+  k4d_set_symmetries(ctx, obj, R9, n);
+  return PGP_OK;
+}
+
+// the value checks shared by the distinct calls
+static int distinct_value_checks(pgp_ctx* ctx, const char* fn, int k, double max_dist, double cos_angle) {
+  if (k < 1 || k > K4_MAX_K) return pgp_fail(ctx, PGP_E_INVALID, "%s: k = %d outside 1 .. %d", fn, k, K4_MAX_K);
+  if (!std::isfinite(max_dist) || !(max_dist >= 0.0)) return pgp_fail(ctx, PGP_E_INVALID, "%s: max_dist must be finite and >= 0", fn);
+  if (std::isnan(cos_angle)) return pgp_fail(ctx, PGP_E_INVALID, "%s: cos_angle is NaN", fn);
+  return PGP_OK;
+}
+
+int pgp_distinct_dev(pgp_ctx* ctx, const int32_t* objs, const int64_t* pool_offsets, int n_lists, const pgp_hyp* pool_dev, int k, double max_dist,
+                     double cos_angle, pgp_hyp* out_dev, double* poses16_dev, int32_t* n_kept_dev) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_distinct_dev";
+  if (n_lists < 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: n_lists < 0", fn);
+  int rc = distinct_value_checks(ctx, fn, k, max_dist, cos_angle);
+  if (rc) return rc;
+  if (n_lists == 0) return PGP_OK;
+  if (!objs || !pool_offsets || !pool_dev || !out_dev) return pgp_fail(ctx, PGP_E_INVALID, "%s: null argument", fn);
+  if (pool_offsets[0] != 0) return pgp_fail(ctx, PGP_E_INVALID, "%s: pool_offsets[0] must be 0", fn);
+  for (int l = 0; l < n_lists; ++l) {
+    const int64_t m = pool_offsets[l + 1] - pool_offsets[l];
+    if (m < 1 || m > K4_MAX_K) return pgp_fail(ctx, PGP_E_INVALID, "%s: list %d has %lld records (1 .. %d)", fn, l, (long long)m, K4_MAX_K);
+    if (objs[l] < 0 || objs[l] >= PGP_MAX_OBJECTS) return pgp_fail(ctx, PGP_E_INVALID, "%s: list %d: object slot %d out of range", fn, l, objs[l]);
+    if (!get_model(ctx, objs[l])) return pgp_fail(ctx, PGP_E_NO_MODEL, "%s: list %d: no model in slot %d", fn, l, objs[l]);
+  }
+  if (poses16_dev && !ctx->scene.ready) return pgp_fail(ctx, PGP_E_NO_SCENE, "%s: camera-frame poses need pgp_set_scene first", fn);
+  const struct { const void* p; bool used; const char* name; } bufs[] = {
+      {pool_dev, true, "pool_dev"}, {out_dev, true, "out_dev"}, {poses16_dev, poses16_dev != nullptr, "poses16_dev"},
+      {n_kept_dev, n_kept_dev != nullptr, "n_kept_dev"}};
+  for (const auto& b : bufs)
+    if (b.used && !on_ctx_device(ctx, b.p)) return pgp_fail(ctx, PGP_E_INVALID, "%s: %s is not device memory of device %d", fn, b.name, ctx->device);
+  return k4d_distinct_dev(ctx, objs, pool_offsets, n_lists, pool_dev, k, max_dist, cos_angle, out_dev, poses16_dev, n_kept_dev);
+}
+
+int pgp_topk_distinct(pgp_ctx* ctx, int obj, int m, int k, double max_dist, double cos_angle, pgp_hyp* out_host) {
+  CHECK_CTX(ctx);
+  const char* fn = "pgp_topk_distinct";
+  if (m < 1 || m > K4_MAX_K) return pgp_fail(ctx, PGP_E_INVALID, "%s: m = %d outside 1 .. %d", fn, m, K4_MAX_K);
+  int rc = distinct_value_checks(ctx, fn, k, max_dist, cos_angle);
+  if (rc) return rc;
+  if (!out_host) return pgp_fail(ctx, PGP_E_INVALID, "%s: null output", fn);
+  std::vector<pgp_hyp> pool((size_t)m);
+  const int n = pgp_topk(ctx, obj, m, PGP_INDEX_AUTO, pool.data());     // collective on a communicator context
+  if (n <= 0) return n;
+  return k4d_distinct_host(ctx, obj, pool.data(), n, k, max_dist, cos_angle, out_host);
 }

@@ -22,6 +22,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -628,6 +629,25 @@ int pgp_group_topk(pgp_group* g, int obj, int k, pgp_hyp* out_host) {
 int pgp_group_improving_chain(pgp_group* g, int obj, pgp_hyp* out_host, int cap) {
   if (!g || !out_host || cap <= 0) return PGP_E_INVALID;
   return group_select(g, obj, PGP_CHAIN_EXCHANGE_CAP, 1, group_index_bases(g, obj), out_host, cap);
+}
+
+int pgp_group_set_symmetries(pgp_group* g, int obj, const double* R9, int n) {
+  if (!g) return PGP_E_INVALID;
+  return group_run(g, [&](int, pgp_ctx* c) { return pgp_set_symmetries(c, obj, R9, n); });
+}
+
+// the merged pool of pgp_group_topk is the same on every device: device 0 selects from it
+int pgp_group_topk_distinct(pgp_group* g, int obj, int m, int k, double max_dist, double cos_angle, pgp_hyp* out_host) {
+  if (!g || !out_host) return PGP_E_INVALID;
+  if (m < 1 || m > K4_MAX_K || k < 1 || k > K4_MAX_K || !std::isfinite(max_dist) || !(max_dist >= 0.0) || std::isnan(cos_angle))
+    return group_fail(g, PGP_E_INVALID, "pgp_group_topk_distinct: m or k outside 1 .. 4096, max_dist not finite and >= 0, or cos_angle NaN");
+  std::vector<pgp_hyp> pool((size_t)m);
+  const int n = pgp_group_topk(g, obj, m, pool.data());
+  if (n <= 0) return n;
+  pgp_ctx* c = g->ctx[0];
+  cudaSetDevice(c->device);
+  const int r = k4d_distinct_host(c, obj, pool.data(), n, k, max_dist, cos_angle, out_host);
+  return r < 0 ? group_fail(g, r, c->err) : r;
 }
 
 }  // extern "C"

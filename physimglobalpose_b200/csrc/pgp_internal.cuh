@@ -225,6 +225,7 @@ struct pgp_ctx {
   void* k6_scratch = nullptr;              // k6_explained.cu (k6_release)
   void* k7_scratch = nullptr;              // k7_segment.cu (k7_release)
   void* k8_scratch = nullptr;              // k8_render.cu: meshes, observation, rasterizer scratch (k8_release)
+  void* k4d_scratch = nullptr;             // k4d_distinct.cu: symmetries, suppression mask, staging (k4d_release)
   int k7_mls = 1;                          // segment preparation: 1 = MLS polynomial projection + normals (what the reference runs), 0 = PCA normals on the centroids
   int stream_upload = 1;  // pgp_score_lcp: overlap the batch upload with the scoring launch (0: upload first; use under profilers)
   int tail_split = 4;     // K3 fine kernel: model chunks per hypothesis in the last wave (1 = off)
@@ -263,6 +264,14 @@ int k4_topk(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, pgp_hyp
 int k4_topk_dev(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, pgp_hyp* out_dev);
 int k4_chain(pgp_ctx* ctx, const LastBatch& b, int64_t index_base, pgp_hyp* out_host, int cap, int* n_out);
 int k4_select_dev(pgp_ctx* ctx, const LastBatch& b, int k, int64_t index_base, int mode, pgp_hyp* hdr_dev, pgp_hyp* out_dev);
+// k4d_distinct.cu (arguments checked by the C ABI in pgp_api.cu)
+void k4d_set_symmetries(pgp_ctx* ctx, int obj, const double* R9, int n);
+// pgp_distinct_dev after its checks: descriptors up from pinned staging, the mask and the scan queued on ctx->stream
+int k4d_distinct_dev(pgp_ctx* ctx, const int32_t* objs, const int64_t* pool_offsets, int n_lists, const pgp_hyp* pool_dev, int k,
+                     double max_dist, double cos_angle, pgp_hyp* out_dev, double* poses16_dev, int32_t* n_kept_dev);
+// one list from host memory: pool up, run, kept records down, one synchronisation; returns the number kept
+int k4d_distinct_host(pgp_ctx* ctx, int obj, const pgp_hyp* pool_host, int m, int k, double max_dist, double cos_angle, pgp_hyp* out_host);
+void k4d_release(pgp_ctx* ctx);
 // pgp_comm.cu
 void pgp_comm_release(pgp_ctx* ctx);
 bool pgp_comm_active(const pgp_ctx* ctx);

@@ -7,6 +7,7 @@ the reference tree at run time)."""
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Optional, Sequence
 
 import numpy as np
@@ -225,6 +226,46 @@ class PoseEngine:
         out = np.zeros(max(self._tickets.pop(ticket), 1), HYP_DTYPE)
         m = self._check(self._lib.pgp_topk_end(self._ctx, ticket, _ptr(out)))
         return out[:m].copy()
+
+    # ------------------------------------------------------------------ K4d
+    def set_symmetries(self, obj: int, R=None):
+        """Discrete symmetries of model slot obj: (n, 3, 3) rotations in the centred model frame, the identity implied; None or an
+        empty array clears the set (pgp_set_symmetries)."""
+        R9 = np.ascontiguousarray(np.zeros((0, 9)) if R is None else R, np.float64).reshape(-1, 9)
+        self._check(self._lib.pgp_set_symmetries(self._ctx, int(obj), _ptr(R9) if len(R9) else None, len(R9)))
+
+    def topk_distinct(self, obj: int, m: int, k: int, max_dist: float, max_angle: float) -> np.ndarray:
+        """pgp_topk_distinct: the top m by score, then greedy suppression of every record within max_dist (metres, centred
+        translation) and max_angle (radians, up to the object's symmetries) of an earlier kept one; at most k records, in score order.
+        The kernel sees cos_angle = math.cos(max_angle)."""
+        out = np.zeros(max(int(k), 1), HYP_DTYPE)
+        n = self._check(self._lib.pgp_topk_distinct(self._ctx, int(obj), int(m), int(k), float(max_dist), math.cos(max_angle), _ptr(out)))
+        return out[:n].copy()
+
+    def distinct_device(self, objs, pool_offsets, pool, k: int, max_dist: float, max_angle: float, out, poses=None, n_kept=None):
+        """pgp_distinct_dev: pose-distinct selection over many pools on device data, asynchronous on the context's stream (set_stream).
+        Structure, numpy: objs (n_lists,) model slots; pool_offsets (n_lists + 1,) int64.  Device data, torch CUDA tensors: pool, the
+        concatenated 64-byte records (any dtype, pool_offsets[-1] x 64 bytes, e.g. topk_device's output); out, n_lists x k records
+        (kept ones first, then index = -1); poses (n_lists x k, 16) or (n_lists x k, 4, 4) f64 or None, the camera-frame poses (identity
+        after the kept ones); n_kept (n_lists,) i32 or None.  The kernel sees cos_angle = math.cos(max_angle).  The tensors are kept
+        alive until the next call."""
+        import torch
+        o = np.ascontiguousarray(objs, np.int32).reshape(-1)
+        off = np.ascontiguousarray(pool_offsets, np.int64).reshape(-1)
+        if len(off) != len(o) + 1:
+            raise ValueError("pool_offsets needs n_lists + 1 entries")
+        nbytes = lambda t: t.numel() * t.element_size()   # noqa: E731
+        for name, t, need in (("pool", pool, 64 * int(off[-1])), ("out", out, 64 * len(o) * int(k))):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.is_contiguous() and nbytes(t) >= need):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of at least {need} bytes")
+        want = {"poses": (poses, torch.float64, 16 * len(o) * int(k)), "n_kept": (n_kept, torch.int32, len(o))}
+        for name, (t, dt, numel) in want.items():
+            if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() >= numel):
+                raise ValueError(f"{name} must be a contiguous CUDA tensor of {numel} {dt}")
+        self._keep["distinct"] = (pool, out, poses, n_kept)
+        dp = lambda t: None if t is None else t.data_ptr()   # noqa: E731
+        self._check(self._lib.pgp_distinct_dev(self._ctx, _ptr(o) if len(o) else None, _ptr(off), len(o), dp(pool), int(k), float(max_dist),
+                                               math.cos(max_angle), dp(out), dp(poses), dp(n_kept)))
 
     # ------------------------------------------------------------------ multi-GPU (one process per GPU)
     @staticmethod
@@ -701,6 +742,16 @@ class PoseGroup:
         out = np.zeros(cap, HYP_DTYPE)
         m = self._check(self._lib.pgp_group_improving_chain(self._g, obj, _ptr(out), cap))
         return out[:m].copy()
+
+    def set_symmetries(self, obj: int, R=None):
+        R9 = np.ascontiguousarray(np.zeros((0, 9)) if R is None else R, np.float64).reshape(-1, 9)
+        self._check(self._lib.pgp_group_set_symmetries(self._g, int(obj), _ptr(R9) if len(R9) else None, len(R9)))
+
+    def topk_distinct(self, obj: int, m: int, k: int, max_dist: float, max_angle: float) -> np.ndarray:
+        """PoseEngine.topk_distinct over the group's merged top m: the same answer as one context on the concatenated batch."""
+        out = np.zeros(max(int(k), 1), HYP_DTYPE)
+        n = self._check(self._lib.pgp_group_topk_distinct(self._g, int(obj), int(m), int(k), float(max_dist), math.cos(max_angle), _ptr(out)))
+        return out[:n].copy()
 
 
 def exchange_merge(wire: np.ndarray, world: int, k: int, kind: int = 0, mode="count", auto_base: bool = False, cap: int = 4096) -> np.ndarray:
