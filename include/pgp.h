@@ -162,8 +162,7 @@ PGP_API int pgp_nearest_in_range(pgp_ctx* ctx, int obj, const float* T12_host, i
  *   "group_cull" = 0        do not skip the 32-point model groups whose bounding sphere cannot reach the scene (cross-check)
  *   "tail_split" = 1..16    model chunks per hypothesis in the last wave of the persistent scoring grid (default 4)
  *   "stream_upload" = 0     pgp_score_lcp uploads the whole batch before the scoring launch (use under profilers, which
- *                           serialise streams)
- *   "k3_warps_count", "k3_warps_weighted" = 16 | 24 | 32   warps per CTA of the scoring kernel (defaults 32 / 24) */
+ *                           serialise streams) */
 PGP_API int pgp_set_option(pgp_ctx* ctx, const char* name, int value);
 /* Number of my kernels launched by this context so far (bench.py's gpu_launches). */
 PGP_API int64_t pgp_launch_count(const pgp_ctx* ctx);

@@ -316,7 +316,7 @@ __global__ void __launch_bounds__(THREADS, 2) k3_lcp_kernel(const __grid_constan
 // and resolved by the exact, non-fused test of the reference in phase 2.  The labels are
 // conservative with respect to the difference between the fast transform and the reference's
 // rounding sequence (GridParams::inflate), so counts stay bit-exact.
-// warps per CTA (one CTA per SM) is a template parameter of the kernel: 32 (64 registers per thread) or 16 (128 registers)
+constexpr int FWARPS = 32;           // warps per CTA, one CTA per SM: 64 registers per thread
 constexpr int FUNROLL = 4;           // model points per lane per step (their label gathers are issued together)
 constexpr int SQCAP = 64;            // second-level (slow) queue slots per warp, weighted mode: < 32 left over + at most 32 new per drain
 constexpr int FQCAP = 32 + 32 * FUNROLL;   // queue slots per warp: < 32 left over + the new ones of one step
@@ -510,7 +510,7 @@ __device__ __forceinline__ void sa_load(unsigned sa, float (&a)[12]) {
 // dist[cell of T c] is a lower bound of the distance from T c to every scene point (cells outside the grid clamp to the border
 // cell: the projection onto the grid box only moves T c closer to the scene).  If that exceeds |A| r + delta + margins, no point
 // of the group can have a scene point within delta: the whole group is skipped -- one test instead of 32 label look-ups.
-template <bool SMEM_TABLE, bool FAST, int MODE, int U>
+template <bool SMEM_TABLE, bool FAST, int MODE>
 __device__ __forceinline__ int score_hypothesis(const LcpParams& p, const FineCtx& f, const float* __restrict__ T, long long h, int g_begin, int g_end) {
   static_assert(FUNROLL == 4, "the survivor list is read four entries at a time");
   const Xf x = load_xf(T, h);
@@ -717,9 +717,8 @@ __device__ __forceinline__ int score_hypothesis(const LcpParams& p, const FineCt
   return __reduce_add_sync(0xffffffffu, good);
 }
 
-template <bool SMEM_TABLE, int MODE, int FWARPS>   // MODE 0 = count (Verify), 1 = weighted with binary priors (WeightedVerify)
+template <bool SMEM_TABLE, int MODE>   // MODE 0 = count (Verify), 1 = weighted with binary priors (WeightedVerify)
 __global__ void __launch_bounds__(FWARPS * 32, 1) k3_fine_kernel(const __grid_constant__ LcpParams p) {
-  constexpr int PU = FWARPS == 32 ? 1 : 4;     // candidates in flight per lane in phase 2
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t mbar;
   __shared__ __align__(16) float s_xf[FWARPS * 12];   // FineCtx::sa
@@ -821,7 +820,7 @@ __global__ void __launch_bounds__(FWARPS * 32, 1) k3_fine_kernel(const __grid_co
           bound = fmaxf(bound, (fabsf(x.m[4 * r]) + fabsf(x.m[4 * r + 1]) + fabsf(x.m[4 * r + 2])) * p.model_rinf + fabsf(x.m[4 * r + 3]));
       }
       const bool fast = bound <= p.g.pos_bound;     // false for NaN / huge matrices: those take the reference's arithmetic
-      const int tot = m_begin >= m_end ? 0 : fast ? score_hypothesis<SMEM_TABLE, true, MODE, PU>(p, f, p.T, h, m_begin, m_end) : score_hypothesis<SMEM_TABLE, false, MODE, 1>(p, f, p.T, h, m_begin, m_end);
+      const int tot = m_begin >= m_end ? 0 : fast ? score_hypothesis<SMEM_TABLE, true, MODE>(p, f, p.T, h, m_begin, m_end) : score_hypothesis<SMEM_TABLE, false, MODE>(p, f, p.T, h, m_begin, m_end);
       if (lane == 0) {
         if (MODE == 0) {
           if (p.n_tiles == 1 && whole) {
@@ -981,7 +980,6 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
   if (fine_ok) {
     // shared-memory plan of k3_fine_kernel: model tile + one NaN group | normals (weighted) | bmrank | group spheres | survivor lists | queues
     const size_t smem_max = 216 * 1024;       // of the 227 KB a CTA may take; the kernel has 8 bytes of static shared memory
-    const int FWARPS = mode == PGP_LCP_WEIGHTED ? ctx->k3_warps_weighted : ctx->k3_warps_count;
     auto smem_need = [&](int cap, size_t table) {
       return (size_t)(cap + 32) * 16 + (mode == PGP_LCP_WEIGHTED ? (size_t)cap * 16 : 0) + table + (size_t)(cap >> 5) * 16 +
              (size_t)(FWARPS * ((cap >> 5) + FUNROLL)) * 2 + (size_t)FWARPS * (mode == PGP_LCP_WEIGHTED ? FQCAP * 7 + SQCAP * 7 : FQCAP * 6);
@@ -989,7 +987,8 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
     size_t bm = (size_t)s.bitmap_words * 8;
     int tile_cap = std::min((m.nv + 127) & ~127, 8192);
     if (smem_need(std::min(tile_cap, 2048), bm) > smem_max) bm = 0;          // table too big for smem: read it through L1
-    if (ctx->k3_smem_table == 0 || (ctx->k3_smem_table < 0 && mode == PGP_LCP_WEIGHTED)) bm = 0;   // see pgp_ctx::k3_smem_table
+    // weighted mode gathers three more tables and is faster with the 96 KB left to the L1 than with the table staged (measured)
+    if (mode == PGP_LCP_WEIGHTED) bm = 0;
     while (tile_cap > 128 && smem_need(tile_cap, bm) > smem_max) tile_cap -= 128;
     p.tile_cap = tile_cap;
     p.n_tiles = (m.nv + tile_cap - 1) / tile_cap;
@@ -1007,8 +1006,7 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
     p.dist_scale = (float)s.dist_r * 0.125f;
     p.sub_h2 = (s.g.h / (float)s.dist_r) * (s.g.h / (float)s.dist_r) * (1.0f - 1e-4f);
     p.ddx = s.g.dim[0] * s.dist_r; p.ddy = s.g.dim[1] * s.dist_r; p.ddz = s.g.dim[2] * s.dist_r;
-    size_t smem = smem_need(tile_cap, bm);
-    if (const char* pad = getenv("PGP_K3_SMEM_PAD_KB")) smem = std::min(smem_max, smem + (size_t)atoi(pad) * 1024);   // tuning: shrinks L1 by the same amount
+    const size_t smem = smem_need(tile_cap, bm);
     PGP_CUDA(ctx, cudaMemsetAsync(p.work, 0, 8 * (size_t)p.n_tiles, st));
     int grid = (int)std::min<long long>((n + FWARPS - 1) / FWARPS, ctx->sm_count);
     // the last two hypotheses' worth of work per warp is handed out in quarter-model units (shorter tail of the persistent grid)
@@ -1024,17 +1022,7 @@ int k3_score(pgp_ctx* ctx, const Model& m, const float* T_dev, int64_t n, int mo
       kern<<<grid, FWARPS * 32, smem, st>>>(p);
       return PGP_OK;
     };
-    int rc;
-    if (mode == PGP_LCP_COUNT) {
-      if (FWARPS == 32) rc = bm ? launch(k3_fine_kernel<true, 0, 32>) : launch(k3_fine_kernel<false, 0, 32>);
-      else if (FWARPS == 24) rc = bm ? launch(k3_fine_kernel<true, 0, 24>) : launch(k3_fine_kernel<false, 0, 24>);
-      else rc = bm ? launch(k3_fine_kernel<true, 0, 16>) : launch(k3_fine_kernel<false, 0, 16>);
-    } else {
-      if (FWARPS == 32) rc = bm ? launch(k3_fine_kernel<true, 1, 32>) : launch(k3_fine_kernel<false, 1, 32>);
-      else if (FWARPS == 28) rc = bm ? launch(k3_fine_kernel<true, 1, 28>) : launch(k3_fine_kernel<false, 1, 28>);
-      else if (FWARPS == 24) rc = bm ? launch(k3_fine_kernel<true, 1, 24>) : launch(k3_fine_kernel<false, 1, 24>);
-      else rc = bm ? launch(k3_fine_kernel<true, 1, 16>) : launch(k3_fine_kernel<false, 1, 16>);
-    }
+    const int rc = mode == PGP_LCP_WEIGHTED ? launch(k3_fine_kernel<false, 1>) : bm ? launch(k3_fine_kernel<true, 0>) : launch(k3_fine_kernel<false, 0>);
     if (rc) return rc;
     ctx->launches++;
     if (zero_from < n && scores_dev) {

@@ -153,13 +153,6 @@ int64_t pgp_launch_count(const pgp_ctx* ctx) { return ctx ? ctx->launches : 0; }
 int pgp_set_option(pgp_ctx* ctx, const char* name, int value) {
   CHECK_CTX(ctx);
   if (name && !strcmp(name, "force_coarse")) { ctx->force_coarse = value; return PGP_OK; }
-  if (name && (!strcmp(name, "k3_warps_count") || !strcmp(name, "k3_warps_weighted"))) {
-    if (value != 16 && value != 24 && value != 32 && !(value == 28 && !strcmp(name, "k3_warps_weighted")))
-      return pgp_fail(ctx, PGP_E_INVALID, "%s must be 16, 24 or 32 (weighted: also 28)", name);
-    (strcmp(name, "k3_warps_count") ? ctx->k3_warps_weighted : ctx->k3_warps_count) = value;
-    return PGP_OK;
-  }
-  if (name && !strcmp(name, "k3_smem_table")) { ctx->k3_smem_table = value < 0 ? -1 : (value ? 1 : 0); return PGP_OK; }
   if (name && !strcmp(name, "k7_mls")) { ctx->k7_mls = value ? 1 : 0; return PGP_OK; }
   if (name && !strcmp(name, "group_cull")) { ctx->group_cull = value ? 1 : 0; return PGP_OK; }
   if (name && !strcmp(name, "stream_upload")) { ctx->stream_upload = value ? 1 : 0; return PGP_OK; }

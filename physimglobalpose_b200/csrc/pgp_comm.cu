@@ -101,13 +101,12 @@ struct Comm {
 Comm* comm_of(pgp_ctx* ctx) {
   if (!ctx->comm) {
     Comm* c = new Comm();
-    // Default stream priority.  Measured (tools/gpu_round2_g.sh, gpu_round2_i.sh): giving the exchange stream the highest priority
+    // Least stream priority.  Measured (tools/gpu_round2_g.sh, gpu_round2_i.sh): giving the exchange stream the highest priority
     // does not shorten a scoring step (c2 at N = 4: 0.5637 vs 0.5628 ms) and makes a request made of many small launches slower and
-    // erratic (c3 at N = 2: 159 / 112 ms per step against 82 ms) -- PGP_EXCHANGE_PRIORITY=1 turns it on for experiments.
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    const char* pe = getenv("PGP_EXCHANGE_PRIORITY");
-    if (cudaStreamCreateWithPriority(&c->stream, cudaStreamNonBlocking, (pe && atoi(pe) == 1) ? hi : lo) != cudaSuccess) { delete c; return nullptr; }
+    // erratic (c3 at N = 2: 159 / 112 ms per step against 82 ms).
+    int lo = 0;
+    cudaDeviceGetStreamPriorityRange(&lo, nullptr);
+    if (cudaStreamCreateWithPriority(&c->stream, cudaStreamNonBlocking, lo) != cudaSuccess) { delete c; return nullptr; }
     ctx->comm = c;
   }
   return static_cast<Comm*>(ctx->comm);

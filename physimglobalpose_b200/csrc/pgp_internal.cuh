@@ -229,9 +229,6 @@ struct pgp_ctx {
   int k7_mls = 1;                          // segment preparation: 1 = MLS polynomial projection + normals (what the reference runs), 0 = PCA normals on the centroids
   int stream_upload = 1;  // pgp_score_lcp: overlap the batch upload with the scoring launch (0: upload first; use under profilers)
   int tail_split = 4;     // K3 fine kernel: model chunks per hypothesis in the last wave (1 = off)
-  int k3_warps_count = 32, k3_warps_weighted = 32;   // warps per CTA of k3_fine_kernel (32 -> 64 registers/thread, 24 -> 80, 16 -> 128)
-  int k3_smem_table = -1; // bitmap+rank table of k3_fine_kernel in shared memory: 1 yes, 0 no (read through L1), -1 = count mode yes, weighted mode no
-                          // (measured: weighted mode gathers three more tables and is faster with the 96 KB left to the L1 than with the table staged)
   int group_cull = 1;     // K3 fine kernel: drop groups of 32 model points whose bounding sphere cannot reach the scene (0 = off, test hook)
   int force_coarse = 0;   // test hook: score on the 27-cell path even when the fine grid exists
   std::string err;

@@ -53,6 +53,8 @@ def test_lcp_delta_5mm_golden(engine, lcp):
     d5 = np.load(os.path.join(G, "lcp_small_d5.npz"))
     engine.set_scene(lcp["scene_xyz"], lcp["scene_nrm"], 0.005)
     engine.set_model(0, lcp["model_xyz"], lcp["model_nrm"])
+    # the bitmap+rank table (8 bytes per 32 cells) is larger than the 216 KB shared-memory plan: count mode reads it through L1
+    assert engine.grid_info()["n_cells"] // 4 > 216 * 1024
     counts, _ = engine.score_lcp(0, lcp["T"], "count")
     assert np.array_equal(counts, d5["counts"])
     _, ws = engine.score_lcp(0, lcp["T"], "weighted")

@@ -194,11 +194,14 @@ def test_multi_tile_model(engine, port_lib):
 
 
 def test_c5_shape_parity(engine, port_lib):
-    """configs[4] shape (30k-point model, 300k-point scene): the model spans four shared-memory tiles and the scene's cell table
-    is larger than shared memory (read through L1); counts and weighted scores on a sample of hypotheses equal the oracle's."""
+    """configs[4] shape (30k-point model, 300k-point scene): the model spans several shared-memory tiles, and in count mode the
+    scene's 96 KB bitmap+rank table is staged in shared memory next to each tile; counts and weighted scores on a sample of
+    hypotheses equal the oracle's.  (The table read through L1 in count mode: test_gpu_golden.py::test_lcp_delta_5mm_golden.)"""
     prob = synth.make_problem(30000, 300000, 0.01, seed=51)
     T = synth.make_hypotheses(prob, 48, seed=52)
     _setup(engine, prob)
+    # 8 bytes per 32 cells; k3_score stages it while its plan fits in 216 KB, and the rest of the plan is < 68 KB here
+    assert engine.grid_info()["n_cells"] // 4 < 148 * 1024
     o = _oracle(port_lib, prob)
     want = o.verify(T)
     counts, _ = engine.score_lcp(0, T, "count")
@@ -227,6 +230,18 @@ def test_tail_split_units(engine, port_lib):
     assert np.array_equal(res[4][0][0][sel], o.verify(T[sel]))
     ws, wn = o.weighted_verify(T[sel])
     assert np.array_equal(res[4][1][1][sel], ws) and np.array_equal(res[4][1][0][sel], wn.astype(np.uint32))
+
+
+def test_k3_kernel_shape_is_not_an_option(engine):
+    """K3's fine kernel is built once per mode (32 warps; the cell table staged in count mode when it fits, read through L1
+    otherwise and in weighted mode): warp-count and table-placement names are refused like any unknown option, and the
+    remaining options are still accepted."""
+    from physimglobalpose_b200 import _lib
+    for name in ("k3_warps_count", "k3_warps_weighted", "k3_smem_table"):
+        with pytest.raises(_lib.PgpError) as e:
+            engine.set_option(name, 32)
+        assert _lib.STATUS[e.value.code] == "PGP_E_INVALID" and "unknown option" in str(e.value)
+    engine.set_option("tail_split", 4)
 
 
 def test_group_cull_is_exact(engine, port_lib):

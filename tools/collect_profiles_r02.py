@@ -17,7 +17,7 @@ def raw_metrics(rep):
     return dict(zip(rows[0], rows[2]))
 
 
-KERNELS = {"r02_k3": "k3_fine_kernelILb1ELi0ELi32", "r02_k3w": "k3_fine_kernelILb0ELi1ELi32", "r02_k2_query": "k2_join_queryILb0", "r02_k2_select": "k2_join_select",
+KERNELS = {"r02_k3": "k3_fine_kernelILb1ELi0E", "r02_k3w": "k3_fine_kernelILb0ELi1E", "r02_k2_query": "k2_join_queryILb0", "r02_k2_select": "k2_join_select",
            "r02_k2s_bases": "k2s_select_basesENS", "r02_k5": "k5_tricp_kernel"}
 traffic = {}
 for name, mangled in KERNELS.items():

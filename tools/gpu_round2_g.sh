@@ -1,5 +1,5 @@
-# what costs the last 2-5 % at N > 1?  c2 / c2w at N = $1: as shipped (exchange stream at top priority), exchange at default priority,
-# and N independent replicas without any collective
+# what costs the last 2-5 % at N > 1?  c2 / c2w at N = $1: as shipped (exchange stream at the least priority) and N independent
+# replicas without any collective
 N=${1:-4}
 run() { # config tag
   timeout 400 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29519 bench.py --gpus $N --config $1 > gpurun_out/g_$1_$2.json 2> gpurun_out/g_$1_$2.err
@@ -12,5 +12,4 @@ except Exception as e:
 PY
 }
 run c2 prio; run c2w prio
-PGP_EXCHANGE_PRIORITY=0 run c2 noprio; PGP_EXCHANGE_PRIORITY=0 run c2w noprio
 PGP_BENCH_NO_COMM=1 run c2 nocomm; PGP_BENCH_NO_COMM=1 run c2w nocomm

@@ -9,4 +9,4 @@ except Exception as e:
 PY
 }
 nproc; free -g | head -2
-run prio; PGP_EXCHANGE_PRIORITY=0 run noprio; run prio2
+run prio; run prio2
